@@ -13,7 +13,7 @@ LIB_PATH = Path(__file__).resolve().parent / "lib" / "liblightglue_b200.so"
 
 F32, BF16, F32X3 = 0, 1, 2
 EPI_ROWMAJOR, EPI_HEADS, EPI_LN_GELU = 0, 1, 2
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 _p, _i, _f = C.c_void_p, C.c_int, C.c_float
 
@@ -45,6 +45,8 @@ SIGNATURES = {
     "lgb200_x3_assign_scores": [_p, _p, _p, _i, _i, _p, _i, _i, _p, _p],
     "lgb200_attention_bwd": [_p, _p, _p, _p, _p, _i, _i, _p, _i, _p, _p, _p, _p, _p],
     "lgb200_attention_bwd_workspace": [_i, _i, _p],
+    "lgb200_attention_bwd_bf16": [_p, _p, _p, _p, _p, _i, _i, _p, _i, _p, _p, _p, _p, _p],
+    "lgb200_attention_bwd_bf16_workspace": [_i, _i, _p],
     "lgb200_heads_bwd": [_p, _p, _p, _p, _p, _p, _i, _i, _p, _i, _f, _f, _f, _p, _p, _p],
     "lgb200_ln_gelu_bwd": [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _p],
     "lgb200_assign_dsim": [_p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p],

@@ -694,6 +694,29 @@ extern "C" int lgb200_attention_bwd_workspace(int S, int Lp, long long* n_floats
   return LGB200_OK;
 }
 
+extern "C" int lgb200_attention_bwd_bf16(const void* Q, const void* K, const void* V, const void* ctx, const float* dctx,
+                                         int S, int Lp, const int32_t* lens, int kv_xor, float* dQ, float* dK, float* dV,
+                                         float* workspace, void* stream) {
+  if (!Q || !K || !V || !ctx || !dctx || !dQ || !dK || !dV || !workspace) return LGB200_ERR_NULL;
+  if (S <= 0 || Lp <= 0 || Lp % 128 || (kv_xor != 0 && kv_xor != 1) || (kv_xor && (S & 1))) return LGB200_ERR_SHAPE;
+  cudaStream_t st = lg_stream(stream);
+  cudaError_t e;
+  const size_t nb = (size_t)S * Lp * LG_D * sizeof(float);
+  if ((e = cudaMemsetAsync(dQ, 0, nb, st)) != cudaSuccess) return (int)e;
+  if ((e = cudaMemsetAsync(dK, 0, nb, st)) != cudaSuccess) return (int)e;
+  if ((e = cudaMemsetAsync(dV, 0, nb, st)) != cudaSuccess) return (int)e;
+  using bf = __nv_bfloat16;
+  return lg_bf16_attention_bwd((const bf*)Q, (const bf*)K, (const bf*)V, (const bf*)ctx, dctx, S, Lp, lens, kv_xor, dQ,
+                               dK, dV, workspace, st);
+}
+
+extern "C" int lgb200_attention_bwd_bf16_workspace(int S, int Lp, long long* n_floats) {
+  if (!n_floats) return LGB200_ERR_NULL;
+  if (S <= 0 || Lp <= 0 || Lp % 128) return LGB200_ERR_SHAPE;
+  *n_floats = (long long)lg_bf16_attention_bwd_ws_floats(S, Lp);
+  return LGB200_OK;
+}
+
 extern "C" int lgb200_heads_bwd(const float* dQ, const float* dK, const float* dV, const float* Q, const float* K,
                                 const float* rot, int S, int Lp, const int32_t* lens, int n_parts, float scale0,
                                 float scale1, float scale2, float* out, float* dtheta, void* stream) {

@@ -40,6 +40,11 @@ size_t lg_x3_attention_bwd_ws_floats(int S, int Lp);
 int lg_x3_attention_bwd(const float* Q, const float* K, const float* V, const float* ctx, const float* dctx, int S,
                         int Lp, const int32_t* lens, int kv_xor, float* dQ, float* dK, float* dV, float* ws,
                         cudaStream_t st);
+// the same kernel template on bf16 operands: backward of the bf16 forward (lg_x3_attn_bwd.cu)
+size_t lg_bf16_attention_bwd_ws_floats(int S, int Lp);
+int lg_bf16_attention_bwd(const __nv_bfloat16* Q, const __nv_bfloat16* K, const __nv_bfloat16* V,
+                          const __nv_bfloat16* ctx, const float* dctx, int S, int Lp, const int32_t* lens, int kv_xor,
+                          float* dQ, float* dK, float* dV, float* ws, cudaStream_t st);
 // x3 plane scaling: a plane pair stores x * 2^e so that the LOW plane stays a normal fp16 number (fp16 normals end at
 // 6.1e-5 and lo ~ 2^-11 |x|: unscaled, the low planes of all weights and of every activation below 0.12 are subnormal
 // (or flushed) and the pair carries ~12 bits instead of 22).  Powers of two: exact, undone in the consuming epilogue.

@@ -28,8 +28,16 @@
 // tools/attn_bwd_accuracy.py, profiles/r2_attn_bwd_tcgen05.txt).  out1 / out2 therefore collect XB_FLUSH tiles (48 MMAs)
 // and are then added, round-to-nearest, to fp32 running sums that every softmax thread keeps for its own row in shared
 // memory ([column][row]: conflict-free); the first MMA after a flush overwrites the accumulator.
+//
+// BF16 INSTANTIATION (template parameter BF, lg_bf16_attention_bwd): the backward of the bf16 forward kernels
+// (lg_tc_attn.cu) on the operands that forward read -- Q, K, V bf16 as they are, dO converted once to a head-major bf16
+// copy.  Every product is ONE kind::f16 MMA with bf16 A / B formats; P and D go to TMEM as one bf16 plane each, X and U
+// take 32 TMEM columns each.  No plane scalings (bf16 has the exponent range of fp32): g = 1, D is stored unscaled;
+// P keeps the factor 256 of the shared lse - 8 convention.  delta = <dO, O> is taken in fp32 from the fp32 dctx and the
+// bf16 ctx of the forward.  The stage / TMEM layout and the two-level accumulation are those of the x3 kernel.
 #include "lg_internal.cuh"
 #include "lg_tc_common.cuh"
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <stdlib.h>
 #include <type_traits>
@@ -41,7 +49,7 @@ constexpr int XB_TBY = XB_OT * 64 * 2;          // one plane of an other tile (6
 constexpr int XB_NST = 4;                       // stages of (Yh | Yl | Wh | Wl)
 constexpr int XB_Y = 0;                         // XB_NST x 32 KB
 constexpr int XB_BAR = XB_Y + XB_NST * 4 * XB_TBY;  // 128 KB of tiles
-constexpr int XB_NBAR = 1 + 2 * XB_NST + 2 + 2 + 1 + 1;
+constexpr int XB_NBAR = 1 + 2 * XB_NST + 2 + 2 + 2 + 1;
 constexpr int XB_ACC = XB_BAR + 256;            // [128 columns][128 rows] fp32 running sums of out1 | out2 (64 KB)
 constexpr int XB_XCH = XB_ACC;                  // [128 rows][NP parts] float4 (max, sum, partial delta): statistics sweep only
 constexpr int XB_SMEM = XB_ACC + 128 * 128 * 4;
@@ -52,15 +60,26 @@ static_assert(XB_SMEM <= 227 * 1024, "attention backward: shared memory");
 constexpr uint32_t XT_SC = 0, XT_DP = 128, XT_O1 = 256, XT_O2 = 320, XT_XH = 384, XT_XL = 416, XT_UH = 448, XT_UL = 480;
 constexpr float XB_DC = 1.f / 64.f;             // D planes hold (g / 64) D
 // The exponentials are taken against lse - 8, i.e. they ARE the P plane values 256 P (LG_X3_EP); the workspace holds
-// lse2 - 8 and delta * g * XB_DT so that D = (256 P) * (dp * XB_DPS - delta') needs no further scaling (powers of two).
-constexpr float XB_DT = XB_DC / LG_X3_EP;       // delta' = delta * g * XB_DT
+// lse2 - 8 and delta * g * DT so that D = (256 P) * (dp * DPS - delta') needs no further scaling (powers of two).
 static_assert(LG_X3_EP == 256.f, "the exponentials are taken against lse - 8 = lse - log2(LG_X3_EP)");
-constexpr float XB_DPS = XB_DT / LG_X3_EA;      // dp arrives as g * 64 * dP
 constexpr float XB_LN2 = 0.69314718055994530942f;
 
 __host__ __device__ constexpr uint32_t xb_idesc(int M, int N, int b_mn_major) {  // kind::f16, fp16 x fp16 -> fp32
   return (1u << 4) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
+// per-instantiation scalings: BF = false is the x3 kernel (planes of 64 Q / K / V, g dO and (g / 64) D), BF = true
+// uses unscaled bf16 operands
+template <bool BF>
+struct XbMode {
+  static constexpr int NPL = BF ? 1 : 2;                  // planes per operand
+  static constexpr float EA = BF ? 1.f : LG_X3_EA;        // scaling of Q, K, V (and of Y, W)
+  static constexpr float DC = BF ? 1.f : XB_DC;           // D planes hold (g DC) D
+  static constexpr float DT = DC / LG_X3_EP;              // delta' = delta * g * DT
+  static constexpr float DPS = DT / EA;                   // dp arrives as g EA dP
+  static constexpr uint32_t idesc(int M, int N, int b_mn_major) {
+    return BF ? tc::idesc_bf16(M, N, b_mn_major) : xb_idesc(M, N, b_mn_major);
+  }
+};
 __device__ __forceinline__ float xb_ex2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -86,6 +105,11 @@ __device__ __forceinline__ void xb_split(float a, float b, uint32_t& hi, uint32_
   const __half2 ll = __floats2half2_rn(a - hf.x, b - hf.y);
   hi = *reinterpret_cast<const uint32_t*>(&hh);
   lo = *reinterpret_cast<const uint32_t*>(&ll);
+}
+// (a, b) -> bf16 pair (a in the low half)
+__device__ __forceinline__ uint32_t xb_pack_bf16(float a, float b) {
+  const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
+  return *reinterpret_cast<const uint32_t*>(&v);
 }
 
 // ----------------------------------------------------------------------------------------------- operand preparation
@@ -142,16 +166,36 @@ __global__ void __launch_bounds__(256) xb_split_kernel(const float* __restrict__
   *reinterpret_cast<uint4*>(out + row * LG_DH + d8 * 8) = hi;
   *reinterpret_cast<uint4*>(out + plane + row * LG_DH + d8 * 8) = lo;
 }
+// bf16 backward: dctx fp32 [S,Lp,256] -> dO bf16 head-major [S,4,Lp,64]; rows >= lens are zero
+__global__ void __launch_bounds__(256) xb_bf16_dout_kernel(const float* __restrict__ src, int S, int Lp,
+                                                           const int32_t* __restrict__ lens, __nv_bfloat16* __restrict__ out) {
+  const size_t n8 = (size_t)S * LG_HEADS * Lp * (LG_DH / 8);
+  const size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+  if (i >= n8) return;
+  const int d8 = (int)(i % (LG_DH / 8));
+  const size_t row = i / (LG_DH / 8);  // (s, h, l)
+  const int l = (int)(row % Lp), h = (int)((row / Lp) % LG_HEADS), s = (int)(row / ((size_t)Lp * LG_HEADS));
+  uint4 o = make_uint4(0, 0, 0, 0);
+  if (!lens || l < lens[s]) {
+    const float* p = src + ((size_t)s * Lp + l) * LG_D + h * LG_DH + d8 * 8;
+    const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
+    o = make_uint4(xb_pack_bf16(a.x, a.y), xb_pack_bf16(a.z, a.w), xb_pack_bf16(b.x, b.y), xb_pack_bf16(b.z, b.w));
+  }
+  *reinterpret_cast<uint4*>(out + row * LG_DH + d8 * 8) = o;
+}
 
 // ----------------------------------------------------------------------------------------------- the backward kernel
-// NP = softmax threads per own row: 2 (8 warps, 32 score columns each) or 4 (16 warps, 16 columns each)
-template <bool DKV, int NP>
+// NP = softmax threads per own row: 2 (8 warps, 32 score columns each) or 4 (16 warps, 16 columns each).
+// BF: bf16 operands (Xp / Up are then bf16 rows addressed as 2-byte elements, plane unused, ctx bf16, gptr unused).
+template <bool DKV, int NP, bool BF>
 __global__ void __launch_bounds__(64 + 128 * NP, 1)
 x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up, size_t plane,
                    const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmW, int Lp,
-                   const int32_t* __restrict__ lens, int kv_xor, const float* __restrict__ ctx,
+                   const int32_t* __restrict__ lens, int kv_xor, const void* __restrict__ ctx,
                    const float* __restrict__ dctx, const float* __restrict__ gptr, float* __restrict__ lse2,
                    float* __restrict__ dlt, float* __restrict__ out1, float* __restrict__ out2) {
+  using M = XbMode<BF>;
+  constexpr int W_OFF = M::NPL * XB_TBY;  // W planes behind the Y planes of a stage
   const int h = blockIdx.y, r0 = blockIdx.x * 128, s = blockIdx.z;
   const int so = s ^ kv_xor;
   const int n_own = lens ? lens[s] : Lp, n_oth = lens ? lens[so] : Lp;
@@ -171,8 +215,11 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
   uint64_t* y_empty = y_full + XB_NST;
   uint64_t* sc_full = y_empty + XB_NST;  // [2]
   uint64_t* sc_free = sc_full + 2;       // [2] statistics sweep only
+  // [2], per score buffer: a warp that is done with tile j may already arrive for tile j + 1 (its scores were issued
+  // before the issuer waits for tile j's planes) while another warp still works on tile j; on ONE barrier that early
+  // arrival would complete tile j's phase without the late warp's planes
   uint64_t* pd_ready = sc_free + 2;
-  uint64_t* out_done = pd_ready + 1;     // one phase per flush group
+  uint64_t* out_done = pd_ready + 2;     // one phase per flush group
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + XB_NBAR);
   float4* xch = reinterpret_cast<float4*>(smem + XB_XCH);
 
@@ -182,7 +229,7 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
     tc::mbar_init(xu_ready, 4 * NP);
     for (int i = 0; i < XB_NST; ++i) { tc::mbar_init(&y_full[i], 1); tc::mbar_init(&y_empty[i], 1); }
     for (int i = 0; i < 2; ++i) { tc::mbar_init(&sc_full[i], 1); tc::mbar_init(&sc_free[i], 4 * NP); }
-    tc::mbar_init(pd_ready, 4 * NP);
+    for (int i = 0; i < 2; ++i) tc::mbar_init(&pd_ready[i], 4 * NP);
     tc::mbar_init(out_done, 1);
     tc::fence_barrier_init();
   }
@@ -201,22 +248,22 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
         tc::mbar_wait_relaxed(&y_empty[st], ((it / XB_NST) & 1) ^ 1);  // (sleeping polls: the issue slots belong to the softmax warps)
         uint8_t* dst = smem + XB_Y + st * 4 * XB_TBY;
         const bool main = it >= first_main;
-        tc::mbar_arrive_expect_tx(&y_full[st], (main ? 4 : 2) * XB_TBY);
+        tc::mbar_arrive_expect_tx(&y_full[st], (main ? 2 : 1) * W_OFF);
         tc::tma_load_3d(dst, &tmY, &y_full[st], 0, oth_row + j * XB_OT, 0);
-        tc::tma_load_3d(dst + XB_TBY, &tmY, &y_full[st], 0, oth_row + j * XB_OT, 1);
+        if (!BF) tc::tma_load_3d(dst + XB_TBY, &tmY, &y_full[st], 0, oth_row + j * XB_OT, 1);
         if (main) {
-          tc::tma_load_3d(dst + 2 * XB_TBY, &tmW, &y_full[st], 0, oth_row + j * XB_OT, 0);
-          tc::tma_load_3d(dst + 3 * XB_TBY, &tmW, &y_full[st], 0, oth_row + j * XB_OT, 1);
+          tc::tma_load_3d(dst + W_OFF, &tmW, &y_full[st], 0, oth_row + j * XB_OT, 0);
+          if (!BF) tc::tma_load_3d(dst + 3 * XB_TBY, &tmW, &y_full[st], 0, oth_row + j * XB_OT, 1);
         }
       }
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------------------------------- MMA issuer
-    constexpr uint32_t idesc_sc = xb_idesc(128, XB_OT, 0);
-    constexpr uint32_t idesc_out = xb_idesc(128, 64, 1);
+    constexpr uint32_t idesc_sc = M::idesc(128, XB_OT, 0);
+    constexpr uint32_t idesc_out = M::idesc(128, 64, 1);
     const uint32_t tXh = tmem + XT_XH, tXl = tmem + XT_XL, tUh = tmem + XT_UH, tUl = tmem + XT_UL;
     // TMEM address of the A operand of K step ks in a plane pair that a softmax thread wrote over ITS score columns:
-    // [part][hi: KP steps x 8 columns | lo: KP steps x 8 columns]
+    // [part][hi: KP steps x 8 columns | lo: KP steps x 8 columns] (BF: the hi half only, lo = 0)
     auto plane_col = [](int lo, int ks) -> uint32_t { return (uint32_t)((ks / KP) * COLS + lo * (COLS / 2) + (ks % KP) * 8); };
     auto issue_sc = [&](int it) {  // sc[it & 1] = X . Y^T and (main sweep) dp[it & 1] = U . W^T, A operands from TMEM
       const int st = it % XB_NST, b = it & 1;
@@ -230,21 +277,30 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
       tc::fence_after_sync();
       const uint32_t ybase = tc::smem_u32(smem + XB_Y + st * 4 * XB_TBY);
       const uint64_t dYh = tc::smem_desc_sw128(ybase, 0, 1024), dYl = tc::smem_desc_sw128(ybase + XB_TBY, 0, 1024);
-      const uint64_t dWh = tc::smem_desc_sw128(ybase + 2 * XB_TBY, 0, 1024), dWl = tc::smem_desc_sw128(ybase + 3 * XB_TBY, 0, 1024);
+      const uint64_t dWh = tc::smem_desc_sw128(ybase + W_OFF, 0, 1024), dWl = tc::smem_desc_sw128(ybase + 3 * XB_TBY, 0, 1024);
       const uint32_t tS = tmem + XT_SC + b * XB_OT, tP = tmem + XT_DP + b * XB_OT;
       if (tc::elect_one()) {
+        if constexpr (BF) {  // one MMA per product
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          tc::umma_ts(tS, tXl + k * 8, dYh + 2 * k, idesc_sc, k != 0);
-          tc::umma_ts(tS, tXh + k * 8, dYl + 2 * k, idesc_sc, 1);
-          tc::umma_ts(tS, tXh + k * 8, dYh + 2 * k, idesc_sc, 1);
-        }
-        if (main) {
+          for (int k = 0; k < 4; ++k) tc::umma_ts(tS, tXh + k * 8, dYh + 2 * k, idesc_sc, k != 0);
+          if (main) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) tc::umma_ts(tP, tUh + k * 8, dWh + 2 * k, idesc_sc, k != 0);
+          }
+        } else {
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
-            tc::umma_ts(tP, tUl + k * 8, dWh + 2 * k, idesc_sc, k != 0);
-            tc::umma_ts(tP, tUh + k * 8, dWl + 2 * k, idesc_sc, 1);
-            tc::umma_ts(tP, tUh + k * 8, dWh + 2 * k, idesc_sc, 1);
+            tc::umma_ts(tS, tXl + k * 8, dYh + 2 * k, idesc_sc, k != 0);
+            tc::umma_ts(tS, tXh + k * 8, dYl + 2 * k, idesc_sc, 1);
+            tc::umma_ts(tS, tXh + k * 8, dYh + 2 * k, idesc_sc, 1);
+          }
+          if (main) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+              tc::umma_ts(tP, tUl + k * 8, dWh + 2 * k, idesc_sc, k != 0);
+              tc::umma_ts(tP, tUh + k * 8, dWl + 2 * k, idesc_sc, 1);
+              tc::umma_ts(tP, tUh + k * 8, dWh + 2 * k, idesc_sc, 1);
+            }
           }
         }
         tc::umma_commit(&sc_full[b]);
@@ -259,17 +315,22 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
       if (it + 1 < n_iter) issue_sc(it + 1);
       if (it < first_main) continue;
       const int jm = it - first_main, st = it % XB_NST, b = it & 1;
-      tc::mbar_wait_relaxed(pd_ready, jm & 1, 32);
+      tc::mbar_wait_relaxed(&pd_ready[b], (jm >> 1) & 1, 32);
       tc::fence_after_sync();
       const uint32_t ybase = tc::smem_u32(smem + XB_Y + st * 4 * XB_TBY);
       // MN-major B operands: row = other row (the K index of these MMAs), 16 rows = 2048 B per K step
       const uint64_t mYh = tc::smem_desc_sw128(ybase, XB_TBY, 1024), mYl = tc::smem_desc_sw128(ybase + XB_TBY, XB_TBY, 1024);
-      const uint64_t mWh = tc::smem_desc_sw128(ybase + 2 * XB_TBY, XB_TBY, 1024), mWl = tc::smem_desc_sw128(ybase + 3 * XB_TBY, XB_TBY, 1024);
+      const uint64_t mWh = tc::smem_desc_sw128(ybase + W_OFF, XB_TBY, 1024), mWl = tc::smem_desc_sw128(ybase + 3 * XB_TBY, XB_TBY, 1024);
       const uint32_t tD = tmem + XT_DP + b * XB_OT, tPp = tmem + XT_SC + b * XB_OT;  // D planes over dp, P planes over sc
       if (tc::elect_one()) {
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
           const uint32_t acc = ((jm % XB_FLUSH) | k) != 0;  // fresh accumulators after every flush
+          if constexpr (BF) {
+            tc::umma_ts(tmem + XT_O1, tD + plane_col(0, k), mYh + k * (2048 >> 4), idesc_out, acc);
+            if (DKV) tc::umma_ts(tmem + XT_O2, tPp + plane_col(0, k), mWh + k * (2048 >> 4), idesc_out, acc);
+            continue;
+          }
           tc::umma_ts(tmem + XT_O1, tD + plane_col(1, k), mYh + k * (2048 >> 4), idesc_out, acc);
           tc::umma_ts(tmem + XT_O1, tD + plane_col(0, k), mYl + k * (2048 >> 4), idesc_out, 1);
           tc::umma_ts(tmem + XT_O1, tD + plane_col(0, k), mYh + k * (2048 >> 4), idesc_out, 1);
@@ -299,8 +360,8 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
     };
     const int r = quarter * 32 + lane;
     const bool row_ok = r0 + r < n_own;
-    constexpr float s_us = 1.f / (LG_X3_EA * LG_X3_EA);
-    const float g = *gptr;
+    constexpr float s_us = 1.f / (M::EA * M::EA);
+    const float g = BF ? 1.f : *gptr;
     const size_t own_stat = ((size_t)s * LG_HEADS + h) * Lp + r0 + r;
     const size_t oth_stat = ((size_t)so * LG_HEADS + h) * Lp;
     float lse_own = 0.f, dlt_own = 0.f;  // DQ: this row's log-sum-exp and g * delta
@@ -314,6 +375,7 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
       const uint32_t cols[4] = {XT_XH, XT_XL, XT_UH, XT_UL};
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
+        if (BF && (q & 1)) continue;  // (no lo planes)
         uint32_t w[NW];
         const uint4* src = reinterpret_cast<const uint4*>(srcs[q]) + part * (NW / 4);
 #pragma unroll
@@ -363,11 +425,26 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
       float dot = 0.f;
       if (row_ok) {
         const size_t off = ((size_t)s * Lp + r0 + r) * LG_D + h * LG_DH + part * OC;
+        if constexpr (BF) {
 #pragma unroll
-        for (int i = 0; i < OC / 4; ++i) {
-          const float4 o = *reinterpret_cast<const float4*>(ctx + off + 4 * i);
-          const float4 gr = *reinterpret_cast<const float4*>(dctx + off + 4 * i);
-          dot += (o.x * gr.x + o.y * gr.y) + (o.z * gr.z + o.w * gr.w);
+          for (int i = 0; i < OC / 8; ++i) {
+            const uint4 o = *reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(ctx) + off + 8 * i);
+            const float4 ga = *reinterpret_cast<const float4*>(dctx + off + 8 * i);
+            const float4 gb = *reinterpret_cast<const float4*>(dctx + off + 8 * i + 4);
+            const float2 o0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&o.x));
+            const float2 o1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&o.y));
+            const float2 o2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&o.z));
+            const float2 o3 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&o.w));
+            dot += (o0.x * ga.x + o0.y * ga.y) + (o1.x * ga.z + o1.y * ga.w);
+            dot += (o2.x * gb.x + o2.y * gb.y) + (o3.x * gb.z + o3.y * gb.w);
+          }
+        } else {
+#pragma unroll
+          for (int i = 0; i < OC / 4; ++i) {
+            const float4 o = *reinterpret_cast<const float4*>(reinterpret_cast<const float*>(ctx) + off + 4 * i);
+            const float4 gr = *reinterpret_cast<const float4*>(dctx + off + 4 * i);
+            dot += (o.x * gr.x + o.y * gr.y) + (o.z * gr.z + o.w * gr.w);
+          }
         }
       }
       xch[r * NP + part] = make_float4(m, l, dot, 0.f);
@@ -386,7 +463,7 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
         delta += pt[i].z;
       }
       lse_own = lsum > 0.f ? mnew + log2f(lsum) - 8.f : INFINITY;  // (2^(s - lse_own) = 256 P)
-      dlt_own = delta * g * XB_DT;
+      dlt_own = delta * g * M::DT;
       if (part == 0 && row_ok) {
         lse2[own_stat] = lse_own;
         dlt[own_stat] = dlt_own;
@@ -456,7 +533,16 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
             const int i = 4 * i4 + c;
             const bool ok = FULL || n0 + i < n_oth;  // (statistics of padding rows are undefined: select, not multiply)
             p[c] = ok ? xb_ex2(fmaf(__uint_as_float(sv[i]), s_us, -lq[c])) : 0.f;            // 256 P
-            d[c] = ok ? p[c] * fmaf(__uint_as_float(dv[i]), XB_DPS, -dq[c]) : 0.f;           // (g / 64) P (dP - delta)
+            d[c] = ok ? p[c] * fmaf(__uint_as_float(dv[i]), M::DPS, -dq[c]) : 0.f;           // (g DC) P (dP - delta)
+          }
+          if constexpr (BF) {
+            dh[2 * i4] = xb_pack_bf16(d[0], d[1]);
+            dh[2 * i4 + 1] = xb_pack_bf16(d[2], d[3]);
+            if (DKV) {
+              ph[2 * i4] = xb_pack_bf16(p[0], p[1]);
+              ph[2 * i4 + 1] = xb_pack_bf16(p[2], p[3]);
+            }
+            continue;
           }
           xb_split_sat(d[0], d[1], dh[2 * i4], dl[2 * i4]);
           xb_split_sat(d[2], d[3], dh[2 * i4 + 1], dl[2 * i4 + 1]);
@@ -477,22 +563,22 @@ x3_attn_bwd_kernel(const __half* __restrict__ Xp, const __half* __restrict__ Up,
       }
       // the plane pairs go over this thread's OWN score columns (hi | lo), read above: no other thread touches them
       st_plane(XT_DP + b * XB_OT + part * COLS, dh);
-      st_plane(XT_DP + b * XB_OT + part * COLS + COLS / 2, dl);
+      if (!BF) st_plane(XT_DP + b * XB_OT + part * COLS + COLS / 2, dl);
       if (DKV) {
         st_plane(XT_SC + b * XB_OT + part * COLS, ph);
-        st_plane(XT_SC + b * XB_OT + part * COLS + COLS / 2, pl);
+        if (!BF) st_plane(XT_SC + b * XB_OT + part * COLS + COLS / 2, pl);
       }
       tc::tmem_st_wait();
       tc::fence_before_sync();
       __syncwarp();
-      if (lane == 0) tc::mbar_arrive(pd_ready);
+      if (lane == 0) tc::mbar_arrive(&pd_ready[b]);
     }
     // ---- epilogue: this thread's OC output columns of its row
     tc::mbar_wait(out_done, ((n_tiles + XB_FLUSH - 1) / XB_FLUSH - 1) & 1);
     tc::fence_after_sync();
     flush();
     if (row_ok) {
-      const float k1 = XB_LN2 / (g * XB_DC * LG_X3_EA);  // raw = ((g / 64) D) . (64 Y)
+      const float k1 = XB_LN2 / (g * M::DC * M::EA);  // raw = ((g DC) D) . (EA Y)
       float4* dst = reinterpret_cast<float4*>(out1 + own_stat * LG_DH + part * OC);
 #pragma unroll
       for (int i = 0; i < OC / 4; ++i)
@@ -575,10 +661,57 @@ int lg_x3_attention_bwd(const float* Q, const float* K, const float* V, const fl
     LG_LAUNCH_CHECK();
     return LGB200_OK;
   };
-  if (np_cfg / 10 == 2) rc = launch(x3_attn_bwd_kernel<false, 2>, 2, Qp, Gp, tk, tv, dQ, nullptr);
-  else rc = launch(x3_attn_bwd_kernel<false, 4>, 4, Qp, Gp, tk, tv, dQ, nullptr);
+  if (np_cfg / 10 == 2) rc = launch(x3_attn_bwd_kernel<false, 2, false>, 2, Qp, Gp, tk, tv, dQ, nullptr);
+  else rc = launch(x3_attn_bwd_kernel<false, 4, false>, 4, Qp, Gp, tk, tv, dQ, nullptr);
   if (rc) return rc;
-  if (np_cfg % 10 == 2) rc = launch(x3_attn_bwd_kernel<true, 2>, 2, Kp, Vp, tq, tg, dK, dV);
-  else rc = launch(x3_attn_bwd_kernel<true, 4>, 4, Kp, Vp, tq, tg, dK, dV);
+  if (np_cfg % 10 == 2) rc = launch(x3_attn_bwd_kernel<true, 2, false>, 2, Kp, Vp, tq, tg, dK, dV);
+  else rc = launch(x3_attn_bwd_kernel<true, 4, false>, 4, Kp, Vp, tq, tg, dK, dV);
+  return rc;
+}
+
+size_t lg_bf16_attention_bwd_ws_floats(int S, int Lp) {
+  return 2 * (size_t)S * LG_HEADS * Lp + 16 + (size_t)S * Lp * LG_D / 2;
+}
+
+// Q, K, V bf16 [S,4,Lp,64] as the bf16 forward read them (rows >= lens finite); ctx bf16 [S,Lp,256] (the forward's
+// output), dctx fp32 [S,Lp,256]; dQ, dK, dV fp32 [S,4,Lp,64] (zero-filled by the caller);
+// ws: lg_bf16_attention_bwd_ws_floats(S, Lp) floats (row statistics | head-major bf16 dO).
+int lg_bf16_attention_bwd(const __nv_bfloat16* Q, const __nv_bfloat16* K, const __nv_bfloat16* V,
+                          const __nv_bfloat16* ctx, const float* dctx, int S, int Lp, const int32_t* lens, int kv_xor,
+                          float* dQ, float* dK, float* dV, float* ws, cudaStream_t st) {
+  const size_t n_stat = (size_t)S * LG_HEADS * Lp, n_el = (size_t)S * Lp * LG_D;
+  float* lse2 = ws;
+  float* dlt = ws + n_stat;
+  __nv_bfloat16* Gp = reinterpret_cast<__nv_bfloat16*>(ws + 2 * n_stat + 16);
+  xb_bf16_dout_kernel<<<(unsigned)((n_el / 8 + 255) / 256), 256, 0, st>>>(dctx, S, Lp, lens, Gp);
+  LG_LAUNCH_CHECK();
+
+  CUtensorMap tq, tk, tv, tg;
+  const uint64_t rows = (uint64_t)S * LG_HEADS * Lp;
+  const uint64_t d[3] = {64, rows, 1}, sb[2] = {128, rows * 128};
+  const uint32_t box[3] = {64, 64, 1};
+  int rc;
+  if ((rc = lg_make_tmap_bf16(&tq, Q, 3, d, sb, box))) return rc;
+  if ((rc = lg_make_tmap_bf16(&tk, K, 3, d, sb, box))) return rc;
+  if ((rc = lg_make_tmap_bf16(&tv, V, 3, d, sb, box))) return rc;
+  if ((rc = lg_make_tmap_bf16(&tg, Gp, 3, d, sb, box))) return rc;
+  // softmax threads per own row, per role (LGB200_BF16_BWD_NP = "<dq><dkv>", e.g. 24)
+  static const int np_cfg = getenv("LGB200_BF16_BWD_NP") ? atoi(getenv("LGB200_BF16_BWD_NP")) : 44;
+  const dim3 grid(Lp / 128, LG_HEADS, S);
+  auto h = [](const __nv_bfloat16* p) { return reinterpret_cast<const __half*>(p); };  // (2-byte rows, see the kernel)
+  auto launch = [&](auto kern, int np, const __nv_bfloat16* xp, const __nv_bfloat16* up, const CUtensorMap& ty,
+                    const CUtensorMap& tw, float* o1, float* o2) -> int {
+    cudaError_t le = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, XB_SMEM);
+    if (le != cudaSuccess) return (int)le;
+    kern<<<grid, 64 + 128 * np, XB_SMEM, st>>>(h(xp), h(up), 0, ty, tw, Lp, lens, kv_xor, ctx, dctx, nullptr, lse2, dlt,
+                                               o1, o2);
+    LG_LAUNCH_CHECK();
+    return LGB200_OK;
+  };
+  if (np_cfg / 10 == 2) rc = launch(x3_attn_bwd_kernel<false, 2, true>, 2, Q, Gp, tk, tv, dQ, nullptr);
+  else rc = launch(x3_attn_bwd_kernel<false, 4, true>, 4, Q, Gp, tk, tv, dQ, nullptr);
+  if (rc) return rc;
+  if (np_cfg % 10 == 2) rc = launch(x3_attn_bwd_kernel<true, 2, true>, 2, K, V, tq, tg, dK, dV);
+  else rc = launch(x3_attn_bwd_kernel<true, 4, true>, 4, K, V, tq, tg, dK, dV);
   return rc;
 }

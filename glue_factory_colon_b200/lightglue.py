@@ -148,6 +148,11 @@ class LightGlue(nn.Module):
         # with cuda_graph: return the graph's own output buffers (valid until the next call) instead of copies --
         # saves the 16.8 MB-per-pair copy of log_assignment at 2048 keypoints
         "graph_static_outputs": False,
+        # B200 extension: arithmetic of a training step (module in training mode, autograd on; the no-grad forward
+        # follows `precision`).  "fp32" = the fp32-accurate tensor-core mode; "bf16" = mixed precision: the bf16
+        # inference kernels forward (outputs bit-equal to the no-grad forward with precision="bf16"), bf16 tensor-core
+        # products with fp32 accumulation backward (train.py)
+        "train_precision": "fp32",
     }
 
     required_data_keys = ["keypoints0", "keypoints1", "descriptors0", "descriptors1"]
@@ -155,6 +160,7 @@ class LightGlue(nn.Module):
     def __init__(self, conf=None) -> None:
         super().__init__()
         self.conf = conf = _merge_conf(self.default_conf, conf)
+        self._train_bf16()  # (validates conf.train_precision)
         d = conf.descriptor_dim
         if d != 256 or conf.num_heads != 4:
             raise NotImplementedError("the B200 kernels are specialised for descriptor_dim=256, num_heads=4")
@@ -279,7 +285,7 @@ class LightGlue(nn.Module):
             check(lib.lgb200_assign_lse(prec, ptr(md), S, Lp, ptr(lens), ptr(lse), st), "assign_lse")
         R, C = m + 1, n + 1
         if keep is not None:  # what the backward pass (train.AssignFn) and the training forward need
-            keep.update(z=z, lse=lse, Lp=Lp, lens=lens, md_planes=md if x3 else None)
+            keep.update(z=z, lse=lse, Lp=Lp, lens=lens, md_planes=md if x3 else None, md16=md if bf else None)
         if bf:
             rows = torch.empty(3, B, m, **f32)
             row_arg = torch.empty(B, m, device=dev, dtype=torch.int32)
@@ -311,6 +317,45 @@ class LightGlue(nn.Module):
             lv = lg_.view(B, 2, Lp)
             logits = (lv[:, 0, :m], lv[:, 1, :n])
         return pos_sum, pos_cnt, row_exp, row_arg, col_arg, dust0, dust1, logits
+
+    def _assign_match_bf16(self, lib, d0, d1, layer: int):
+        """MatchAssignment `layer` and filter_matches on bf16 descriptors d0 [B,m,256] / d1 [B,n,256], with the kernels
+        and arguments of the no-grad bf16 forward's tail (_forward_impl) -> (log_assignment [B,m+1,n+1], m0, m1, ms0,
+        ms1).  The bf16 training forward's outputs are therefore the no-grad forward's, bit for bit."""
+        dev = d0.device
+        B, m, _ = d0.shape
+        n = d1.shape[1]
+        W = self._pack(BF16, dev)
+        st = torch.cuda.current_stream(dev).cuda_stream
+        S = 2 * B
+        Lp = max(128, ((max(m, n) + 127) // 128) * 128)
+        T = S * Lp
+        f32, b16 = dict(device=dev, dtype=torch.float32), dict(device=dev, dtype=torch.bfloat16)
+        lens = None if (m == Lp and n == Lp) else torch.tensor([m, n] * B, device=dev, dtype=torch.int32)
+        x = torch.zeros(T, 256, **b16)
+        for img, dsc, cnt in ((0, d0, m), (1, d1, n)):
+            check(lib.lgb200_pack_rows(ptr(dsc.to(torch.float32).contiguous()), B, cnt, 256, img, Lp, None, ptr(x), st),
+                  "pack_rows")
+        a = W["assign"][layer]
+        md = torch.zeros(T, 256, **b16)
+        check(lib.lgb200_linear(BF16, EPI_ROWMAJOR, ptr(x), None, 256, ptr(a["fp_w"]), ptr(a["fp_b"]), T, 256, 256,
+                                ptr(lens), Lp, 0.25, 1.0, 1.0, None, None, None, ptr(md), None, None, 0, None, None,
+                                None, None, None, st), "lgb200_linear")
+        z, lse = torch.zeros(T, **f32), torch.zeros(T, **f32)
+        check(lib.lgb200_rowdot(BF16, ptr(x), ptr(a["m_w"]), ptr(a["m_b"]), S, Lp, ptr(lens), 0, ptr(z), st), "rowdot")
+        check(lib.lgb200_assign_lse(BF16, ptr(md), S, Lp, ptr(lens), ptr(lse), st), "assign_lse")
+        R, C = m + 1, n + 1
+        scores = torch.empty(B, R, C, **f32)
+        fm_ws = torch.empty(B * (R + C), device=dev, dtype=torch.int64)
+        check(lib.lgb200_assign_scores(BF16, ptr(md), ptr(z), ptr(lse), B, Lp, ptr(lens), R, C, ptr(scores), ptr(fm_ws),
+                                       st), "assign_scores")
+        m0 = torch.empty(B, m, device=dev, dtype=torch.int64)
+        m1 = torch.empty(B, n, device=dev, dtype=torch.int64)
+        ms0, ms1 = torch.empty(B, m, **f32), torch.empty(B, n, **f32)
+        check(lib.lgb200_filter_matches(ptr(scores), B, R, C, ptr(lens), float(self.conf.filter_threshold), None, None,
+                                        2 * Lp, m, n, ptr(m0), ptr(m1), ptr(ms0), ptr(ms1), ptr(fm_ws), 1, st),
+              "filter_matches")
+        return scores, m0, m1, ms0, ms1
 
     @staticmethod
     def _reduce(lib, la, gt, st):
@@ -445,6 +490,12 @@ class LightGlue(nn.Module):
             raise ValueError(f"precision must be fp32, fp32_simt, bf16 or auto, got {p}")
         return {"bf16": BF16, "fp32": F32X3, "fp32_simt": F32}[p]
 
+    def _train_bf16(self) -> bool:
+        p = self.conf.get("train_precision", "fp32")
+        if p not in ("fp32", "bf16"):
+            raise ValueError(f"train_precision must be fp32 or bf16, got {p}")
+        return p == "bf16"
+
     def _apply(self, fn, *args, **kwargs):  # .to() / .cuda() / .half(): parameters may be replaced
         self._plist = None
         return super()._apply(fn, *args, **kwargs)
@@ -549,7 +600,8 @@ class LightGlue(nn.Module):
         `ref_descriptors0/1` carry an autograd graph to the descriptors and to every parameter
         (lightglue.py:484-498, :546-547).  conf.checkpointed (:485-494) selects recomputation of the attention
         operands in the backward pass instead of keeping them.  The matches / log_assignment of the last layer are
-        computed without a graph (the reference's loss reads pred["log_assignment"] detached, :606, :625-630)."""
+        computed without a graph (the reference's loss reads pred["log_assignment"] detached, :606, :625-630).
+        conf.train_precision = "bf16" runs train.TransformerBf16Fn and the bf16 assignment kernels instead."""
         from . import train as _train
 
         for key in self.required_data_keys:
@@ -588,8 +640,17 @@ class LightGlue(nn.Module):
         desc1 = data["descriptors1"].to(torch.float32)
         assert desc0.shape[-1] == conf.input_dim and desc1.shape[-1] == conf.input_dim
         params = [p for _, p in _train.transformer_params(self)]
-        r0, r1 = _train.TransformerFn.apply(self, geom, desc0, desc1, *params)
         L = conf.n_layers
+        if self._train_bf16():  # mixed precision: the bf16 inference kernels forward (conf.train_precision)
+            r0, r1 = _train.TransformerBf16Fn.apply(self, geom, desc0, desc1, *params)
+            with torch.no_grad():
+                scores, m0, m1, ms0, ms1 = self._assign_match_bf16(lib, r0[:, -1], r1[:, -1], L - 1)
+            return {
+                "matches0": m0, "matches1": m1, "matching_scores0": ms0, "matching_scores1": ms1,
+                "ref_descriptors0": r0, "ref_descriptors1": r1, "log_assignment": scores,
+                "prune0": torch.full((B, m), float(L), device=dev), "prune1": torch.full((B, n), float(L), device=dev),
+            }
+        r0, r1 = _train.TransformerFn.apply(self, geom, desc0, desc1, *params)
         with torch.no_grad():
             keep: Dict = {}
             # (fp32-accurate tensor-core kernels, as the rest of the training forward; CUDA cores with LGB200_TRAIN_SIMT_LINEAR=1)

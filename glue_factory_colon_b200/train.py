@@ -20,8 +20,18 @@ layer's descriptors in training mode, :588-637 turns them into the deep-supervis
 Plain GEMMs of the backward pass (dX = dY.W, dW = dY^T.X) go to cuBLAS -- they are library GEMMs with nothing to fuse --
 as three fp16 tensor-core GEMMs on split planes with fp32 accumulation (_Kern.mm3; LGB200_TRAIN_SGEMM=1: one fp32
 sgemm on the CUDA cores).  Gradients span a range (1e-8 ... 1e-2) that a fixed plane scaling does not cover, so
-lgb200_split_dynamic scales every gradient tensor by its own power of two first.  Everything is fp32-accurate whatever conf.precision says (the bf16 kernels are inference kernels); CPU tensors
-raise as everywhere else in this package.
+lgb200_split_dynamic scales every gradient tensor by its own power of two first.  That is the default,
+conf.train_precision = "fp32": fp32-accurate whatever conf.precision says.
+
+conf.train_precision = "bf16" (mixed precision, the counterpart of the reference under torch.autocast(bfloat16)):
+`TransformerBf16Fn` runs the bf16 inference kernels forward exactly as the no-grad forward with precision="bf16" does
+(bf16 weight pack with out_proj / to_out folded into the first FFN matrix, bf16 residual stream, rot16), so the training
+forward's outputs are bit-equal to it; the backward recomputes the pre-LayerNorm activations in fp32 from the bf16
+operands, runs lgb200_ln_gelu_bwd, the bf16 attention backward (lgb200_attention_bwd_bf16: one bf16 tcgen05 MMA per
+product) and lgb200_heads_bwd, and does every plain GEMM as ONE bf16 cuBLAS product with fp32 output.  Gradients of the
+folded weights follow by the chain rule (see _ffn_bwd16).  `AssignFn` uses the bf16 assignment kernels.
+
+CPU tensors raise as everywhere else in this package.
 """
 from __future__ import annotations
 
@@ -34,7 +44,7 @@ import torch
 from torch import nn
 
 from . import _abi
-from ._abi import EPI_HEADS, EPI_LN_GELU, EPI_ROWMAJOR, F32, F32X3, check, ptr
+from ._abi import BF16, EPI_HEADS, EPI_LN_GELU, EPI_ROWMAJOR, F32, F32X3, check, ptr
 
 LOG2E = 1.4426950408889634
 Q_SCALE = LOG2E / math.sqrt(64.0)   # folded into q: the attention kernels work in the log2 domain
@@ -171,6 +181,37 @@ class _Kern:
         ws = self.empty(n_ws.value)
         check(self.lib.lgb200_attention_bwd(ptr(q), ptr(k), ptr(v), ptr(ctx), ptr(dctx), self.S, self.Lp, ptr(self.lens),
                                             kv_xor, ptr(dq), ptr(dk), ptr(dv), ptr(ws), self.st), "lgb200_attention_bwd")
+        return dq, dk, dv
+
+    # ---- bf16 mixed-precision training (conf.train_precision = "bf16") ----
+
+    def zeros16(self, *shape):
+        return torch.zeros(*shape, device=self.dev, dtype=torch.bfloat16)
+
+    def linear16(self, epi, A0, W, b, N, K, A1=None, K0=None, scale=(1.0, 1.0, 1.0), resid=None, out=None, out32=None,
+                 rot16=None, n_rot=0, outp=(None, None, None), gamma=None, beta=None, lens=True):
+        """lgb200_linear(LGB200_BF16): bf16 A0 / A1 / W / resid / out / outp, fp32 out32; lens=False: no counts."""
+        check(self.lib.lgb200_linear(BF16, epi, ptr(A0), ptr(A1), K if K0 is None else K0, ptr(W), ptr(b), self.T, N, K,
+                                     ptr(self.lens) if lens else None, self.Lp, scale[0], scale[1], scale[2], None,
+                                     ptr(resid), ptr(out32), ptr(out), None, ptr(rot16), n_rot, ptr(outp[0]),
+                                     ptr(outp[1]), ptr(outp[2]), ptr(gamma), ptr(beta), self.st), "lgb200_linear (bf16)")
+
+    def attention16(self, q, k, v, kv_xor):
+        ctx = self.zeros16(self.T, 256)
+        check(self.lib.lgb200_attention(BF16, ptr(q), ptr(k), ptr(v), self.S, self.Lp, ptr(self.lens), kv_xor, ptr(ctx),
+                                        self.st), "lgb200_attention (bf16)")
+        return ctx
+
+    def attention_bwd16(self, q, k, v, ctx, dctx, kv_xor):
+        """lgb200_attention_bwd_bf16: bf16 q / k / v / ctx of the forward, fp32 dctx -> fp32 dq, dk, dv."""
+        dq, dk, dv = self.empty(self.T * 256), self.empty(self.T * 256), self.empty(self.T * 256)
+        n_ws = C.c_longlong(0)
+        check(self.lib.lgb200_attention_bwd_bf16_workspace(self.S, self.Lp, C.byref(n_ws)),
+              "lgb200_attention_bwd_bf16_workspace")
+        ws = self.empty(n_ws.value)
+        check(self.lib.lgb200_attention_bwd_bf16(ptr(q), ptr(k), ptr(v), ptr(ctx), ptr(dctx), self.S, self.Lp,
+                                                 ptr(self.lens), kv_xor, ptr(dq), ptr(dk), ptr(dv), ptr(ws), self.st),
+              "lgb200_attention_bwd_bf16")
         return dq, dk, dv
 
     def heads_bwd(self, dq, dk, dv, q, k, rot, n_parts, scales, dtheta):
@@ -461,6 +502,178 @@ class TransformerFn(torch.autograd.Function):
                 *[grads[key] if need[4 + j] else None for j, key in enumerate(ctx.keys)])
 
 
+# ---- bf16 mixed-precision training (conf.train_precision = "bf16") ------------------------------------------------
+
+
+def _mm16(a, b):
+    """a . b as one bf16 tensor-core GEMM with fp32 accumulation and fp32 output (cuBLAS)."""
+    return torch.mm(a.to(torch.bfloat16), b.to(torch.bfloat16), out_dtype=torch.float32)
+
+
+def _self_attend16(k: _Kern, w: Dict, x, rot16):
+    """Self block up to the context, as the no-grad bf16 forward runs it: (q, k, v, ctx), all bf16."""
+    q, kk, v = k.zeros16(k.T * 256), k.zeros16(k.T * 256), k.zeros16(k.T * 256)
+    k.linear16(EPI_HEADS, x, w["qkv_w"], w["qkv_b"], 768, 256, scale=(Q_SCALE, 1.0, 1.0), rot16=rot16, n_rot=2,
+               outp=(q, kk, v))
+    return q, kk, v, k.attention16(q, kk, v, 0)
+
+
+def _cross_attend16(k: _Kern, w: Dict, x, rot16):
+    qk, v = k.zeros16(k.T * 256), k.zeros16(k.T * 256)
+    k.linear16(EPI_HEADS, x, w["cqv_w"], w["cqv_b"], 512, 256, scale=(C_SCALE, 1.0, 1.0), rot16=rot16, n_rot=0,
+               outp=(qk, v, None))
+    return qk, v, k.attention16(qk, qk, v, 1)
+
+
+def _ffn16(k: _Kern, w: Dict, pre: str, x, c):
+    """x + ffn(cat[x, out_proj(c)]) with out_proj folded into the first FFN matrix (bf16 pack): a new bf16 tensor."""
+    hid = k.zeros16(k.T, 512)
+    k.linear16(EPI_LN_GELU, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=c, K0=256, gamma=w[pre + "ln_g"],
+               beta=w[pre + "ln_b"], out=hid)
+    out = x.clone()  # (the no-grad forward updates its residual stream in place; the block input is kept here)
+    k.linear16(EPI_ROWMAJOR, hid, w[pre + "f3_w"], w[pre + "f3_b"], 256, 512, resid=out, out=out)
+    return out
+
+
+def _ffn_bwd16(k: _Kern, w: Dict, pre: str, ffn0: nn.Linear, proj: nn.Linear, x, c, dy):
+    """Backward of y = x + ffn(cat[x, proj(c)]) in the bf16 forward's folded form h = [W1x | W1m.Wo].cat[x, c] +
+    (b1 + W1m.bo), given dy [T,256]: (d x through the ffn, d c, parameter gradients incl. those of proj).  With
+    G = dh^T c (the [512,256] block of d W1') and gb = sum dh: dW1m = G Wo^T + gb bo^T (W1m enters the folded bias
+    too), dWo = W1m^T G, dbo = W1m^T gb, db1 = gb."""
+    h = k.empty(k.T, 512)  # pre-LayerNorm activations, recomputed in fp32 from the same bf16 operands
+    k.linear16(EPI_ROWMAJOR, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=c, K0=256, out32=h)
+    dy16 = dy.to(torch.bfloat16)
+    da = _mm16(dy16, w[pre + "f3_w"])
+    dh, act, gsum = k.ln_gelu_bwd(h, w[pre + "ln_g"], w[pre + "ln_b"], da)
+    dh16 = dh.to(torch.bfloat16)
+    g3 = _mm16(dy16.t(), act)
+    gx, G = _mm16(dh16.t(), x), _mm16(dh16.t(), c)
+    dcat = _mm16(dh16, w[pre + "f0_w"])
+    gb = dh.sum(0)
+    d = proj.weight.shape[0]
+    w1m, wo, bo = ffn0.weight.detach()[:, d:], proj.weight.detach(), proj.bias.detach()
+    po = "so" if pre == "s" else "co"
+    g = {
+        pre + "f3_w": g3, pre + "f3_b": dy.sum(0),
+        pre + "ln_g": gsum[:512], pre + "ln_b": gsum[512:],
+        pre + "f0_w": torch.cat([gx, G @ wo.t() + torch.outer(gb, bo)], 1), pre + "f0_b": gb,
+        po + "_w": w1m.t() @ G, po + "_b": w1m.t() @ gb,
+    }
+    return dcat[:, :256], dcat[:, 256:].contiguous(), g
+
+
+def _proj_bwd16(dy, x, w16):
+    """Backward of y = x W^T + b with bf16 x / W: (dy^T x, dy^T 1, dy W)."""
+    dy16 = dy.to(torch.bfloat16)
+    return _mm16(dy16.t(), x), dy.sum(0), _mm16(dy16, w16)
+
+
+class TransformerBf16Fn(torch.autograd.Function):
+    """TransformerFn for conf.train_precision = "bf16": ref_descriptors0/1 (bf16, as the no-grad bf16 forward returns
+    them) with the bf16 inference kernels forward and bf16 tensor-core products backward."""
+
+    @staticmethod
+    def forward(ctx, model, geom: Dict, desc0, desc1, *params):
+        dev = desc0.device
+        B, m, _ = desc0.shape
+        n = desc1.shape[1]
+        k = _Kern(dev, B, m, n)
+        W = model._pack(BF16, dev)
+        L = model.conf.n_layers
+        xin = None
+        if isinstance(model.input_proj, nn.Linear):
+            din = model.conf.input_dim
+            xin = k.zeros16(k.T, din)
+            x = k.zeros16(k.T, 256)
+            for img, dsc, cnt in ((0, desc0, m), (1, desc1, n)):
+                check(k.lib.lgb200_pack_rows(ptr(dsc.contiguous()), B, cnt, din, img, k.Lp, None, ptr(xin), k.st),
+                      "lgb200_pack_rows")
+            k.linear16(EPI_ROWMAJOR, xin, W["in_w"], W["in_b"], 256, din, out=x, lens=False)
+        else:
+            x = k.zeros16(k.T, 256)
+            for img, dsc, cnt in ((0, desc0, m), (1, desc1, n)):
+                check(k.lib.lgb200_pack_rows(ptr(dsc.contiguous()), B, cnt, 256, img, k.Lp, None, ptr(x), k.st),
+                      "lgb200_pack_rows")
+        rot = k.zeros(k.T, 64)  # fp32 angles for lgb200_heads_bwd, rot16 for the forward's QKV epilogue (one call)
+        rot16 = torch.zeros(k.T, 32, device=dev, dtype=torch.int32)
+        kdim = geom["k0"].shape[-1]
+        for img, kk, cnt, sz in ((0, geom["k0"], m, geom["size0"]), (1, geom["k1"], n, geom["size1"])):
+            check(k.lib.lgb200_posenc(ptr(kk), B, cnt, kdim, ptr(sz), ptr(W["wr"]), ptr(k.lens), img, k.Lp, ptr(rot),
+                                      ptr(rot16), k.st), "lgb200_posenc")
+        keep = not bool(model.conf.checkpointed)
+        xs_in, xs_mid, outs, kept = [], [], [], []
+        for i in range(L):
+            w = W["layers"][i]
+            xs_in.append(x)
+            sa = _self_attend16(k, w, x, rot16)
+            x = _ffn16(k, w, "s", x, sa[-1])
+            xs_mid.append(x)
+            ca = _cross_attend16(k, w, x, rot16)
+            x = _ffn16(k, w, "c", x, ca[-1])
+            outs.append(x)
+            kept.append((sa, ca) if keep else None)
+        ctx.k, ctx.W, ctx.geom, ctx.model = k, W, geom, model
+        ctx.xs_in, ctx.xs_mid, ctx.rot, ctx.rot16, ctx.xin, ctx.kept = xs_in, xs_mid, rot, rot16, xin, kept
+        ctx.keys = [key for key, _ in transformer_params(model)]
+        r0 = torch.stack([k.unpack(o)[0] for o in outs], 1)
+        r1 = torch.stack([k.unpack(o)[1] for o in outs], 1)
+        return r0, r1
+
+    @staticmethod
+    def backward(ctx, g0, g1):
+        k, W, geom, model = ctx.k, ctx.W, ctx.geom, ctx.model
+        L = len(ctx.xs_in)
+        rot, rot16 = ctx.rot, ctx.rot16
+        dx = k.zeros(k.T, 256)
+        dtheta = k.zeros(k.T, 32)
+        grads: Dict[object, torch.Tensor] = {}
+        perm = _PERM.to(dx.device)
+        for i in reversed(range(L)):
+            w = W["layers"][i]
+            sa_m, ca_m = model.transformers[i].self_attn, model.transformers[i].cross_attn
+            dx = dx + k.pack2(g0[:, i], g1[:, i])
+            x_in, x_mid = ctx.xs_in[i], ctx.xs_mid[i]
+            # ---- cross block (lightglue.py:193-222) ----
+            qk, v, c = ctx.kept[i][1] if ctx.kept[i] is not None else _cross_attend16(k, w, x_mid, rot16)
+            dxa, dc, g = _ffn_bwd16(k, w, "c", ca_m.ffn[0], ca_m.to_out, x_mid, c, dx)
+            for name, val in g.items():
+                grads[(i, name)] = val
+            dq, dk, dv = k.attention_bwd16(qk, qk, v, c, dc, 1)
+            dqv = k.heads_bwd(dq, dk, dv, None, None, None, 2, (C_SCALE, 1.0, 1.0), None)
+            gw, gb, dxp = _proj_bwd16(dqv, x_mid, w["cqv_w"])
+            grads[(i, "cqk_w")], grads[(i, "cv_w")] = gw[:256], gw[256:]
+            grads[(i, "cqk_b")], grads[(i, "cv_b")] = gb[:256], gb[256:]
+            dxm = dx + dxa + dxp
+            # ---- self block (lightglue.py:151-164) ----
+            q, kk, v, c = ctx.kept[i][0] if ctx.kept[i] is not None else _self_attend16(k, w, x_in, rot16)
+            ctx.kept[i] = None
+            dxa, dc, g = _ffn_bwd16(k, w, "s", sa_m.ffn[0], sa_m.out_proj, x_in, c, dxm)
+            for name, val in g.items():
+                grads[(i, name)] = val
+            dq, dk, dv = k.attention_bwd16(q, kk, v, c, dc, 0)
+            dqkv = k.heads_bwd(dq, dk, dv, q.float(), kk.float(), rot, 3, (Q_SCALE, 1.0, 1.0), dtheta)
+            gw = torch.empty(768, 256, device=dqkv.device, dtype=torch.float32)
+            gb = torch.empty(768, device=dqkv.device, dtype=torch.float32)
+            gw[perm], gb[perm], dxp = _proj_bwd16(dqkv, x_in, w["qkv_w"])
+            grads[(i, "qkv_w")], grads[(i, "qkv_b")] = gw, gb
+            dx = dxm + dxa + dxp
+        # positional encoding: theta = Wr . normalised keypoints (lightglue.py:61-66)
+        kdim = geom["k0"].shape[-1]
+        kn = k.zeros(k.T, kdim)
+        knv = kn.view(k.B, 2, k.Lp, kdim)
+        for img, kk, sz, cnt in ((0, geom["k0"], geom["size0"], k.m), (1, geom["k1"], geom["size1"], k.n)):
+            knv[:, img, :cnt, :2] = normalize_keypoints(kk[..., :2], sz)
+            knv[:, img, :cnt, 2:] = kk[..., 2:]
+        grads["wr"] = dtheta.t() @ kn
+        if ctx.xin is not None:  # input_proj (lightglue.py:464-465)
+            grads["in_w"], grads["in_b"] = dx.t() @ ctx.xin.float(), dx.sum(0)
+            dx = dx @ model.input_proj.weight.detach()
+        gd0, gd1 = k.unpack(dx)
+        need = ctx.needs_input_grad
+        return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None,
+                *[grads[key] if need[4 + j] else None for j, key in enumerate(ctx.keys)])
+
+
 class AssignFn(torch.autograd.Function):
     """MatchAssignment `layer` on (d0, d1) reduced to the inputs of NLLLoss: pos_sum [B] = sum of log_assignment over
     the ground-truth matches, dust0 [B,m] / dust1 [B,n] = the dustbin column / row (differentiable); pos_cnt, row_exp,
@@ -470,13 +683,16 @@ class AssignFn(torch.autograd.Function):
     def forward(ctx, model, layer: int, gt, d0, d1, fp_w, fp_b, m_w, m_b):
         lib = _abi.load()
         keep: Dict = {}
+        bf = model._train_bf16()
+        prec = BF16 if bf else (F32 if _SIMT_LINEAR else F32X3)
         pos_sum, pos_cnt, row_exp, row_arg, col_arg, dust0, dust1, _ = model._log_assignment_of(
-            lib, F32 if _SIMT_LINEAR else F32X3, d0, d1, layer, gt, keep=keep)
+            lib, prec, d0, d1, layer, gt, keep=keep)
         ctx.save_for_backward(d0, d1, fp_w, fp_b, m_w, gt, keep["z"], keep["lse"])
         ctx.Lp = keep["Lp"]
         # x3 mode: the split planes of final_proj(desc) / 4 (33 MB at 8 x 2048) -- the backward recomputes the similarity
         # from them on tcgen05 instead of redoing final_proj and the N x M product in fp32 on the CUDA cores
-        ctx.md_planes, ctx.lens = (None, None) if _SGEMM else (keep["md_planes"], keep["lens"])
+        ctx.md_planes, ctx.lens = (None, None) if (_SGEMM or bf) else (keep["md_planes"], keep["lens"])
+        ctx.md16 = keep["md16"] if bf else None  # bf16: final_proj(desc) / 4 as the forward's kernels computed it
         ctx.mark_non_differentiable(pos_cnt, row_exp, row_arg, col_arg)
         return pos_sum, dust0.contiguous(), dust1.contiguous(), pos_cnt, row_exp, row_arg, col_arg
 
@@ -490,8 +706,13 @@ class AssignFn(torch.autograd.Function):
         dev = d0.device
         x0, x1 = d0.to(torch.float32), d1.to(torch.float32)
         st = torch.cuda.current_stream(dev).cuda_stream
-        mdp = ctx.md_planes
-        if mdp is None:
+        mdp, md16 = ctx.md_planes, ctx.md16
+        f32 = torch.float32
+        if md16 is not None:  # bf16: the similarity as one bf16 bmm with fp32 output (bf16 output: ~0.1 at |sim| ~ 30)
+            mv = md16.view(B, 2, Lp, 256)
+            md0, md1 = mv[:, 0, :m], mv[:, 1, :n]
+            sim = torch.bmm(md0, md1.transpose(1, 2), out_dtype=f32).contiguous()
+        elif mdp is None:
             md0 = torch.addmm(fp_b, x0.reshape(-1, 256), fp_w.t()).view(B, m, 256) * 0.25  # lightglue.py:281-283
             md1 = torch.addmm(fp_b, x1.reshape(-1, 256), fp_w.t()).view(B, n, 256) * 0.25
             sim = torch.bmm(md0, md1.transpose(1, 2)).contiguous()
@@ -503,7 +724,11 @@ class AssignFn(torch.autograd.Function):
         r = (g[:, None] * gt.sum(2)).contiguous()
         c = (g[:, None] * gt.sum(1)).contiguous()
         check(lib.lgb200_assign_dsim(ptr(sim), B, m, n, ptr(lse), Lp, ptr(gt), ptr(g), ptr(r), ptr(c), st), "assign_dsim")
-        if mdp is None:
+        if md16 is not None:
+            s16 = sim.to(torch.bfloat16)
+            dmd0 = torch.bmm(s16, md1, out_dtype=f32)
+            dmd1 = torch.bmm(s16.transpose(1, 2), md0, out_dtype=f32)
+        elif mdp is None:
             dmd0 = torch.bmm(sim, md1)
             dmd1 = torch.bmm(sim.transpose(1, 2), md0)
         else:  # three fp16 tensor-core products per GEMM, as _Kern.mm3
@@ -512,7 +737,6 @@ class AssignFn(torch.autograd.Function):
             check(lib.lgb200_split_dynamic(ptr(sim), sim.numel(), ptr(sp), ptr(inv), 0, None, 0, st), "lgb200_split_dynamic")
             mv = mdp.view(2, B, 2, Lp, 256)
             mp0, mp1 = mv[:, :, 0, :m], mv[:, :, 1, :n]
-            f32 = torch.float32
 
             def bmm3(A, Bm):
                 o = torch.bmm(A[1], Bm[0], out_dtype=f32)

@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define LGB200_ABI_VERSION 6
+#define LGB200_ABI_VERSION 7
 
 enum { LGB200_F32 = 0, LGB200_BF16 = 1, LGB200_F32X3 = 2 };
 
@@ -316,6 +316,17 @@ int lgb200_attention_bwd(const float* Q, const float* K, const float* V, const f
                          int S, int Lp, const int32_t* lens, int kv_xor, float* dQ, float* dK, float* dV,
                          float* workspace, void* stream);
 int lgb200_attention_bwd_workspace(int S, int Lp, long long* n_floats);
+/* lgb200_attention_bwd_bf16: backward of lgb200_attention(LGB200_BF16, ...) on what that forward read and wrote --
+ *   Q, K, V bf16 [S,4,Lp,64] (Q pre-scaled into the log2 domain; rows >= lens must be finite, as for the forward),
+ *   ctx bf16 [S,Lp,256] = the forward's output, dctx fp32 [S,Lp,256] = its gradient.  dQ, dK, dV fp32 [S,4,Lp,64] as
+ *   for lgb200_attention_bwd (the layout lgb200_heads_bwd reads); rows >= lens are zero.  tcgen05, one bf16 MMA per
+ *   product with fp32 accumulation; <dO, O> is formed in fp32.  workspace: lgb200_attention_bwd_bf16_workspace(S, Lp)
+ *   floats (row log-sum-exp, <dO, O>, and dO as head-major bf16).
+ * lgb200_attention_bwd_bf16_workspace: *n_floats = the workspace size of lgb200_attention_bwd_bf16 for (S, Lp). */
+int lgb200_attention_bwd_bf16(const void* Q, const void* K, const void* V, const void* ctx, const float* dctx,
+                              int S, int Lp, const int32_t* lens, int kv_xor, float* dQ, float* dK, float* dV,
+                              float* workspace, void* stream);
+int lgb200_attention_bwd_bf16_workspace(int S, int Lp, long long* n_floats);
 int lgb200_heads_bwd(const float* dQ, const float* dK, const float* dV, const float* Q, const float* K,
                      const float* rot, int S, int Lp, const int32_t* lens, int n_parts, float scale0,
                      float scale1, float scale2, float* out, float* dtheta, void* stream);

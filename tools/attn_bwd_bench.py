@@ -1,6 +1,9 @@
-"""Attention backward kernels alone (csrc/lg_bwd.cu through lgb200_attention_bwd): S sequences x 4 heads x Lp keypoints,
-fp32.  Prints ms per call and the useful fp32-equivalent TFLOP/s (8 tile products of 2.Lp^2.64 per head: 1 statistics +
-3 dQ + 4 dK/dV).  Usage: python tools/attn_bwd_bench.py [S] [Lp] [reps]   (LGB200_ATTN_BWD_SIMT=1: CUDA-core kernels)"""
+"""Attention backward kernels alone: S sequences x 4 heads x Lp keypoints.  Two arms, timed alternately on the same
+inputs: the fp32 entry lgb200_attention_bwd (csrc/lg_bwd.cu -> the x3 tcgen05 kernel) and the bf16 entry
+lgb200_attention_bwd_bf16 (the same kernel template on bf16 operands, fed by the bf16 forward).  Prints ms per call and
+the useful TFLOP/s on one product count for both (8 tile products of 2.Lp^2.64 per head: 1 statistics + 3 dQ +
+4 dK/dV), and the card's name and power limit.  Usage: python tools/attn_bwd_bench.py [S] [Lp] [reps]
+(LGB200_ATTN_BWD_SIMT=1: CUDA-core kernels in the fp32 arm)"""
 import ctypes
 import sys
 from pathlib import Path
@@ -29,22 +32,57 @@ assert lib.lgb200_attention_bwd_workspace(S, Lp, ctypes.byref(n_ws)) == 0
 ws = torch.empty(n_ws.value, device=dev)
 
 
-def call():
+q16, k16, v16 = (t.to(torch.bfloat16) for t in (q, k, v))
+ctx16 = torch.zeros(S, Lp, 256, device=dev, dtype=torch.bfloat16)
+assert lib.lgb200_attention(_abi.BF16, ptr(q16), ptr(k16), ptr(v16), S, Lp, None, 0, ptr(ctx16), st) == 0
+assert lib.lgb200_attention_bwd_bf16_workspace(S, Lp, ctypes.byref(n_ws)) == 0
+ws16 = torch.empty(n_ws.value, device=dev)
+dq16, dk16, dv16 = (torch.empty(S, 4, Lp, 64, device=dev) for _ in range(3))
+
+
+def call_x3():
     rc = lib.lgb200_attention_bwd(ptr(q), ptr(k), ptr(v), ptr(ctx), ptr(dctx), S, Lp, None, 0, ptr(dq), ptr(dk), ptr(dv),
                                   ptr(ws), st)
     assert rc == 0
 
 
-for _ in range(2):
-    call()
+def call_bf16():
+    rc = lib.lgb200_attention_bwd_bf16(ptr(q16), ptr(k16), ptr(v16), ptr(ctx16), ptr(dctx), S, Lp, None, 0, ptr(dq16),
+                                       ptr(dk16), ptr(dv16), ptr(ws16), st)
+    assert rc == 0
+
+
+def timed(call):
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(REPS):
+        call()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / REPS
+
+
+arms = {"x3 (fp32-accurate, three fp16 MMAs per product)": call_x3, "bf16 (one bf16 MMA per product)": call_bf16}
+for call in arms.values():
+    for _ in range(2):
+        call()
 torch.cuda.synchronize()
-e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-e0.record()
-for _ in range(REPS):
-    call()
-e1.record()
-torch.cuda.synchronize()
-ms = e0.elapsed_time(e1) / REPS
+times = {name: [] for name in arms}
+for _ in range(3):  # alternating rounds
+    for name, call in arms.items():
+        times[name].append(timed(call))
 flop = 8 * 2.0 * Lp * Lp * 64 * 4 * S
-print(f"attention backward S={S} Lp={Lp}: {ms:.3f} ms per call, {flop / ms / 1e9:.1f} TFLOP/s useful (fp32-equivalent), "
-      f"checksum {float(dq.abs().mean()):.6f} {float(dk.abs().mean()):.6f} {float(dv.abs().mean()):.6f}")
+card = torch.cuda.get_device_name(dev)
+try:
+    import subprocess
+
+    plim = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
+                          capture_output=True, text=True).stdout.strip()
+except OSError:
+    plim = "unknown"
+for name, ts in times.items():
+    ms = min(ts)
+    print(f"attention backward {name} S={S} Lp={Lp}: {ms:.3f} ms per call (rounds {', '.join(f'{t:.3f}' for t in ts)}), "
+          f"{flop / ms / 1e9:.1f} TFLOP/s useful; {card}, power limit {plim}")
+rel = lambda a, b: float((a - b).norm() / b.norm())  # noqa: E731
+print(f"bf16 vs x3 arm, norm-wise: dq {rel(dq16, dq):.2e} dk {rel(dk16, dk):.2e} dv {rel(dv16, dv):.2e}")
