@@ -13,7 +13,7 @@ LIB_PATH = Path(__file__).resolve().parent / "lib" / "liblightglue_b200.so"
 
 F32, BF16, F32X3 = 0, 1, 2
 EPI_ROWMAJOR, EPI_HEADS, EPI_LN_GELU = 0, 1, 2
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 _p, _i, _f = C.c_void_p, C.c_int, C.c_float
 
@@ -35,6 +35,7 @@ SIGNATURES = {
     "lgb200_nn_match": [_p, _i, _i, _i, _p, _f, _f, _i, _p, _p, _p, _p, _p, _p],
     "lgb200_npair_loss": [_p, _p, _i, _i, _i, _f, _p, _p, _p, _p],
     "lgb200_loss_reduce": [_p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p],
+    "lgb200_loss_reduce_ragged": [_p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],
     "lgb200_assign_loss": [_i, _p, _p, _p, _i, _i, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],
     "lgb200_exit_check": [_p, _i, _i, _p, _p, _f, _f, _i, _p, _p, _p],
     "lgb200_split_rows": [_p, C.c_longlong, _p, _p],
@@ -50,6 +51,7 @@ SIGNATURES = {
     "lgb200_heads_bwd": [_p, _p, _p, _p, _p, _p, _i, _i, _p, _i, _f, _f, _f, _p, _p, _p],
     "lgb200_ln_gelu_bwd": [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _p],
     "lgb200_assign_dsim": [_p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p],
+    "lgb200_assign_dsim_ragged": [_p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p, _p],
     "lgb200_prune_compact": [_p, _p, _f, _f, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
 }
 

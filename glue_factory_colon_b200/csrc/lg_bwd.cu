@@ -13,7 +13,7 @@
 //   heads_bwd_kernel        head-major dq/dk/dv -> token-major d(qkv) incl. the transposed rotary embedding and the
 //                           gradient of the rotary angles (-> posenc.Wr)                   lightglue.py:43-50, 157-161
 //   ln_gelu_bwd_kernel      GELU(erf)' . LayerNorm backward, d gamma / d beta partials     lightglue.py:144-149
-//   assign_dsim_kernel      d sim of sigmoid_log_double_softmax                            lightglue.py:257-269
+//   assign_dsim_kernel      d sim of sigmoid_log_double_softmax (optionally per-pair counts) lightglue.py:257-269
 #include "lg_common.cuh"
 #include "lg_internal.cuh"
 #include <stdlib.h>
@@ -636,14 +636,21 @@ __global__ void __launch_bounds__(256) ln_gelu_bwd_kernel(const float* __restric
 
 // sim [B,m,n] -> d sim in place: 2 g gt - r_i exp(sim - lse0_i) - c_j exp(sim - lse1_j)   (g = d loss / d pos_sum[b],
 // r / c = g times the row / column sums of gt; lse from lgb200_assign_lse: rows of image 0, columns of image 1)
+// lens (nullable): per-pair counts -- entries outside pair b's valid block (i >= lens[2b] or j >= lens[2b+1]) become 0
+// and neither gt nor r / c nor lse is read there
 __global__ void __launch_bounds__(256) assign_dsim_kernel(float* __restrict__ sim, int m, int n,
                                                           const float* __restrict__ lse, int Lp,
+                                                          const int32_t* __restrict__ lens,
                                                           const uint8_t* __restrict__ gt, const float* __restrict__ g_pos,
                                                           const float* __restrict__ r, const float* __restrict__ c) {
   const int b = blockIdx.z, i = blockIdx.y;
   const int j = blockIdx.x * 256 + threadIdx.x;
   if (j >= n) return;
   const size_t off = ((size_t)b * m + i) * n + j;
+  if (lens && (i >= lens[2 * b] || j >= lens[2 * b + 1])) {
+    sim[off] = 0.f;
+    return;
+  }
   const float sv = sim[off];
   const float l0 = lse[(size_t)(2 * b) * Lp + i], l1 = lse[(size_t)(2 * b + 1) * Lp + j];
   const float g = gt[off] ? 2.f * g_pos[b] : 0.f;
@@ -748,7 +755,18 @@ extern "C" int lgb200_assign_dsim(float* sim, int B, int m, int n, const float* 
   if (!sim || !lse || !gt_assignment || !g_pos || !r || !c) return LGB200_ERR_NULL;
   if (B <= 0 || m <= 0 || n <= 0 || m > Lp || n > Lp || m > 65535) return LGB200_ERR_SHAPE;
   dim3 grid((n + 255) / 256, m, B);
-  assign_dsim_kernel<<<grid, 256, 0, lg_stream(stream)>>>(sim, m, n, lse, Lp, gt_assignment, g_pos, r, c);
+  assign_dsim_kernel<<<grid, 256, 0, lg_stream(stream)>>>(sim, m, n, lse, Lp, nullptr, gt_assignment, g_pos, r, c);
+  LG_LAUNCH_CHECK();
+  return LGB200_OK;
+}
+
+extern "C" int lgb200_assign_dsim_ragged(float* sim, int B, int m, int n, const float* lse, int Lp,
+                                         const int32_t* lens, const uint8_t* gt_assignment, const float* g_pos,
+                                         const float* r, const float* c, void* stream) {
+  if (!sim || !lse || !lens || !gt_assignment || !g_pos || !r || !c) return LGB200_ERR_NULL;
+  if (B <= 0 || m <= 0 || n <= 0 || m > Lp || n > Lp || m > 65535) return LGB200_ERR_SHAPE;
+  dim3 grid((n + 255) / 256, m, B);
+  assign_dsim_kernel<<<grid, 256, 0, lg_stream(stream)>>>(sim, m, n, lse, Lp, lens, gt_assignment, g_pos, r, c);
   LG_LAUNCH_CHECK();
   return LGB200_OK;
 }

@@ -408,12 +408,17 @@ tc_assign_kernel(const __grid_constant__ CUtensorMap tmMd, const __grid_constant
 
 // LOSS: arg-maxima including the dustbins from the packed inner maxima, and the dustbin column's share of row_exp.
 // torch.max tie rule: the dustbin has the highest index, so it wins only if strictly larger (or the first NaN).
+// Rows / columns past pair b's counts (lens) keep row_exp = 0 and get arg-maximum -1, as lgb200_loss_reduce_ragged.
 __global__ void assign_loss_finish_kernel(const float* __restrict__ z, int Lp, int R, int C,
+                                          const int32_t* __restrict__ lens,
                                           const unsigned long long* __restrict__ best0,
                                           const unsigned long long* __restrict__ best1, float* __restrict__ row_exp,
                                           int32_t* __restrict__ row_arg, int32_t* __restrict__ col_arg) {
   const int b = blockIdx.y, t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t < R - 1) {
+  const int n0 = lens ? lens[2 * b] : R - 1, n1 = lens ? lens[2 * b + 1] : C - 1;
+  if (t < R - 1 && t >= n0) {
+    if (row_arg) row_arg[(size_t)b * (R - 1) + t] = -1;
+  } else if (t < R - 1) {
     const float dz = lg_logsigmoid(-z[(size_t)(2 * b) * Lp + t]);
     const unsigned long long p = best0[(size_t)b * R + t];
     const float v = fm_value(p);
@@ -421,7 +426,9 @@ __global__ void assign_loss_finish_kernel(const float* __restrict__ z, int Lp, i
     if (row_arg) row_arg[(size_t)b * (R - 1) + t] = inner ? fm_index(p) : C - 1;
     if (row_exp) row_exp[(size_t)b * (R - 1) + t] += __expf(dz);
   }
-  if (t < C - 1 && col_arg) {
+  if (t < C - 1 && col_arg && t >= n1) {
+    col_arg[(size_t)b * (C - 1) + t] = -1;
+  } else if (t < C - 1 && col_arg) {
     const float dz = lg_logsigmoid(-z[(size_t)(2 * b + 1) * Lp + t]);
     const unsigned long long p = best1[(size_t)b * C + t];
     const float v = fm_value(p);
@@ -550,8 +557,8 @@ int lg_tc_assign_loss(const __nv_bfloat16* md, const float* z, const float* lse,
   }
   const int nmax = (R > C ? R : C) - 1;
   if (nmax > 0) {
-    assign_loss_finish_kernel<<<dim3((nmax + 255) / 256, B), 256, 0, st>>>(z, Lp, R, C, best0, best1, row_exp, row_arg,
-                                                                          col_arg);
+    assign_loss_finish_kernel<<<dim3((nmax + 255) / 256, B), 256, 0, st>>>(z, Lp, R, C, lens, best0, best1, row_exp,
+                                                                          row_arg, col_arg);
     LG_LAUNCH_CHECK();
   }
   return LGB200_OK;

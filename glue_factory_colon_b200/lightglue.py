@@ -227,13 +227,16 @@ class LightGlue(nn.Module):
     # ---- loss (forward values; SURVEY.md 8(f) rank 2) ------------------------------------------
 
     def _log_assignment_of(self, lib, prec, d0, d1, layer: int, gt, token_layer: Optional[int] = None,
-                           keep: Optional[dict] = None):
+                           keep: Optional[dict] = None, counts: Optional[torch.Tensor] = None):
         """MatchAssignment `layer` applied to descriptors d0 [B,m,256] / d1 [B,n,256] (lightglue.py:279-288 as called
         from loss_params, :589-595) and the loss reductions on its output.  fp32 (CUDA cores) / fp32-accurate tensor-core
         mode (F32X3: split-fp16 final_proj and similarity GEMM): the forward's assignment kernels write scores
         [B,m+1,n+1], lgb200_loss_reduce reads them.  bf16: lgb200_assign_loss, the tcgen05 pass 2 with the
         reductions in its epilogue -- the matrix is never written.  Returns (pos_sum, pos_cnt, row_exp, row_arg,
-        col_arg, dustbin column la[:, :m, n], dustbin row la[:, m, :n], token logits of `token_layer` or None)."""
+        col_arg, dustbin column la[:, :m, n], dustbin row la[:, m, :n], token logits of `token_layer` or None).
+        counts (device int32 [2B] or None): per-pair valid counts of a padded batch; the staged rows past them are
+        zeroed, log_assignment takes the inference layout of such a batch and every reduction covers each pair's valid
+        block only (lgb200_loss_reduce_ragged)."""
         bf = prec == BF16
         x3 = prec == F32X3  # fp32-accurate tensor-core mode: split-fp16 final_proj + similarity GEMM, fp32 normalisers
         hprec = F32 if x3 else prec  # the per-token heads read the fp32 rows in x3 mode
@@ -248,14 +251,16 @@ class LightGlue(nn.Module):
         T = S * Lp
         f32 = dict(device=dev, dtype=torch.float32)
         adt = dict(device=dev, dtype=torch.bfloat16 if bf else torch.float32)
-        lens = None
-        if m != Lp or n != Lp:
+        lens = counts
+        if counts is None and (m != Lp or n != Lp):
             lens = torch.tensor([m, n] * B, device=dev, dtype=torch.int32)
         x = torch.zeros(T, 256, **adt)
         for img, dsc, cnt in ((0, d0, m), (1, d1, n)):
             dsc = dsc.to(torch.float32).contiguous()
             x32_, x16_ = (None, x) if bf else (x, None)
             check(lib.lgb200_pack_rows(ptr(dsc), B, cnt, 256, img, Lp, ptr(x32_), ptr(x16_), st), "pack_rows")
+        if counts is not None:
+            x.masked_fill_((torch.arange(Lp, device=dev)[None] >= counts[:, None]).reshape(-1, 1), 0)
         a = W["assign"][layer]
         if x3:
             xs = torch.empty(2, T, 256, device=dev, dtype=torch.float16)
@@ -305,7 +310,7 @@ class LightGlue(nn.Module):
             else:
                 check(lib.lgb200_assign_scores(prec, ptr(md), ptr(z), ptr(lse), B, Lp, ptr(lens), R, C, ptr(scores), None,
                                                st), "assign_scores")
-            pos_sum, pos_cnt, row_exp, row_arg, col_arg = self._reduce(lib, scores, gt, st)
+            pos_sum, pos_cnt, row_exp, row_arg, col_arg = self._reduce(lib, scores, gt, st, counts)
             dust0, dust1 = scores[:, :m, n], scores[:, m, :n]
             if keep is not None:
                 keep["scores"] = scores
@@ -318,10 +323,11 @@ class LightGlue(nn.Module):
             logits = (lv[:, 0, :m], lv[:, 1, :n])
         return pos_sum, pos_cnt, row_exp, row_arg, col_arg, dust0, dust1, logits
 
-    def _assign_match_bf16(self, lib, d0, d1, layer: int):
+    def _assign_match_bf16(self, lib, d0, d1, layer: int, counts: Optional[torch.Tensor] = None):
         """MatchAssignment `layer` and filter_matches on bf16 descriptors d0 [B,m,256] / d1 [B,n,256], with the kernels
         and arguments of the no-grad bf16 forward's tail (_forward_impl) -> (log_assignment [B,m+1,n+1], m0, m1, ms0,
-        ms1).  The bf16 training forward's outputs are therefore the no-grad forward's, bit for bit."""
+        ms1).  The bf16 training forward's outputs are therefore the no-grad forward's, bit for bit.  counts: per-pair
+        valid counts (device int32 [2B]) or None."""
         dev = d0.device
         B, m, _ = d0.shape
         n = d1.shape[1]
@@ -331,7 +337,9 @@ class LightGlue(nn.Module):
         Lp = max(128, ((max(m, n) + 127) // 128) * 128)
         T = S * Lp
         f32, b16 = dict(device=dev, dtype=torch.float32), dict(device=dev, dtype=torch.bfloat16)
-        lens = None if (m == Lp and n == Lp) else torch.tensor([m, n] * B, device=dev, dtype=torch.int32)
+        lens = counts
+        if counts is None and (m != Lp or n != Lp):
+            lens = torch.tensor([m, n] * B, device=dev, dtype=torch.int32)
         x = torch.zeros(T, 256, **b16)
         for img, dsc, cnt in ((0, d0, m), (1, d1, n)):
             check(lib.lgb200_pack_rows(ptr(dsc.to(torch.float32).contiguous()), B, cnt, 256, img, Lp, None, ptr(x), st),
@@ -358,17 +366,40 @@ class LightGlue(nn.Module):
         return scores, m0, m1, ms0, ms1
 
     @staticmethod
-    def _reduce(lib, la, gt, st):
+    def _reduce(lib, la, gt, st, counts=None):
         """lgb200_loss_reduce on one log-assignment matrix: per-row positive sums / counts / exp sums and the
-        row / column arg-maxima including the dustbins."""
+        row / column arg-maxima including the dustbins.  counts (device int32 [2B]): lgb200_loss_reduce_ragged, each
+        pair over its valid block."""
         B, R, C = la.shape
         dev = la.device
         rows = torch.zeros(3, B, R - 1, device=dev, dtype=torch.float32)
         row_arg = torch.zeros(B, R - 1, device=dev, dtype=torch.int32)
         col_arg = torch.zeros(B, C - 1, device=dev, dtype=torch.int32)
-        check(lib.lgb200_loss_reduce(ptr(la), B, R, C, ptr(gt), ptr(rows[0]), ptr(rows[1]), ptr(rows[2]), ptr(row_arg),
-                                     ptr(col_arg), st), "loss_reduce")
+        if counts is None:
+            check(lib.lgb200_loss_reduce(ptr(la), B, R, C, ptr(gt), ptr(rows[0]), ptr(rows[1]), ptr(rows[2]),
+                                         ptr(row_arg), ptr(col_arg), st), "loss_reduce")
+        else:
+            check(lib.lgb200_loss_reduce_ragged(ptr(la), B, R, C, ptr(counts), ptr(gt), ptr(rows[0]), ptr(rows[1]),
+                                                ptr(rows[2]), ptr(row_arg), ptr(col_arg), st), "loss_reduce_ragged")
         return rows[0].sum(1), rows[1].sum(1), rows[2], row_arg, col_arg
+
+    @staticmethod
+    def _counts_of(data: dict, B: int, m: int, n: int) -> Optional[np.ndarray]:
+        """Per-pair valid counts [B, 2] (host int32) from data["num_keypoints0/1"] (the B200 extension for padded
+        batches, SURVEY.md 8(c)), or None without them -- and when every count equals the padded size, so that such a
+        batch takes exactly the path of a batch without counts."""
+        lens_host = np.empty((B, 2), dtype=np.int32)
+        lens_host[:, 0], lens_host[:, 1] = m, n
+        variable = False
+        for idx in (0, 1):
+            cnt = data.get(f"num_keypoints{idx}")
+            if cnt is not None:
+                lens_host[:, idx] = torch.as_tensor(cnt).to("cpu", torch.int32).numpy().reshape(-1)
+                variable = True
+        assert (lens_host[:, 0] <= m).all() and (lens_host[:, 1] <= n).all() and (lens_host >= 0).all()
+        if not variable or ((lens_host[:, 0] == m).all() and (lens_host[:, 1] == n).all()):
+            return None
+        return lens_host
 
     def loss(self, pred, data):
         from . import train as _train
@@ -387,7 +418,10 @@ class LightGlue(nn.Module):
         MatchAssignment goes through train.AssignFn (fp32; backward = lgb200_assign_dsim + cuBLAS GEMMs), the vector
         arithmetic below is tracked by autograd, and the token-confidence logits are a torch matrix-vector product on
         the detached descriptors (lightglue.py:83-84), so `losses["total"].mean().backward()` reaches every parameter
-        the reference's does."""
+        the reference's does.
+        With data["num_keypoints0/1"] every entry of `losses` and `metrics` is, per pair, that of the pair un-padded:
+        ground truth outside the valid block is ignored (padded rows of gt_matches count as -2), means over an empty
+        side are 0 (row_norm, the token-confidence BCE)."""
         lib = _abi.load()
         conf = self.conf
         r0, r1 = pred["ref_descriptors0"], pred["ref_descriptors1"]
@@ -404,6 +438,14 @@ class LightGlue(nn.Module):
         gt = data["gt_assignment"].to(dev).to(torch.bool).contiguous()
         assert gt.shape == (B, m, n), "gt_assignment must be [B, M, N]"
         gm0, gm1 = data["gt_matches0"].to(dev), data["gt_matches1"].to(dev)
+        counts_h = self._counts_of(data, B, m, n)
+        counts = valid0 = valid1 = None
+        if counts_h is not None:  # padded batch: everything outside a pair's valid block is ignored
+            counts = torch.from_numpy(counts_h.reshape(-1)).to(dev)
+            valid0 = torch.arange(m, device=dev)[None] < counts[0::2, None]
+            valid1 = torch.arange(n, device=dev)[None] < counts[1::2, None]
+            gt = (gt & valid0[:, :, None] & valid1[:, None, :]).contiguous()
+            gm0, gm1 = torch.where(valid0, gm0, -2), torch.where(valid1, gm1, -2)
         neg0, neg1 = (gm0 == -1).float(), (gm1 == -1).float()
         num_neg0, num_neg1 = neg0.sum(-1).clamp(min=1.0), neg1.sum(-1).clamp(min=1.0)
         bal = float(conf.loss.nll_balancing)
@@ -415,7 +457,7 @@ class LightGlue(nn.Module):
                 a = self.log_assignment[mod]
                 d0_, d1_ = r0[:, layer_idx], r1[:, layer_idx]
                 pos_sum, dust0, dust1, pos_cnt, _, row_arg, col_arg = AssignFn.apply(
-                    self, mod, gt, d0_, d1_, a.final_proj.weight, a.final_proj.bias, a.matchability.weight,
+                    self, mod, gt, counts, d0_, d1_, a.final_proj.weight, a.final_proj.bias, a.matchability.weight,
                     a.matchability.bias)
                 logits = None
                 if token_layer is not None:  # TokenConfidence.loss reads detached descriptors (lightglue.py:83-84)
@@ -425,7 +467,7 @@ class LightGlue(nn.Module):
                               lin(d1_.detach().float(), tk.weight, tk.bias).squeeze(-1))
             else:
                 pos_sum, pos_cnt, _, row_arg, col_arg, dust0, dust1, logits = self._log_assignment_of(
-                    lib, prec, r0[:, layer_idx], r1[:, layer_idx], mod, gt, token_layer)
+                    lib, prec, r0[:, layer_idx], r1[:, layer_idx], mod, gt, token_layer, counts=counts)
             num_pos = pos_cnt.clamp(min=1.0)
             nll_pos = -pos_sum / num_pos
             nll_neg = (-(dust0 * neg0).sum(-1) - (dust1 * neg1).sum(-1)) / (num_neg0 + num_neg1)
@@ -440,9 +482,19 @@ class LightGlue(nn.Module):
         if self.training:
             losses["confidence"] = torch.zeros_like(nll)
         la_pred = pred["log_assignment"].detach().to(torch.float32).contiguous()
-        _, _, row_exp_f, row_arg_f, col_arg_f = self._reduce(lib, la_pred, None, st)
-        losses["row_norm"] = row_exp_f.mean(1)  # lightglue.py:606
+        _, _, row_exp_f, row_arg_f, col_arg_f = self._reduce(lib, la_pred, None, st, counts)
+        if counts is None:
+            losses["row_norm"] = row_exp_f.mean(1)  # lightglue.py:606
+        else:  # (rows past the count hold 0; the mean over an empty side is 0)
+            losses["row_norm"] = row_exp_f.sum(1) / valid0.sum(1).clamp(min=1)
         bce = torch.nn.functional.binary_cross_entropy_with_logits
+
+        def bce_mean(lg, target, valid):
+            e = bce(lg, target, reduction="none")
+            if valid is None:
+                return e.mean(-1)
+            return torch.where(valid, e, 0.0).sum(-1) / valid.sum(-1).clamp(min=1)
+
         sum_w = 1.0
         for i in range(N - 1):
             nll_i, _, _, _, row_arg_i, col_arg_i, (lg0, lg1) = nll_of(i, i, token_layer=i)
@@ -451,7 +503,7 @@ class LightGlue(nn.Module):
             sum_w += w
             losses["total"] = losses["total"] + nll_i * w
             c0, c1 = (row_arg_f == row_arg_i).float(), (col_arg_f == col_arg_i).float()
-            conf_i = (bce(lg0, c0, reduction="none").mean(-1) + bce(lg1, c1, reduction="none").mean(-1)) / 2.0
+            conf_i = (bce_mean(lg0, c0, valid0) + bce_mean(lg1, c1, valid1)) / 2.0
             losses["confidence"] = losses["confidence"] + conf_i / (N - 1)
         losses["total"] = losses["total"] / sum_w
         if self.training:
@@ -601,7 +653,9 @@ class LightGlue(nn.Module):
         (lightglue.py:484-498, :546-547).  conf.checkpointed (:485-494) selects recomputation of the attention
         operands in the backward pass instead of keeping them.  The matches / log_assignment of the last layer are
         computed without a graph (the reference's loss reads pred["log_assignment"] detached, :606, :625-630).
-        conf.train_precision = "bf16" runs train.TransformerBf16Fn and the bf16 assignment kernels instead."""
+        conf.train_precision = "bf16" runs train.TransformerBf16Fn and the bf16 assignment kernels instead.
+        data["num_keypoints0/1"] (padded batches): every kernel reads the per-pair counts, the padding's descriptors and
+        keypoints are replaced by zeros, and the outputs take the layout of the no-grad forward with the same counts."""
         from . import train as _train
 
         for key in self.required_data_keys:
@@ -611,12 +665,12 @@ class LightGlue(nn.Module):
         if not kpts0.is_cuda:
             raise _abi.LightGlueB200Error(
                 "glue_factory_colon_b200.LightGlue runs on CUDA (sm_100a) tensors only; there is no CPU path")
-        if "num_keypoints0" in data or "num_keypoints1" in data:
-            raise NotImplementedError("per-pair keypoint counts are an inference extension; train on full batches")
         lib = _abi.load()
         dev = kpts0.device
         B, m, _ = kpts0.shape
         n = kpts1.shape[1]
+        counts_h = self._counts_of(data, B, m, n)  # None: no counts, or all full (exactly the path without counts)
+        counts = None if counts_h is None else torch.from_numpy(counts_h.reshape(-1)).to(dev)
 
         def size_of(v):
             sz = data[v].get("image_size") if v in data else None
@@ -635,7 +689,8 @@ class LightGlue(nn.Module):
                 k = torch.cat([k, sc.to(k), ori.to(k)], -1)
             return k.contiguous()
 
-        geom = {"k0": kpts_of(0, kpts0), "k1": kpts_of(1, kpts1), "size0": size_of("view0"), "size1": size_of("view1")}
+        geom = {"k0": kpts_of(0, kpts0), "k1": kpts_of(1, kpts1), "size0": size_of("view0"), "size1": size_of("view1"),
+                "counts": counts_h}
         desc0 = data["descriptors0"].to(torch.float32)
         desc1 = data["descriptors1"].to(torch.float32)
         assert desc0.shape[-1] == conf.input_dim and desc1.shape[-1] == conf.input_dim
@@ -644,7 +699,7 @@ class LightGlue(nn.Module):
         if self._train_bf16():  # mixed precision: the bf16 inference kernels forward (conf.train_precision)
             r0, r1 = _train.TransformerBf16Fn.apply(self, geom, desc0, desc1, *params)
             with torch.no_grad():
-                scores, m0, m1, ms0, ms1 = self._assign_match_bf16(lib, r0[:, -1], r1[:, -1], L - 1)
+                scores, m0, m1, ms0, ms1 = self._assign_match_bf16(lib, r0[:, -1], r1[:, -1], L - 1, counts)
             return {
                 "matches0": m0, "matches1": m1, "matching_scores0": ms0, "matching_scores1": ms1,
                 "ref_descriptors0": r0, "ref_descriptors1": r1, "log_assignment": scores,
@@ -654,7 +709,8 @@ class LightGlue(nn.Module):
         with torch.no_grad():
             keep: Dict = {}
             # (fp32-accurate tensor-core kernels, as the rest of the training forward; CUDA cores with LGB200_TRAIN_SIMT_LINEAR=1)
-            self._log_assignment_of(lib, F32 if _train._SIMT_LINEAR else F32X3, r0[:, -1], r1[:, -1], L - 1, None, keep=keep)
+            self._log_assignment_of(lib, F32 if _train._SIMT_LINEAR else F32X3, r0[:, -1], r1[:, -1], L - 1, None, keep=keep,
+                                    counts=counts)
             scores = keep["scores"]
             m0 = torch.empty(B, m, device=dev, dtype=torch.int64)
             m1 = torch.empty(B, n, device=dev, dtype=torch.int64)

@@ -31,6 +31,11 @@ operands, runs lgb200_ln_gelu_bwd, the bf16 attention backward (lgb200_attention
 product) and lgb200_heads_bwd, and does every plain GEMM as ONE bf16 cuBLAS product with fp32 output.  Gradients of the
 folded weights follow by the chain rule (see _ffn_bwd16).  `AssignFn` uses the bf16 assignment kernels.
 
+Padded batches (data["num_keypoints0/1"], the counts padding.py produces): every kernel of the stack reads the
+per-pair counts from the device `lens`, the staged descriptor and keypoint rows past the counts are zeroed (so the
+padding's values cannot reach an output or a gradient), and AssignFn reduces each pair over its valid block only.  A
+padded batch with counts trains like the same pairs run one at a time, un-padded (DESIGN.md 3.9).
+
 CPU tensors raise as everywhere else in this package.
 """
 from __future__ import annotations
@@ -40,6 +45,7 @@ import math
 import os
 from typing import Dict, List, Tuple
 
+import numpy as np
 import torch
 from torch import nn
 
@@ -71,18 +77,29 @@ _PERM = torch.arange(768).view(4, 64, 3).permute(2, 0, 1).reshape(-1)
 
 
 class _Kern:
-    """Launch helpers for one (B, m, n) problem: S = 2B sequences padded to Lp rows, lens on the device."""
+    """Launch helpers for one (B, m, n) problem: S = 2B sequences padded to Lp rows, lens on the device.
+    counts (host int array [B, 2], or None): per-pair valid counts of a padded batch; m / n stay the padded sizes."""
 
-    def __init__(self, dev, B: int, m: int, n: int):
+    def __init__(self, dev, B: int, m: int, n: int, counts=None):
         self.lib = _abi.load()
         check(self.lib.lgb200_device_ok(), "device check")
         self.dev, self.B, self.m, self.n = dev, B, m, n
         self.S = 2 * B
         self.Lp = max(128, ((max(m, n) + 127) // 128) * 128)
         self.T = self.S * self.Lp
-        self.lens = None
-        if m != self.Lp or n != self.Lp:
+        self.counts = counts
+        self.lens = self.valid = None
+        if counts is not None:  # one host -> device upload
+            self.lens = torch.from_numpy(np.ascontiguousarray(counts, dtype=np.int32).reshape(-1)).to(dev)
+            self.valid = (torch.arange(self.Lp, device=dev)[None] < self.lens[:, None]).reshape(-1)  # [T] bool
+        elif m != self.Lp or n != self.Lp:
             self.lens = torch.tensor([m, n] * B, device=dev, dtype=torch.int32)
+
+    def mask_rows(self, x):
+        """Zeroes the rows of x [T, ...] past the per-pair counts, in place (nothing without counts)."""
+        if self.valid is not None:
+            x.view(self.T, -1).masked_fill_(~self.valid[:, None], 0)
+        return x
 
     @property
     def st(self):
@@ -234,10 +251,11 @@ class _Kern:
                                         self.st), "lgb200_pack_rows")
 
     def pack2(self, a0, a1):
+        """[B, m, dim] / [B, n, dim] -> [T, dim], rows past the padded sizes and the per-pair counts zero."""
         dst = self.zeros(self.T, a0.shape[-1])
         self.pack(a0, 0, dst)
         self.pack(a1, 1, dst)
-        return dst
+        return self.mask_rows(dst)
 
     def unpack(self, x):
         xv = x.view(self.B, 2, self.Lp, x.shape[-1])
@@ -252,6 +270,27 @@ def normalize_keypoints(kpts: torch.Tensor, size) -> torch.Tensor:
     shift = size / 2
     scale = size.max(-1).values / 2
     return (kpts - shift[..., None, :]) / scale[..., None, None]
+
+
+def _posenc_rows(k: _Kern, geom: Dict) -> torch.Tensor:
+    """[T, kdim]: the rows posenc.Wr multiplies (lightglue.py:61-66) -- keypoints normalised as the posenc kernel does
+    (over each pair's valid points when size is None), scale / orientation un-normalised (lightglue.py:436-454);
+    rows past the per-pair counts zero."""
+    kdim = geom["k0"].shape[-1]
+    kn = k.zeros(k.T, kdim)
+    knv = kn.view(k.B, 2, k.Lp, kdim)
+    for img, kk, sz, cnt in ((0, geom["k0"], geom["size0"], k.m), (1, geom["k1"], geom["size1"], k.n)):
+        if k.counts is None:
+            knv[:, img, :cnt, :2] = normalize_keypoints(kk[..., :2], sz)
+            knv[:, img, :cnt, 2:] = kk[..., 2:]
+            continue
+        valid = k.valid.view(k.B, 2, k.Lp)[:, img, :cnt, None]
+        xy = kk[..., :2]
+        if sz is None:  # extent of the valid points only (an empty side gives non-finite values, all masked)
+            sz = 1 + torch.where(valid, xy, -math.inf).max(-2).values - torch.where(valid, xy, math.inf).min(-2).values
+        knv[:, img, :cnt, :2] = torch.where(valid, normalize_keypoints(xy, sz), 0.0)
+        knv[:, img, :cnt, 2:] = torch.where(valid, kk[..., 2:], 0.0)
+    return kn
 
 
 def transformer_params(model) -> List[Tuple[object, nn.Parameter]]:
@@ -405,7 +444,7 @@ class TransformerFn(torch.autograd.Function):
         dev = desc0.device
         B, m, _ = desc0.shape
         n = desc1.shape[1]
-        k = _Kern(dev, B, m, n)
+        k = _Kern(dev, B, m, n, geom.get("counts"))
         W = model._pack(F32, dev)
         L = model.conf.n_layers
         if not _SIMT_LINEAR:  # split-fp16 planes of the weight matrices, cached with the pack (rebuilt when a weight changes)
@@ -486,17 +525,11 @@ class TransformerFn(torch.autograd.Function):
             grads[(i, "qkv_w")], grads[(i, "qkv_b")] = gw, gb
             dx = dxm + dxa + dxp
         # positional encoding: theta = Wr . normalised keypoints (lightglue.py:61-66)
-        kdim = geom["k0"].shape[-1]
-        kn = k.zeros(k.T, kdim)
-        knv = kn.view(k.B, 2, k.Lp, kdim)
-        for img, kk, sz, cnt in ((0, geom["k0"], geom["size0"], k.m), (1, geom["k1"], geom["size1"], k.n)):
-            knv[:, img, :cnt, :2] = normalize_keypoints(kk[..., :2], sz)
-            knv[:, img, :cnt, 2:] = kk[..., 2:]  # scale / orientation enter un-normalised (lightglue.py:436-454)
-        grads["wr"] = dtheta.t() @ kn
+        grads["wr"] = dtheta.t() @ _posenc_rows(k, geom)
         if ctx.xin is not None:  # input_proj (lightglue.py:464-465)
             grads["in_w"], grads["in_b"] = dx.t() @ ctx.xin, dx.sum(0)
             dx = dx @ W["in_w"]
-        gd0, gd1 = k.unpack(dx)
+        gd0, gd1 = k.unpack(k.mask_rows(dx))
         need = ctx.needs_input_grad
         return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None,
                 *[grads[key] if need[4 + j] else None for j, key in enumerate(ctx.keys)])
@@ -577,7 +610,7 @@ class TransformerBf16Fn(torch.autograd.Function):
         dev = desc0.device
         B, m, _ = desc0.shape
         n = desc1.shape[1]
-        k = _Kern(dev, B, m, n)
+        k = _Kern(dev, B, m, n, geom.get("counts"))
         W = model._pack(BF16, dev)
         L = model.conf.n_layers
         xin = None
@@ -588,12 +621,14 @@ class TransformerBf16Fn(torch.autograd.Function):
             for img, dsc, cnt in ((0, desc0, m), (1, desc1, n)):
                 check(k.lib.lgb200_pack_rows(ptr(dsc.contiguous()), B, cnt, din, img, k.Lp, None, ptr(xin), k.st),
                       "lgb200_pack_rows")
+            k.mask_rows(xin)
             k.linear16(EPI_ROWMAJOR, xin, W["in_w"], W["in_b"], 256, din, out=x, lens=False)
         else:
             x = k.zeros16(k.T, 256)
             for img, dsc, cnt in ((0, desc0, m), (1, desc1, n)):
                 check(k.lib.lgb200_pack_rows(ptr(dsc.contiguous()), B, cnt, 256, img, k.Lp, None, ptr(x), k.st),
                       "lgb200_pack_rows")
+            k.mask_rows(x)
         rot = k.zeros(k.T, 64)  # fp32 angles for lgb200_heads_bwd, rot16 for the forward's QKV epilogue (one call)
         rot16 = torch.zeros(k.T, 32, device=dev, dtype=torch.int32)
         kdim = geom["k0"].shape[-1]
@@ -658,17 +693,11 @@ class TransformerBf16Fn(torch.autograd.Function):
             grads[(i, "qkv_w")], grads[(i, "qkv_b")] = gw, gb
             dx = dxm + dxa + dxp
         # positional encoding: theta = Wr . normalised keypoints (lightglue.py:61-66)
-        kdim = geom["k0"].shape[-1]
-        kn = k.zeros(k.T, kdim)
-        knv = kn.view(k.B, 2, k.Lp, kdim)
-        for img, kk, sz, cnt in ((0, geom["k0"], geom["size0"], k.m), (1, geom["k1"], geom["size1"], k.n)):
-            knv[:, img, :cnt, :2] = normalize_keypoints(kk[..., :2], sz)
-            knv[:, img, :cnt, 2:] = kk[..., 2:]
-        grads["wr"] = dtheta.t() @ kn
+        grads["wr"] = dtheta.t() @ _posenc_rows(k, geom)
         if ctx.xin is not None:  # input_proj (lightglue.py:464-465)
             grads["in_w"], grads["in_b"] = dx.t() @ ctx.xin.float(), dx.sum(0)
             dx = dx @ model.input_proj.weight.detach()
-        gd0, gd1 = k.unpack(dx)
+        gd0, gd1 = k.unpack(k.mask_rows(dx))
         need = ctx.needs_input_grad
         return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None,
                 *[grads[key] if need[4 + j] else None for j, key in enumerate(ctx.keys)])
@@ -677,17 +706,20 @@ class TransformerBf16Fn(torch.autograd.Function):
 class AssignFn(torch.autograd.Function):
     """MatchAssignment `layer` on (d0, d1) reduced to the inputs of NLLLoss: pos_sum [B] = sum of log_assignment over
     the ground-truth matches, dust0 [B,m] / dust1 [B,n] = the dustbin column / row (differentiable); pos_cnt, row_exp,
-    row_arg, col_arg as in lgb200_loss_reduce (not differentiable)."""
+    row_arg, col_arg as in lgb200_loss_reduce (not differentiable).  counts (device int32 [2B] or None): per-pair valid
+    counts of a padded batch -- every pair is then reduced over its valid block (lgb200_loss_reduce_ragged semantics)
+    and the gradients are exactly 0 outside it; gt must be False outside it."""
 
     @staticmethod
-    def forward(ctx, model, layer: int, gt, d0, d1, fp_w, fp_b, m_w, m_b):
+    def forward(ctx, model, layer: int, gt, counts, d0, d1, fp_w, fp_b, m_w, m_b):
         lib = _abi.load()
         keep: Dict = {}
         bf = model._train_bf16()
         prec = BF16 if bf else (F32 if _SIMT_LINEAR else F32X3)
         pos_sum, pos_cnt, row_exp, row_arg, col_arg, dust0, dust1, _ = model._log_assignment_of(
-            lib, prec, d0, d1, layer, gt, keep=keep)
+            lib, prec, d0, d1, layer, gt, keep=keep, counts=counts)
         ctx.save_for_backward(d0, d1, fp_w, fp_b, m_w, gt, keep["z"], keep["lse"])
+        ctx.counts = counts
         ctx.Lp = keep["Lp"]
         # x3 mode: the split planes of final_proj(desc) / 4 (33 MB at 8 x 2048) -- the backward recomputes the similarity
         # from them on tcgen05 instead of redoing final_proj and the N x M product in fp32 on the CUDA cores
@@ -723,7 +755,13 @@ class AssignFn(torch.autograd.Function):
         g = (g_pos if g_pos is not None else torch.zeros(B, device=dev)).to(torch.float32).contiguous()
         r = (g[:, None] * gt.sum(2)).contiguous()
         c = (g[:, None] * gt.sum(1)).contiguous()
-        check(lib.lgb200_assign_dsim(ptr(sim), B, m, n, ptr(lse), Lp, ptr(gt), ptr(g), ptr(r), ptr(c), st), "assign_dsim")
+        counts = ctx.counts
+        if counts is None:
+            check(lib.lgb200_assign_dsim(ptr(sim), B, m, n, ptr(lse), Lp, ptr(gt), ptr(g), ptr(r), ptr(c), st),
+                  "assign_dsim")
+        else:  # exact zeros outside every pair's valid block
+            check(lib.lgb200_assign_dsim_ragged(ptr(sim), B, m, n, ptr(lse), Lp, ptr(counts), ptr(gt), ptr(g), ptr(r),
+                                                ptr(c), st), "assign_dsim_ragged")
         if md16 is not None:
             s16 = sim.to(torch.bfloat16)
             dmd0 = torch.bmm(s16, md1, out_dtype=f32)
@@ -753,14 +791,20 @@ class AssignFn(torch.autograd.Function):
         # la = ... + logsigmoid(z0_i) + logsigmoid(z1_j) inside, logsigmoid(-z) in the dustbins (lightglue.py:262-267)
         dz0 = r * torch.sigmoid(-z0) - gd0 * torch.sigmoid(z0)
         dz1 = c * torch.sigmoid(-z1) - gd1 * torch.sigmoid(z1)
+        if counts is not None:  # rows past the counts: no matchability gradient (their z is not a keypoint's)
+            v0 = torch.arange(m, device=dev)[None] < counts[0::2, None]
+            v1 = torch.arange(n, device=dev)[None] < counts[1::2, None]
+            dz0, dz1 = torch.where(v0, dz0, 0.0), torch.where(v1, dz1, 0.0)
         mw = m_w.reshape(1, 1, 256)
         gx0 = 0.25 * (dmd0 @ fp_w) + dz0[..., None] * mw
         gx1 = 0.25 * (dmd1 @ fp_w) + dz1[..., None] * mw
+        if counts is not None:
+            gx0, gx1 = torch.where(v0[..., None], gx0, 0.0), torch.where(v1[..., None], gx1, 0.0)
         g_fp_w = 0.25 * (dmd0.reshape(-1, 256).t() @ x0.reshape(-1, 256) + dmd1.reshape(-1, 256).t() @ x1.reshape(-1, 256))
         g_fp_b = 0.25 * (dmd0.sum((0, 1)) + dmd1.sum((0, 1)))
         g_m_w = ((dz0[..., None] * x0).sum((0, 1)) + (dz1[..., None] * x1).sum((0, 1))).reshape(m_w.shape)
         g_m_b = (dz0.sum() + dz1.sum()).reshape(1)
-        return None, None, None, gx0, gx1, g_fp_w, g_fp_b, g_m_w, g_m_b
+        return None, None, None, None, gx0, gx1, g_fp_w, g_fp_b, g_m_w, g_m_b
 
 
 def wants_grad(model, data=None) -> bool:

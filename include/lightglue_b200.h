@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define LGB200_ABI_VERSION 7
+#define LGB200_ABI_VERSION 8
 
 enum { LGB200_F32 = 0, LGB200_BF16 = 1, LGB200_F32X3 = 2 };
 
@@ -222,13 +222,25 @@ int lgb200_npair_loss(const float* similarity, const uint8_t* gt_assignment, int
 int lgb200_loss_reduce(const float* log_assignment, int B, int R, int C, const uint8_t* gt_assignment,
                        float* row_pos, float* row_cnt, float* row_exp, int32_t* row_arg, int32_t* col_arg,
                        void* stream);
+/* lgb200_loss_reduce_ragged: the same for a padded batch with per-pair counts lens [2B] (device; lens[2b] rows of
+ * image 0, lens[2b+1] of image 1, each at most R-1 / C-1) in the inference layout of such a batch -- dustbin column
+ * C-1 and dustbin row R-1 whatever the counts.  Pair b is reduced over rows i < lens[2b] and columns j < lens[2b+1]
+ * of the inner block plus the dustbins: row_pos / row_cnt / row_exp sum over that region only (gt_assignment is read
+ * only inside it), row_arg covers the valid columns plus the dustbin C-1, col_arg the valid rows plus the dustbin
+ * R-1.  Rows i >= lens[2b] get row_pos = row_cnt = row_exp = 0 and row_arg = -1; columns j >= lens[2b+1] get
+ * col_arg = -1.  lens must not be NULL (full counts: lgb200_loss_reduce). */
+int lgb200_loss_reduce_ragged(const float* log_assignment, int B, int R, int C, const int32_t* lens,
+                              const uint8_t* gt_assignment, float* row_pos, float* row_cnt, float* row_exp,
+                              int32_t* row_arg, int32_t* col_arg, void* stream);
 
 /* Fused form for LGB200_BF16 (tcgen05): MatchAssignment pass 2 of lgb200_assign_scores with the reductions above in
  * its epilogue instead of the store -- the [B,R,C] matrix of a layer that only the loss looks at (every layer but
  * the last in training mode, lightglue.py:607-608) is never written.  Same outputs as lgb200_loss_reduce on the
- * matrix lgb200_assign_scores would have produced; md / z / lse as for lgb200_assign_scores; lens entries must be
- * R-1 / C-1 (or lens NULL when R-1 == C-1 == Lp).  workspace: 8 * B * (R + C) bytes.  LGB200_F32 is refused
- * (LGB200_ERR_PRECISION): the fp32 parity mode materialises and calls lgb200_loss_reduce. */
+ * matrix lgb200_assign_scores would have produced; md / z / lse as for lgb200_assign_scores.  lens (nullable when
+ * R-1 == C-1 == Lp) holds per-pair counts of at most R-1 / C-1: with counts below R-1 / C-1 the outputs are those of
+ * lgb200_loss_reduce_ragged with the same lens (rows and columns past the counts: sums 0, arg-maximum -1; the
+ * dustbin folded in only inside the counts).  workspace: 8 * B * (R + C) bytes.  LGB200_F32 is refused
+ * (LGB200_ERR_PRECISION): the fp32 parity mode materialises and calls lgb200_loss_reduce(_ragged). */
 int lgb200_assign_loss(int precision, const void* md, const float* z, const float* lse, int B, int Lp,
                        const int32_t* lens, int R, int C, const uint8_t* gt_assignment, float* row_pos,
                        float* row_cnt, float* row_exp, int32_t* row_arg, int32_t* col_arg, void* workspace,
@@ -311,7 +323,10 @@ int lgb200_x3_assign_scores(const float* sim, const float* z, const float* lse, 
  * lgb200_assign_dsim: backward of sigmoid_log_double_softmax (lightglue.py:257-269) w.r.t. the similarity, for a
  *   loss that is linear in log_assignment (NLLLoss, losses.py:6-26): sim [B,m,n] is replaced in place by
  *   2 g_pos[b] gt - r[b,i] exp(sim - lse0[i]) - c[b,j] exp(sim - lse1[j]); lse as written by lgb200_assign_lse
- *   ([S,Lp]: rows of image 0, columns of image 1), r / c = g_pos times the row / column sums of gt. */
+ *   ([S,Lp]: rows of image 0, columns of image 1), r / c = g_pos times the row / column sums of gt.
+ * lgb200_assign_dsim_ragged: the same for a padded batch (m, n = padded sizes) with per-pair counts lens [2B]
+ *   (device, not NULL): entries of pair b with i >= lens[2b] or j >= lens[2b+1] become exactly 0, and gt, r, c and
+ *   lse are read only inside the valid block. */
 int lgb200_attention_bwd(const float* Q, const float* K, const float* V, const float* ctx, const float* dctx,
                          int S, int Lp, const int32_t* lens, int kv_xor, float* dQ, float* dK, float* dV,
                          float* workspace, void* stream);
@@ -336,6 +351,9 @@ int lgb200_ln_gelu_bwd(const float* h, const float* gamma, const float* beta, co
 int lgb200_assign_dsim(float* sim, int B, int m, int n, const float* lse, int Lp,
                        const uint8_t* gt_assignment, const float* g_pos, const float* r, const float* c,
                        void* stream);
+int lgb200_assign_dsim_ragged(float* sim, int B, int m, int n, const float* lse, int Lp, const int32_t* lens,
+                              const uint8_t* gt_assignment, const float* g_pos, const float* r, const float* c,
+                              void* stream);
 
 #ifdef __cplusplus
 }
