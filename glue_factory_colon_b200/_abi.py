@@ -34,6 +34,7 @@ SIGNATURES = {
     "lgb200_nn_scores": [_p, _p, _i, _i, _p, _i, _i, _p, _p, _p],
     "lgb200_nn_match": [_p, _i, _i, _i, _p, _f, _f, _i, _p, _p, _p, _p, _p, _p],
     "lgb200_npair_loss": [_p, _p, _i, _i, _i, _f, _p, _p, _p, _p],
+    "lgb200_npair_loss_bwd": [_p, _p, _i, _i, _i, _f, _p, _p, _p, _p, _p, _p, _p],
     "lgb200_loss_reduce": [_p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p],
     "lgb200_loss_reduce_ragged": [_p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],
     "lgb200_assign_loss": [_i, _p, _p, _p, _i, _i, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],

@@ -4,6 +4,7 @@
 //   lgb200_nn_match  : find_nn (:15-31) in both directions (top-2 by value for the ratio test, distance threshold),
 //                      mutual_check (:34-43), matching_scores = (match > -1) (:75-76)
 //   lgb200_npair_loss: the N_pair loss (:85-109) on the similarity matrix, forward values
+//   lgb200_npair_loss_bwd: its gradient w.r.t. the similarity and the temperature
 // fp32 CUDA-core kernels (the baseline matcher is not on the headline path; its cost is the N x M write).
 #include "lg_internal.cuh"
 
@@ -101,9 +102,8 @@ __global__ void nn_mutual_kernel(const long long* __restrict__ nn0, const long l
 // column log-softmax of scores.  Three streaming passes over sim [B,N,M]: row LSE (warp per row), column LSE (32 columns
 // x 8 row groups per CTA, online max/sum merged through shared memory), then the ground-truth pass (warp per row ->
 // per-row partial sums, no atomics: bit-reproducible).
-__device__ __forceinline__ float npair_score(float sim, float T) {
-  return T * (2.f - sqrtf(fmaxf(2.f * (1.f - sim), 1e-6f)));
-}
+__device__ __forceinline__ float npair_q(float sim) { return sqrtf(fmaxf(2.f * (1.f - sim), 1e-6f)); }
+__device__ __forceinline__ float npair_score(float sim, float T) { return T * (2.f - npair_q(sim)); }
 __device__ __forceinline__ void lse_push(float& mx, float& sm, float v) {
   if (v > mx) { sm = sm * __expf(mx - v) + 1.f; mx = v; }
   else sm += __expf(v - mx);
@@ -170,6 +170,76 @@ __global__ void npair_gt_kernel(const float* __restrict__ sim, const uint8_t* __
   }
 }
 
+// ---- N_pair loss backward --------------------------------------------------------------------------------------------
+// d nll_b / d s_ij = coef_b (2 a_ij - r_i exp(s_ij - lse_r_i) - c_j exp(s_ij - lse_c_j)), coef_b = -g_b / (2 num_b),
+// r / c = row / column counts of a.  d s / d sim = T / q where the clamp passes (2 (1 - sim) >= 1e-6, torch's rule for
+// clamp(min=)), 0 where it clamps; d s / d T = 2 - q.
+
+// c[b,j] = sum_i a_ij: 128 columns x 32 row groups per CTA; a warp load is one 32-byte segment of a row.  The sums are
+// integer-valued floats, exact in any order.
+__global__ void __launch_bounds__(1024) npair_colcnt_kernel(const uint8_t* __restrict__ gt, int N, int M,
+                                                            float* __restrict__ col_cnt) {
+  __shared__ float sh[32][129];
+  const int b = blockIdx.y, lane = threadIdx.x & 31, ry = threadIdx.x >> 5;
+  const int c0 = blockIdx.x * 128 + lane;
+  const uint8_t* p = gt + (size_t)b * N * M;
+  float acc[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 4
+  for (int r = ry; r < N; r += 32) {
+    const uint8_t* q = p + (size_t)r * M;
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+      if (c0 + 32 * k < M && q[c0 + 32 * k]) acc[k] += 1.f;
+  }
+#pragma unroll
+  for (int k = 0; k < 4; ++k) sh[ry][lane + 32 * k] = acc[k];
+  __syncthreads();
+  if (threadIdx.x < 128) {
+    const int col = blockIdx.x * 128 + threadIdx.x;
+    float s = 0.f;
+    for (int k = 0; k < 32; ++k) s += sh[k][threadIdx.x];
+    if (col < M) col_cnt[(size_t)b * M + col] = s;
+  }
+}
+
+// warp per row, four coalesced 128-byte column chunks in flight per lane: dsim (nullable) and the row's partial
+// sum_j d s_ij (2 - q_ij) of d nll / d T (per-row partials, no atomics: bit-reproducible)
+__global__ void npair_bwd_kernel(const float* __restrict__ sim, const uint8_t* __restrict__ gt, int N, int M, float T,
+                                 const float* __restrict__ lse_r, const float* __restrict__ lse_c,
+                                 const float* __restrict__ row_cnt, const float* __restrict__ col_cnt,
+                                 const float* __restrict__ coef, float* __restrict__ dsim,
+                                 float* __restrict__ dtemp_rows) {
+  const int b = blockIdx.y, row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (row >= N) return;
+  const size_t off = ((size_t)b * N + row) * M;
+  const float lr = lse_r[(size_t)b * N + row], r = row_cnt[(size_t)b * N + row], k = coef[b];
+  const float* lc = lse_c + (size_t)b * M;
+  const float* cc = col_cnt + (size_t)b * M;
+  float acc = 0.f;
+  for (int c0 = lane; c0 < M; c0 += 128) {
+    float sv[4];
+    bool av[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int c = c0 + 32 * u;
+      sv[u] = c < M ? sim[off + c] : 0.f;
+      av[u] = c < M && gt[off + c];
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int c = c0 + 32 * u;
+      if (c < M) {
+        const float q = npair_q(sv[u]), s = npair_score(sv[u], T);
+        const float ds = k * ((av[u] ? 2.f : 0.f) - r * __expf(s - lr) - cc[c] * __expf(s - lc[c]));
+        if (dsim) dsim[off + c] = 2.f * (1.f - sv[u]) >= 1e-6f ? ds * T / q : 0.f;
+        acc += ds * (2.f - q);
+      }
+    }
+  }
+  for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if (lane == 0) dtemp_rows[(size_t)b * N + row] = acc;
+}
+
 }  // namespace
 
 extern "C" int lgb200_npair_loss(const float* similarity, const uint8_t* gt_assignment, int B, int N, int M,
@@ -185,6 +255,22 @@ extern "C" int lgb200_npair_loss(const float* similarity, const uint8_t* gt_assi
   LG_LAUNCH_CHECK();
   npair_gt_kernel<<<dim3((N + 7) / 8, B), 256, 0, st>>>(similarity, gt_assignment, N, M, temperature, lse_r, lse_c,
                                                         row_sum, row_cnt);
+  LG_LAUNCH_CHECK();
+  return LGB200_OK;
+}
+
+extern "C" int lgb200_npair_loss_bwd(const float* similarity, const uint8_t* gt_assignment, int B, int N, int M,
+                                     float temperature, const float* workspace, const float* row_cnt, const float* coef,
+                                     float* col_cnt, float* dsim, float* dtemp_rows, void* stream) {
+  if (!similarity || !gt_assignment || !workspace || !row_cnt || !coef || !col_cnt || !dtemp_rows) return LGB200_ERR_NULL;
+  if (B <= 0 || N <= 0 || M <= 0 || B > 65535) return LGB200_ERR_SHAPE;
+  cudaStream_t st = lg_stream(stream);
+  const float* lse_r = workspace;
+  const float* lse_c = workspace + (size_t)B * N;
+  npair_colcnt_kernel<<<dim3((M + 127) / 128, B), 1024, 0, st>>>(gt_assignment, N, M, col_cnt);
+  LG_LAUNCH_CHECK();
+  npair_bwd_kernel<<<dim3((N + 7) / 8, B), 256, 0, st>>>(similarity, gt_assignment, N, M, temperature, lse_r, lse_c,
+                                                         row_cnt, col_cnt, coef, dsim, dtemp_rows);
   LG_LAUNCH_CHECK();
   return LGB200_OK;
 }

@@ -262,6 +262,17 @@ class _Kern:
         return xv[:, 0, : self.m], xv[:, 1, : self.n]
 
 
+def bmm3(A, B, scale):
+    """Batched _Kern.mm3: fp32-accurate A.B from plane pairs A [2, b, M, K], B [2, b, K, N] (views may be transposed)
+    as three fp16 tensor-core bmms with fp32 accumulation and fp32 output, times `scale` (float or 0-dim device
+    tensor)."""
+    f32 = torch.float32
+    o = torch.bmm(A[1], B[0], out_dtype=f32)
+    torch.baddbmm(o, A[0], B[1], out_dtype=f32, out=o)
+    torch.baddbmm(o, A[0], B[0], out_dtype=f32, out=o)
+    return o.mul_(scale)
+
+
 def normalize_keypoints(kpts: torch.Tensor, size) -> torch.Tensor:
     """lightglue.py:28-40 (only needed for the gradient of posenc.Wr; the forward's posenc kernel has it fused)."""
     if size is None:
@@ -775,15 +786,8 @@ class AssignFn(torch.autograd.Function):
             check(lib.lgb200_split_dynamic(ptr(sim), sim.numel(), ptr(sp), ptr(inv), 0, None, 0, st), "lgb200_split_dynamic")
             mv = mdp.view(2, B, 2, Lp, 256)
             mp0, mp1 = mv[:, :, 0, :m], mv[:, :, 1, :n]
-
-            def bmm3(A, Bm):
-                o = torch.bmm(A[1], Bm[0], out_dtype=f32)
-                torch.baddbmm(o, A[0], Bm[1], out_dtype=f32, out=o)
-                torch.baddbmm(o, A[0], Bm[0], out_dtype=f32, out=o)
-                return o.mul_(inv[0] * AI)
-
-            dmd0 = bmm3(sp, mp1)
-            dmd1 = bmm3(sp.transpose(2, 3), mp0)
+            dmd0 = bmm3(sp, mp1, inv[0] * AI)
+            dmd1 = bmm3(sp.transpose(2, 3), mp0, inv[0] * AI)
         zv = z.view(B, 2, Lp)
         z0, z1 = zv[:, 0, :m], zv[:, 1, :n]
         gd0 = g_d0 if g_d0 is not None else torch.zeros_like(z0)

@@ -209,6 +209,19 @@ int lgb200_nn_match(const float* similarity, int B, int N, int M, const int32_t*
  * workspace: B * (N + M) floats. */
 int lgb200_npair_loss(const float* similarity, const uint8_t* gt_assignment, int B, int N, int M,
                       float temperature, float* workspace, float* row_sum, float* row_cnt, void* stream);
+/* Backward of lgb200_npair_loss (what autograd derives for nearest_neighbor_matcher.py:85-109), on the same
+ * similarity, gt_assignment and temperature, after that call: workspace = its row / column log-sum-exps LR | LC,
+ * row_cnt = its r.  coef [B] = -g_b / (2 num_b) with g_b the gradient of nll_b.  With s = T (2 - q),
+ * q = sqrt(clamp(2 (1 - sim), 1e-6)) and c_j = sum_i a_ij:
+ *   d nll / d s_ij = coef_b (2 a_ij - r_i exp(s_ij - LR_i) - c_j exp(s_ij - LC_j));
+ *   dsim [B,N,M] (nullable: then nothing is written) = d nll / d s_ij * T / q_ij where 2 (1 - sim) >= 1e-6,
+ *          0 where the clamp holds (torch's rule);
+ *   dtemp_rows [B,N] = sum_j d nll / d s_ij (2 - q_ij), per-row partials of d nll / d T (no atomics: bit-reproducible;
+ *          the caller adds them).
+ * col_cnt [B,M]: scratch, receives c. */
+int lgb200_npair_loss_bwd(const float* similarity, const uint8_t* gt_assignment, int B, int N, int M,
+                          float temperature, const float* workspace, const float* row_cnt, const float* coef,
+                          float* col_cnt, float* dsim, float* dtemp_rows, void* stream);
 
 /* ---- loss-side reductions (SURVEY.md 8(f) rank 2; forward values only) -------------------
  * Replaces the dense [B,R,C] reductions behind LightGlue.loss, lightglue.py:588-637:
