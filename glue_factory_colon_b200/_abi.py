@@ -53,6 +53,9 @@ SIGNATURES = {
     "lgb200_ln_gelu_bwd": [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _i, _p],
     "lgb200_assign_dsim": [_p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p],
     "lgb200_assign_dsim_ragged": [_p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p, _p],
+    "lgb200_assign_bwd": [_p, _p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p, _p],
+    "lgb200_assign_bwd_workspace": [_i, _i, _i, _p],
+    "lgb200_posenc_bwd": [_p, _i, _i, _i, _p, _p, _p, _i, _i, _p, _p, _p],
     "lgb200_prune_compact": [_p, _p, _f, _f, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
 }
 

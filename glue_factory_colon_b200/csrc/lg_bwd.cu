@@ -14,6 +14,8 @@
 //                           gradient of the rotary angles (-> posenc.Wr)                   lightglue.py:43-50, 157-161
 //   ln_gelu_bwd_kernel      GELU(erf)' . LayerNorm backward, d gamma / d beta partials     lightglue.py:144-149
 //   assign_dsim_kernel      d sim of sigmoid_log_double_softmax (optionally per-pair counts) lightglue.py:257-269
+//   abwd_*_kernel           the same for any upstream gradient of log_assignment, plus d z   lightglue.py:257-269
+//   posenc_bwd_kernel       d keypoints through normalize_keypoints and posenc.Wr            lightglue.py:28-40, 61-66
 #include "lg_common.cuh"
 #include "lg_internal.cuh"
 #include <stdlib.h>
@@ -657,6 +659,247 @@ __global__ void __launch_bounds__(256) assign_dsim_kernel(float* __restrict__ si
   sim[off] = g - r[(size_t)b * m + i] * expf(sv - l0) - c[(size_t)b * n + j] * expf(sv - l1);
 }
 
+// ---- backward of log_assignment for any upstream gradient G [B, m+1, n+1] ----------------------------------------
+// With R_i / C_j the row / column sums of G over pair b's valid block (n0 x n1):
+//   d sim_ij = 2 G_ij - R_i exp(sim_ij - lse0_i) - C_j exp(sim_ij - lse1_j)   inside the block, 0 outside;
+//   d z0_i   = R_i sigmoid(-z0_i) - G_{i,n} sigmoid(z0_i),   d z1_j = C_j sigmoid(-z1_j) - G_{m,j} sigmoid(z1_j).
+// Three launches, no atomics (every sum has a fixed order, results are bit-reproducible):
+//   abwd_sums_kernel   reads G once: a warp owns ABWD_ROWS whole rows and sweeps them in blocks of 128 columns, lane =
+//                      column (coalesced 128-byte row segments; the (n+1)-float row pitch rules out vector loads).  Row
+//                      sums stay in registers for the whole sweep (complete R_i, then d z0); column sums of the block
+//                      go out as per-warp partials part[b][p][j].
+//   abwd_cols_kernel   C_j = sum of the partials in warp order, then d z1.
+//   abwd_dsim_kernel   warp per row, streams sim -> d sim in place, reading G a second time.
+constexpr int ABWD_ROWS = 32;  // rows per warp of the sums pass
+constexpr int ABWD_GROUP = 8;  // rows loaded together: 32 independent loads in flight per lane
+
+__device__ __forceinline__ int abwd_chunks(int rows) { return (rows + ABWD_ROWS - 1) / ABWD_ROWS; }
+
+__global__ void __launch_bounds__(128) abwd_sums_kernel(const float* __restrict__ G, int m, int n,
+                                                        const int32_t* __restrict__ lens, const float* __restrict__ z,
+                                                        int Lp, float* __restrict__ rsum, float* __restrict__ part,
+                                                        float* __restrict__ dz0) {
+  const int b = blockIdx.y, lane = threadIdx.x & 31;
+  const int p = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int P = abwd_chunks(m);
+  if (p >= P) return;
+  const int n0 = lens ? min(lens[2 * b], m) : m, n1 = lens ? min(lens[2 * b + 1], n) : n;
+  const int C = n + 1, r0 = p * ABWD_ROWS;
+  const int rows = max(0, min(ABWD_ROWS, n0 - r0));
+  const float* g = G + ((size_t)b * (m + 1) + r0) * C;
+  float* pp = part + ((size_t)b * P + p) * n;
+  float racc[ABWD_ROWS];
+#pragma unroll
+  for (int i = 0; i < ABWD_ROWS; ++i) racc[i] = 0.f;
+  for (int c0 = 0; rows > 0 && c0 < n1; c0 += 128) {
+    float cacc[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int gi = 0; gi < ABWD_ROWS / ABWD_GROUP; ++gi) {
+      float v[ABWD_GROUP][4];
+#pragma unroll
+      for (int i = 0; i < ABWD_GROUP; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const int r = gi * ABWD_GROUP + i, c = c0 + lane + 32 * j;
+          v[i][j] = (r < rows && c < n1) ? __ldg(g + (size_t)r * C + c) : 0.f;
+        }
+#pragma unroll
+      for (int i = 0; i < ABWD_GROUP; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          racc[gi * ABWD_GROUP + i] += v[i][j];
+          cacc[j] += v[i][j];
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (c0 + lane + 32 * j < n1) pp[c0 + lane + 32 * j] = cacc[j];
+  }
+#pragma unroll
+  for (int i = 0; i < ABWD_ROWS; ++i) {
+    float s = racc[i];
+#pragma unroll
+    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    const int r = r0 + i;
+    if (lane == (i & 31) && r < m) {
+      const bool in = i < rows;
+      rsum[(size_t)b * m + r] = in ? s : 0.f;
+      if (dz0) {
+        float d = 0.f;
+        if (in) {
+          const float zv = z[(size_t)(2 * b) * Lp + r];
+          d = s * lg_sigmoid(-zv) - g[(size_t)i * C + n] * lg_sigmoid(zv);
+        }
+        dz0[(size_t)b * m + r] = d;
+      }
+    }
+  }
+}
+
+__global__ void __launch_bounds__(256) abwd_cols_kernel(const float* __restrict__ G, int m, int n,
+                                                        const int32_t* __restrict__ lens, const float* __restrict__ z,
+                                                        int Lp, const float* __restrict__ part,
+                                                        float* __restrict__ csum, float* __restrict__ dz1) {
+  const int b = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  const int n0 = lens ? min(lens[2 * b], m) : m, n1 = lens ? min(lens[2 * b + 1], n) : n;
+  const int P = abwd_chunks(m);
+  float s = 0.f, d = 0.f;
+  if (j < n1) {
+    const float* pp = part + (size_t)b * P * n + j;
+    for (int p = 0; p < abwd_chunks(n0); ++p) s += pp[(size_t)p * n];
+    if (dz1) {
+      const float zv = z[(size_t)(2 * b + 1) * Lp + j];
+      d = s * lg_sigmoid(-zv) - G[((size_t)b * (m + 1) + m) * (n + 1) + j] * lg_sigmoid(zv);
+    }
+  }
+  csum[(size_t)b * n + j] = s;
+  if (dz1) dz1[(size_t)b * n + j] = d;
+}
+
+__global__ void __launch_bounds__(256) abwd_dsim_kernel(const float* __restrict__ G, float* __restrict__ sim, int m,
+                                                        int n, const float* __restrict__ lse, int Lp,
+                                                        const int32_t* __restrict__ lens,
+                                                        const float* __restrict__ rsum,
+                                                        const float* __restrict__ csum) {
+  const int b = blockIdx.y, i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (i >= m) return;
+  const int n0 = lens ? min(lens[2 * b], m) : m, n1 = lens ? min(lens[2 * b + 1], n) : n;
+  float* row = sim + ((size_t)b * m + i) * n;
+  if (i >= n0) {
+    for (int c = lane; c < n; c += 32) row[c] = 0.f;
+    return;
+  }
+  const float* g = G + ((size_t)b * (m + 1) + i) * (n + 1);
+  const float l0 = lse[(size_t)(2 * b) * Lp + i], r = rsum[(size_t)b * m + i];
+  const float* l1 = lse + (size_t)(2 * b + 1) * Lp;
+  const float* cs = csum + (size_t)b * n;
+  for (int c0 = lane; c0 < n; c0 += 128) {
+    float sv[4], gv[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int c = c0 + 32 * u;
+      sv[u] = c < n1 ? row[c] : 0.f;
+      gv[u] = c < n1 ? __ldg(g + c) : 0.f;
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const int c = c0 + 32 * u;
+      if (c < n) row[c] = c < n1 ? 2.f * gv[u] - r * expf(sv[u] - l0) - cs[c] * expf(sv[u] - l1[c]) : 0.f;
+    }
+  }
+}
+
+// ---- backward of the positional encoding's keypoint normalisation (lightglue.py:28-40, 61-66) ----------------------
+// CTA per pair-image.  d kn = d theta . Wr per point; then, with t = max(size) / 2 and kn = (x - size / 2) / t:
+//   d x_l = d kn_l / t  (+ scale / orientation: d kn passes through);
+//   size == NULL (size = 1 + max - min over the valid points): with A = sum_l d kn_l and Q = sum_l <d kn_l, kn_l>,
+//   d size_x = -(A_x + [x extent is the larger] Q) / (2 t), likewise y; it reaches the arg-max point with + and the
+//   arg-min point with -, the lowest index among ties in both (torch's rule for max(dim) / min(dim)), and the x extent
+//   counts as the larger one when the two are equal.  All sums have a fixed order (bit-reproducible).
+__global__ void __launch_bounds__(1024) posenc_bwd_kernel(const float* __restrict__ kpts, int n, int kdim,
+                                                          const float* __restrict__ size, const float* __restrict__ Wr,
+                                                          const int32_t* __restrict__ lens, int img, int Lp,
+                                                          const float* __restrict__ dtheta, float* __restrict__ dkpts) {
+  const int b = blockIdx.x, s = 2 * b + img;
+  const int nv = lens ? min(lens[s], n) : n;
+  const float* kp = kpts + (size_t)b * n * kdim;
+  float* dk = dkpts + (size_t)b * n * kdim;
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  __shared__ float sW[32 * 4];
+  __shared__ unsigned long long ext[4][32];  // packed (value, index) of max x, max y, max -x, max -y per warp
+  __shared__ float red[3][32];
+  __shared__ float sh[3];
+  __shared__ int arg[4], sel;
+  for (int i = threadIdx.x; i < 32 * kdim; i += blockDim.x) sW[i] = Wr[i];
+  if (size) {
+    if (threadIdx.x == 0) {
+      const float wd = size[b * 2 + 0], ht = size[b * 2 + 1];
+      sh[0] = wd / 2.f;
+      sh[1] = ht / 2.f;
+      sh[2] = fmaxf(wd, ht) / 2.f;
+    }
+  } else {
+    unsigned long long e[4] = {0ull, 0ull, 0ull, 0ull};
+    for (int l = threadIdx.x; l < nv; l += blockDim.x) {
+      const float x = kp[(size_t)l * kdim], y = kp[(size_t)l * kdim + 1];
+      const unsigned long long c[4] = {fm_pack(x, l), fm_pack(y, l), fm_pack(-x, l), fm_pack(-y, l)};
+#pragma unroll
+      for (int k = 0; k < 4; ++k) e[k] = c[k] > e[k] ? c[k] : e[k];
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      for (int o = 16; o; o >>= 1) {
+        const unsigned long long t = __shfl_xor_sync(0xffffffffu, e[k], o);
+        e[k] = t > e[k] ? t : e[k];
+      }
+      if (lane == 0) ext[k][w] = e[k];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0 && nv > 0) {
+      for (int i = 1; i < nw; ++i)
+        for (int k = 0; k < 4; ++k) ext[k][0] = ext[k][i] > ext[k][0] ? ext[k][i] : ext[k][0];
+      // the forward's arithmetic (posenc_kernel): size = 1 + max - min, shift = size / 2, t = max(size) / 2
+      const float sx = 1.f + fm_value(ext[0][0]) - (-fm_value(ext[2][0]));
+      const float sy = 1.f + fm_value(ext[1][0]) - (-fm_value(ext[3][0]));
+      sh[0] = sx / 2.f;
+      sh[1] = sy / 2.f;
+      sh[2] = fmaxf(sx, sy) / 2.f;
+      sel = sx >= sy ? 0 : 1;
+      for (int k = 0; k < 4; ++k) arg[k] = fm_index(ext[k][0]);
+    }
+  }
+  __syncthreads();
+  const float shx = sh[0], shy = sh[1], t = sh[2];
+  float ax = 0.f, ay = 0.f, q = 0.f;
+  for (int l = threadIdx.x; l < n; l += blockDim.x) {
+    float d[4] = {0.f, 0.f, 0.f, 0.f};
+    if (l < nv) {
+      const float4* th = reinterpret_cast<const float4*>(dtheta + ((size_t)s * Lp + l) * 32);
+#pragma unroll
+      for (int f4 = 0; f4 < 8; ++f4) {
+        const float4 v = th[f4];
+        const float tv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+#pragma unroll
+          for (int c = 0; c < 4; ++c)
+            if (c < kdim) d[c] = fmaf(tv[u], sW[(f4 * 4 + u) * kdim + c], d[c]);
+      }
+      if (!size) {
+        const float knx = (kp[(size_t)l * kdim] - shx) / t, kny = (kp[(size_t)l * kdim + 1] - shy) / t;
+        ax += d[0];
+        ay += d[1];
+        q += d[0] * knx + d[1] * kny;
+      }
+      d[0] /= t;
+      d[1] /= t;
+    }
+#pragma unroll
+    for (int c = 0; c < 4; ++c)
+      if (c < kdim) dk[(size_t)l * kdim + c] = d[c];
+  }
+  if (size) return;
+  for (int o = 16; o; o >>= 1) {
+    ax += __shfl_xor_sync(0xffffffffu, ax, o);
+    ay += __shfl_xor_sync(0xffffffffu, ay, o);
+    q += __shfl_xor_sync(0xffffffffu, q, o);
+  }
+  if (lane == 0) { red[0][w] = ax; red[1][w] = ay; red[2][w] = q; }
+  __syncthreads();  // (also orders the d x stores above before thread 0's updates below)
+  if (threadIdx.x == 0 && nv > 0) {
+    float A[3] = {0.f, 0.f, 0.f};
+    for (int i = 0; i < nw; ++i)
+      for (int k = 0; k < 3; ++k) A[k] += red[k][i];
+    const float dsx = -(A[0] + (sel == 0 ? A[2] : 0.f)) / (2.f * t);
+    const float dsy = -(A[1] + (sel == 1 ? A[2] : 0.f)) / (2.f * t);
+    dk[(size_t)arg[0] * kdim] += dsx;
+    dk[(size_t)arg[2] * kdim] -= dsx;
+    dk[(size_t)arg[1] * kdim + 1] += dsy;
+    dk[(size_t)arg[3] * kdim + 1] -= dsy;
+  }
+}
+
 }  // namespace
 
 extern "C" int lgb200_attention_bwd(const float* Q, const float* K, const float* V, const float* ctx, const float* dctx,
@@ -767,6 +1010,44 @@ extern "C" int lgb200_assign_dsim_ragged(float* sim, int B, int m, int n, const 
   if (B <= 0 || m <= 0 || n <= 0 || m > Lp || n > Lp || m > 65535) return LGB200_ERR_SHAPE;
   dim3 grid((n + 255) / 256, m, B);
   assign_dsim_kernel<<<grid, 256, 0, lg_stream(stream)>>>(sim, m, n, lse, Lp, lens, gt_assignment, g_pos, r, c);
+  LG_LAUNCH_CHECK();
+  return LGB200_OK;
+}
+
+extern "C" int lgb200_assign_bwd_workspace(int B, int m, int n, long long* n_floats) {
+  if (!n_floats) return LGB200_ERR_NULL;
+  if (B <= 0 || m <= 0 || n <= 0) return LGB200_ERR_SHAPE;
+  const long long P = (m + ABWD_ROWS - 1) / ABWD_ROWS;
+  *n_floats = (long long)B * m + (long long)B * n + (long long)B * P * n;
+  return LGB200_OK;
+}
+
+extern "C" int lgb200_assign_bwd(const float* G, float* sim, int B, int m, int n, const float* lse, int Lp,
+                                 const int32_t* lens, const float* z, float* dz0, float* dz1, float* workspace,
+                                 void* stream) {
+  if (!G || !sim || !lse || !workspace || (z && (!dz0 || !dz1))) return LGB200_ERR_NULL;
+  if (B <= 0 || B > 65535 || m <= 0 || n <= 0 || Lp <= 0 || Lp % 128 || m > Lp || n > Lp) return LGB200_ERR_SHAPE;
+  cudaStream_t st = lg_stream(stream);
+  const int P = (m + ABWD_ROWS - 1) / ABWD_ROWS;
+  float* rsum = workspace;                      // [B, m]
+  float* csum = rsum + (size_t)B * m;           // [B, n]
+  float* part = csum + (size_t)B * n;           // [B, P, n]
+  abwd_sums_kernel<<<dim3((P + 3) / 4, B), 128, 0, st>>>(G, m, n, lens, z, Lp, rsum, part, z ? dz0 : nullptr);
+  LG_LAUNCH_CHECK();
+  abwd_cols_kernel<<<dim3((n + 255) / 256, B), 256, 0, st>>>(G, m, n, lens, z, Lp, part, csum, z ? dz1 : nullptr);
+  LG_LAUNCH_CHECK();
+  abwd_dsim_kernel<<<dim3((m + 7) / 8, B), 256, 0, st>>>(G, sim, m, n, lse, Lp, lens, rsum, csum);
+  LG_LAUNCH_CHECK();
+  return LGB200_OK;
+}
+
+extern "C" int lgb200_posenc_bwd(const float* kpts, int B, int n, int kdim, const float* size, const float* Wr,
+                                 const int32_t* lens, int img, int Lp, const float* dtheta, float* dkpts,
+                                 void* stream) {
+  if (!kpts || !Wr || !dtheta || !dkpts) return LGB200_ERR_NULL;
+  if ((kdim != 2 && kdim != 4) || Lp <= 0 || Lp % 128 || n < 0 || n > Lp || B <= 0 || (img != 0 && img != 1))
+    return LGB200_ERR_SHAPE;
+  posenc_bwd_kernel<<<B, 1024, 0, lg_stream(stream)>>>(kpts, n, kdim, size, Wr, lens, img, Lp, dtheta, dkpts);
   LG_LAUNCH_CHECK();
   return LGB200_OK;
 }

@@ -323,11 +323,13 @@ class LightGlue(nn.Module):
             logits = (lv[:, 0, :m], lv[:, 1, :n])
         return pos_sum, pos_cnt, row_exp, row_arg, col_arg, dust0, dust1, logits
 
-    def _assign_match_bf16(self, lib, d0, d1, layer: int, counts: Optional[torch.Tensor] = None):
+    def _assign_match_bf16(self, lib, d0, d1, layer: int, counts: Optional[torch.Tensor] = None,
+                           keep: Optional[Dict] = None):
         """MatchAssignment `layer` and filter_matches on bf16 descriptors d0 [B,m,256] / d1 [B,n,256], with the kernels
         and arguments of the no-grad bf16 forward's tail (_forward_impl) -> (log_assignment [B,m+1,n+1], m0, m1, ms0,
         ms1).  The bf16 training forward's outputs are therefore the no-grad forward's, bit for bit.  counts: per-pair
-        valid counts (device int32 [2B]) or None."""
+        valid counts (device int32 [2B]) or None.  keep (dict): receives what the backward pass (train.LogAssignFn)
+        needs, as for _log_assignment_of, plus the filter workspace fm_ws."""
         dev = d0.device
         B, m, _ = d0.shape
         n = d1.shape[1]
@@ -363,6 +365,8 @@ class LightGlue(nn.Module):
         check(lib.lgb200_filter_matches(ptr(scores), B, R, C, ptr(lens), float(self.conf.filter_threshold), None, None,
                                         2 * Lp, m, n, ptr(m0), ptr(m1), ptr(ms0), ptr(ms1), ptr(fm_ws), 1, st),
               "filter_matches")
+        if keep is not None:
+            keep.update(z=z, lse=lse, Lp=Lp, lens=lens, md_planes=None, md16=md, fm_ws=fm_ws)
         return scores, m0, m1, ms0, ms1
 
     @staticmethod
@@ -651,8 +655,11 @@ class LightGlue(nn.Module):
         train.TransformerFn -- fp32 kernels forward, hand-written backward kernels + cuBLAS GEMMs backward -- so that
         `ref_descriptors0/1` carry an autograd graph to the descriptors and to every parameter
         (lightglue.py:484-498, :546-547).  conf.checkpointed (:485-494) selects recomputation of the attention
-        operands in the backward pass instead of keeping them.  The matches / log_assignment of the last layer are
-        computed without a graph (the reference's loss reads pred["log_assignment"] detached, :606, :625-630).
+        operands in the backward pass instead of keeping them.  The last layer's MatchAssignment and filter_matches run
+        through train.LogAssignFn, so that `log_assignment` and `matching_scores0/1` carry a graph too (as in the
+        reference: a loss may read them; LightGlue.loss reads log_assignment detached, :606, :625-630).  The staged
+        keypoints (with scales / orientations when add_scale_ori) are inputs of the transformer Function: keypoints0/1,
+        scales0/1 and oris0/1 that require grad receive their gradient through the positional encoding.
         conf.train_precision = "bf16" runs train.TransformerBf16Fn and the bf16 assignment kernels instead.
         data["num_keypoints0/1"] (padded batches): every kernel reads the per-pair counts, the padding's descriptors and
         keypoints are replaced by zeros, and the outputs take the layout of the no-grad forward with the same counts."""
@@ -665,7 +672,6 @@ class LightGlue(nn.Module):
         if not kpts0.is_cuda:
             raise _abi.LightGlueB200Error(
                 "glue_factory_colon_b200.LightGlue runs on CUDA (sm_100a) tensors only; there is no CPU path")
-        lib = _abi.load()
         dev = kpts0.device
         B, m, _ = kpts0.shape
         n = kpts1.shape[1]
@@ -681,7 +687,7 @@ class LightGlue(nn.Module):
             return sz.to(device=dev, dtype=torch.float32).reshape(-1, 2).expand(B, 2).contiguous()
 
         def kpts_of(idx, k):
-            k = k.detach().to(torch.float32)
+            k = k.to(torch.float32)
             if conf.add_scale_ori:  # lightglue.py:436-454
                 sc, ori = data[f"scales{idx}"], data[f"oris{idx}"]
                 sc = sc if sc.dim() == 3 else sc[..., None]
@@ -689,38 +695,21 @@ class LightGlue(nn.Module):
                 k = torch.cat([k, sc.to(k), ori.to(k)], -1)
             return k.contiguous()
 
-        geom = {"k0": kpts_of(0, kpts0), "k1": kpts_of(1, kpts1), "size0": size_of("view0"), "size1": size_of("view1"),
-                "counts": counts_h}
+        k0, k1 = kpts_of(0, kpts0), kpts_of(1, kpts1)
+        geom = {"size0": size_of("view0"), "size1": size_of("view1"), "counts": counts_h}
         desc0 = data["descriptors0"].to(torch.float32)
         desc1 = data["descriptors1"].to(torch.float32)
         assert desc0.shape[-1] == conf.input_dim and desc1.shape[-1] == conf.input_dim
         params = [p for _, p in _train.transformer_params(self)]
         L = conf.n_layers
         if self._train_bf16():  # mixed precision: the bf16 inference kernels forward (conf.train_precision)
-            r0, r1 = _train.TransformerBf16Fn.apply(self, geom, desc0, desc1, *params)
-            with torch.no_grad():
-                scores, m0, m1, ms0, ms1 = self._assign_match_bf16(lib, r0[:, -1], r1[:, -1], L - 1, counts)
-            return {
-                "matches0": m0, "matches1": m1, "matching_scores0": ms0, "matching_scores1": ms1,
-                "ref_descriptors0": r0, "ref_descriptors1": r1, "log_assignment": scores,
-                "prune0": torch.full((B, m), float(L), device=dev), "prune1": torch.full((B, n), float(L), device=dev),
-            }
-        r0, r1 = _train.TransformerFn.apply(self, geom, desc0, desc1, *params)
-        with torch.no_grad():
-            keep: Dict = {}
-            # (fp32-accurate tensor-core kernels, as the rest of the training forward; CUDA cores with LGB200_TRAIN_SIMT_LINEAR=1)
-            self._log_assignment_of(lib, F32 if _train._SIMT_LINEAR else F32X3, r0[:, -1], r1[:, -1], L - 1, None, keep=keep,
-                                    counts=counts)
-            scores = keep["scores"]
-            m0 = torch.empty(B, m, device=dev, dtype=torch.int64)
-            m1 = torch.empty(B, n, device=dev, dtype=torch.int64)
-            ms0 = torch.empty(B, m, device=dev, dtype=torch.float32)
-            ms1 = torch.empty(B, n, device=dev, dtype=torch.float32)
-            fm_ws = torch.empty(B * (m + n + 2), device=dev, dtype=torch.int64)
-            st = torch.cuda.current_stream(dev).cuda_stream
-            check(lib.lgb200_filter_matches(ptr(scores), B, m + 1, n + 1, ptr(keep["lens"]),
-                                            float(conf.filter_threshold), None, None, 0, m, n, ptr(m0), ptr(m1),
-                                            ptr(ms0), ptr(ms1), ptr(fm_ws), 0, st), "filter_matches")
+            r0, r1 = _train.TransformerBf16Fn.apply(self, geom, desc0, desc1, k0, k1, *params)
+        else:
+            r0, r1 = _train.TransformerFn.apply(self, geom, desc0, desc1, k0, k1, *params)
+        a = self.log_assignment[L - 1]
+        scores, m0, m1, ms0, ms1 = _train.LogAssignFn.apply(
+            self, L - 1, counts, r0[:, -1], r1[:, -1], a.final_proj.weight, a.final_proj.bias, a.matchability.weight,
+            a.matchability.bias)
         return {
             "matches0": m0, "matches1": m1, "matching_scores0": ms0, "matching_scores1": ms1,
             "ref_descriptors0": r0, "ref_descriptors1": r1, "log_assignment": scores,

@@ -16,6 +16,10 @@ layer's descriptors in training mode, :588-637 turns them into the deep-supervis
   * `AssignFn`       MatchAssignment of one layer (lightglue.py:272-288) reduced to what NLLLoss reads
     (losses.py:6-26: the sum of log_assignment over the ground-truth matches and the two dustbin vectors).  Forward =
     the library's assignment + reduction kernels; backward = lgb200_assign_dsim (d similarity of the double softmax).
+  * `LogAssignFn`    the training forward's log_assignment / matches / matching_scores of the last layer (lightglue.py:
+    272-288, 294-319) with a graph for losses that read them; backward = lgb200_assign_bwd (any upstream gradient).
+The staged keypoints are inputs of the transformer Functions: with keypoints (scales, orientations) that require grad,
+lgb200_posenc_bwd turns the rotary-angle gradient into their gradient (lightglue.py:28-40, 61-66).
 
 Plain GEMMs of the backward pass (dX = dY.W, dW = dY^T.X) go to cuBLAS -- they are library GEMMs with nothing to fuse --
 as three fp16 tensor-core GEMMs on split planes with fp32 accumulation (_Kern.mm3; LGB200_TRAIN_SGEMM=1: one fp32
@@ -261,6 +265,25 @@ class _Kern:
         xv = x.view(self.B, 2, self.Lp, x.shape[-1])
         return xv[:, 0, : self.m], xv[:, 1, : self.n]
 
+    def posenc(self, geom, Wr, rot, rot16=None):
+        """lgb200_posenc for both images: rot [T,64] fp32 (+ rot16 [T,32] packed fp16) from the staged keypoints."""
+        for img, kk, cnt, sz in ((0, geom["k0"], self.m, geom["size0"]), (1, geom["k1"], self.n, geom["size1"])):
+            check(self.lib.lgb200_posenc(ptr(kk), self.B, cnt, kk.shape[-1], ptr(sz), ptr(Wr), ptr(self.lens), img,
+                                         self.Lp, ptr(rot), ptr(rot16), self.st), "lgb200_posenc")
+
+    def posenc_bwd(self, geom, Wr, dtheta, need):
+        """d staged keypoints [B, cnt, kdim] of image 0 / 1 from the rotary-angle gradient dtheta [T,32]
+        (lgb200_posenc_bwd); None, and nothing launched, where need[img] is False."""
+        out = []
+        for img, kk, cnt, sz in ((0, geom["k0"], self.m, geom["size0"]), (1, geom["k1"], self.n, geom["size1"])):
+            dk = None
+            if need[img]:
+                dk = torch.empty_like(kk)
+                check(self.lib.lgb200_posenc_bwd(ptr(kk), self.B, cnt, kk.shape[-1], ptr(sz), ptr(Wr), ptr(self.lens),
+                                                 img, self.Lp, ptr(dtheta), ptr(dk), self.st), "lgb200_posenc_bwd")
+            out.append(dk)
+        return out
+
 
 def bmm3(A, B, scale):
     """Batched _Kern.mm3: fp32-accurate A.B from plane pairs A [2, b, M, K], B [2, b, K, N] (views may be transposed)
@@ -451,10 +474,13 @@ class TransformerFn(torch.autograd.Function):
     """ref_descriptors0/1 = all layers' outputs of the transformer stack (lightglue.py:456-498)."""
 
     @staticmethod
-    def forward(ctx, model, geom: Dict, desc0, desc1, *params):
+    def forward(ctx, model, geom: Dict, desc0, desc1, k0, k1, *params):
+        """k0 / k1 [B, m / n, kdim]: the staged keypoint rows (coordinates, plus scale and orientation with
+        add_scale_ori) -- inputs, so that their gradient reaches whatever the caller built them from."""
         dev = desc0.device
         B, m, _ = desc0.shape
         n = desc1.shape[1]
+        geom = dict(geom, k0=k0, k1=k1)
         k = _Kern(dev, B, m, n, geom.get("counts"))
         W = model._pack(F32, dev)
         L = model.conf.n_layers
@@ -471,10 +497,7 @@ class TransformerFn(torch.autograd.Function):
         else:
             x = k.pack2(desc0, desc1)
         rot = k.zeros(k.T, 64)
-        kdim = geom["k0"].shape[-1]
-        for img, kk, cnt, sz in ((0, geom["k0"], m, geom["size0"]), (1, geom["k1"], n, geom["size1"])):
-            check(k.lib.lgb200_posenc(ptr(kk), B, cnt, kdim, ptr(sz), ptr(W["wr"]), ptr(k.lens), img, k.Lp, ptr(rot),
-                                      None, k.st), "lgb200_posenc")
+        k.posenc(geom, W["wr"], rot)
         # conf.checkpointed (lightglue.py:485-494): keep only the block inputs and recompute q / k / v / context /
         # message in the backward pass (26 x T KB per layer less); otherwise they are kept, as autograd would
         keep = not bool(model.conf.checkpointed)
@@ -537,13 +560,14 @@ class TransformerFn(torch.autograd.Function):
             dx = dxm + dxa + dxp
         # positional encoding: theta = Wr . normalised keypoints (lightglue.py:61-66)
         grads["wr"] = dtheta.t() @ _posenc_rows(k, geom)
+        need = ctx.needs_input_grad
+        gk0, gk1 = k.posenc_bwd(geom, W["wr"], dtheta, need[4:6])
         if ctx.xin is not None:  # input_proj (lightglue.py:464-465)
             grads["in_w"], grads["in_b"] = dx.t() @ ctx.xin, dx.sum(0)
             dx = dx @ W["in_w"]
         gd0, gd1 = k.unpack(k.mask_rows(dx))
-        need = ctx.needs_input_grad
-        return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None,
-                *[grads[key] if need[4 + j] else None for j, key in enumerate(ctx.keys)])
+        return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None, gk0, gk1,
+                *[grads[key] if need[6 + j] else None for j, key in enumerate(ctx.keys)])
 
 
 # ---- bf16 mixed-precision training (conf.train_precision = "bf16") ------------------------------------------------
@@ -617,10 +641,11 @@ class TransformerBf16Fn(torch.autograd.Function):
     them) with the bf16 inference kernels forward and bf16 tensor-core products backward."""
 
     @staticmethod
-    def forward(ctx, model, geom: Dict, desc0, desc1, *params):
+    def forward(ctx, model, geom: Dict, desc0, desc1, k0, k1, *params):
         dev = desc0.device
         B, m, _ = desc0.shape
         n = desc1.shape[1]
+        geom = dict(geom, k0=k0, k1=k1)
         k = _Kern(dev, B, m, n, geom.get("counts"))
         W = model._pack(BF16, dev)
         L = model.conf.n_layers
@@ -642,10 +667,7 @@ class TransformerBf16Fn(torch.autograd.Function):
             k.mask_rows(x)
         rot = k.zeros(k.T, 64)  # fp32 angles for lgb200_heads_bwd, rot16 for the forward's QKV epilogue (one call)
         rot16 = torch.zeros(k.T, 32, device=dev, dtype=torch.int32)
-        kdim = geom["k0"].shape[-1]
-        for img, kk, cnt, sz in ((0, geom["k0"], m, geom["size0"]), (1, geom["k1"], n, geom["size1"])):
-            check(k.lib.lgb200_posenc(ptr(kk), B, cnt, kdim, ptr(sz), ptr(W["wr"]), ptr(k.lens), img, k.Lp, ptr(rot),
-                                      ptr(rot16), k.st), "lgb200_posenc")
+        k.posenc(geom, W["wr"], rot, rot16)
         keep = not bool(model.conf.checkpointed)
         xs_in, xs_mid, outs, kept = [], [], [], []
         for i in range(L):
@@ -705,13 +727,14 @@ class TransformerBf16Fn(torch.autograd.Function):
             dx = dxm + dxa + dxp
         # positional encoding: theta = Wr . normalised keypoints (lightglue.py:61-66)
         grads["wr"] = dtheta.t() @ _posenc_rows(k, geom)
+        need = ctx.needs_input_grad
+        gk0, gk1 = k.posenc_bwd(geom, W["wr"], dtheta, need[4:6])
         if ctx.xin is not None:  # input_proj (lightglue.py:464-465)
             grads["in_w"], grads["in_b"] = dx.t() @ ctx.xin.float(), dx.sum(0)
             dx = dx @ model.input_proj.weight.detach()
         gd0, gd1 = k.unpack(k.mask_rows(dx))
-        need = ctx.needs_input_grad
-        return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None,
-                *[grads[key] if need[4 + j] else None for j, key in enumerate(ctx.keys)])
+        return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None, gk0, gk1,
+                *[grads[key] if need[6 + j] else None for j, key in enumerate(ctx.keys)])
 
 
 class AssignFn(torch.autograd.Function):
@@ -749,20 +772,7 @@ class AssignFn(torch.autograd.Function):
         dev = d0.device
         x0, x1 = d0.to(torch.float32), d1.to(torch.float32)
         st = torch.cuda.current_stream(dev).cuda_stream
-        mdp, md16 = ctx.md_planes, ctx.md16
-        f32 = torch.float32
-        if md16 is not None:  # bf16: the similarity as one bf16 bmm with fp32 output (bf16 output: ~0.1 at |sim| ~ 30)
-            mv = md16.view(B, 2, Lp, 256)
-            md0, md1 = mv[:, 0, :m], mv[:, 1, :n]
-            sim = torch.bmm(md0, md1.transpose(1, 2), out_dtype=f32).contiguous()
-        elif mdp is None:
-            md0 = torch.addmm(fp_b, x0.reshape(-1, 256), fp_w.t()).view(B, m, 256) * 0.25  # lightglue.py:281-283
-            md1 = torch.addmm(fp_b, x1.reshape(-1, 256), fp_w.t()).view(B, n, 256) * 0.25
-            sim = torch.bmm(md0, md1.transpose(1, 2)).contiguous()
-        else:
-            sim = torch.empty(B, Lp, Lp, device=dev, dtype=torch.float32)
-            check(lib.lgb200_x3_similarity(ptr(mdp), B, Lp, ptr(ctx.lens), ptr(sim), st), "x3_similarity")
-            sim = sim[:, :m, :n].contiguous()
+        sim, md = _assign_similarity(lib, st, x0, x1, fp_w, fp_b, ctx.md_planes, ctx.md16, ctx.lens, Lp)
         g = (g_pos if g_pos is not None else torch.zeros(B, device=dev)).to(torch.float32).contiguous()
         r = (g[:, None] * gt.sum(2)).contiguous()
         c = (g[:, None] * gt.sum(1)).contiguous()
@@ -773,21 +783,6 @@ class AssignFn(torch.autograd.Function):
         else:  # exact zeros outside every pair's valid block
             check(lib.lgb200_assign_dsim_ragged(ptr(sim), B, m, n, ptr(lse), Lp, ptr(counts), ptr(gt), ptr(g), ptr(r),
                                                 ptr(c), st), "assign_dsim_ragged")
-        if md16 is not None:
-            s16 = sim.to(torch.bfloat16)
-            dmd0 = torch.bmm(s16, md1, out_dtype=f32)
-            dmd1 = torch.bmm(s16.transpose(1, 2), md0, out_dtype=f32)
-        elif mdp is None:
-            dmd0 = torch.bmm(sim, md1)
-            dmd1 = torch.bmm(sim.transpose(1, 2), md0)
-        else:  # three fp16 tensor-core products per GEMM, as _Kern.mm3
-            sp = torch.empty(2, B, m, n, device=dev, dtype=torch.float16)
-            inv = torch.empty(2, device=dev, dtype=torch.float32)
-            check(lib.lgb200_split_dynamic(ptr(sim), sim.numel(), ptr(sp), ptr(inv), 0, None, 0, st), "lgb200_split_dynamic")
-            mv = mdp.view(2, B, 2, Lp, 256)
-            mp0, mp1 = mv[:, :, 0, :m], mv[:, :, 1, :n]
-            dmd0 = bmm3(sp, mp1, inv[0] * AI)
-            dmd1 = bmm3(sp.transpose(2, 3), mp0, inv[0] * AI)
         zv = z.view(B, 2, Lp)
         z0, z1 = zv[:, 0, :m], zv[:, 1, :n]
         gd0 = g_d0 if g_d0 is not None else torch.zeros_like(z0)
@@ -795,20 +790,157 @@ class AssignFn(torch.autograd.Function):
         # la = ... + logsigmoid(z0_i) + logsigmoid(z1_j) inside, logsigmoid(-z) in the dustbins (lightglue.py:262-267)
         dz0 = r * torch.sigmoid(-z0) - gd0 * torch.sigmoid(z0)
         dz1 = c * torch.sigmoid(-z1) - gd1 * torch.sigmoid(z1)
-        if counts is not None:  # rows past the counts: no matchability gradient (their z is not a keypoint's)
-            v0 = torch.arange(m, device=dev)[None] < counts[0::2, None]
-            v1 = torch.arange(n, device=dev)[None] < counts[1::2, None]
-            dz0, dz1 = torch.where(v0, dz0, 0.0), torch.where(v1, dz1, 0.0)
-        mw = m_w.reshape(1, 1, 256)
-        gx0 = 0.25 * (dmd0 @ fp_w) + dz0[..., None] * mw
-        gx1 = 0.25 * (dmd1 @ fp_w) + dz1[..., None] * mw
-        if counts is not None:
-            gx0, gx1 = torch.where(v0[..., None], gx0, 0.0), torch.where(v1[..., None], gx1, 0.0)
-        g_fp_w = 0.25 * (dmd0.reshape(-1, 256).t() @ x0.reshape(-1, 256) + dmd1.reshape(-1, 256).t() @ x1.reshape(-1, 256))
-        g_fp_b = 0.25 * (dmd0.sum((0, 1)) + dmd1.sum((0, 1)))
-        g_m_w = ((dz0[..., None] * x0).sum((0, 1)) + (dz1[..., None] * x1).sum((0, 1))).reshape(m_w.shape)
-        g_m_b = (dz0.sum() + dz1.sum()).reshape(1)
-        return None, None, None, None, gx0, gx1, g_fp_w, g_fp_b, g_m_w, g_m_b
+        return (None, None, None, None,
+                *_assign_input_grads(lib, st, sim, dz0, dz1, x0, x1, fp_w, m_w, md, ctx.md_planes, Lp, counts))
+
+
+def _assign_similarity(lib, st, x0, x1, fp_w, fp_b, mdp, md16, lens, Lp):
+    """The similarity [B,m,n] fp32 of MatchAssignment (lightglue.py:281-284) recomputed for a backward pass from what
+    the forward kept -> (sim, (md0, md1)); (md0, md1) = final_proj(desc) / 4 for the d md products (None with the
+    split planes mdp of the x3 mode).  md16: the bf16 forward's md."""
+    B, m, _ = x0.shape
+    n = x1.shape[1]
+    f32 = torch.float32
+    if md16 is not None:  # bf16: the similarity as one bf16 bmm with fp32 output (bf16 output: ~0.1 at |sim| ~ 30)
+        mv = md16.view(B, 2, Lp, 256)
+        md0, md1 = mv[:, 0, :m], mv[:, 1, :n]
+        return torch.bmm(md0, md1.transpose(1, 2), out_dtype=f32).contiguous(), (md0, md1)
+    if mdp is None:
+        md0 = torch.addmm(fp_b, x0.reshape(-1, 256), fp_w.t()).view(B, m, 256) * 0.25  # lightglue.py:281-283
+        md1 = torch.addmm(fp_b, x1.reshape(-1, 256), fp_w.t()).view(B, n, 256) * 0.25
+        return torch.bmm(md0, md1.transpose(1, 2)).contiguous(), (md0, md1)
+    sim = torch.empty(B, Lp, Lp, device=x0.device, dtype=f32)
+    check(lib.lgb200_x3_similarity(ptr(mdp), B, Lp, ptr(lens), ptr(sim), st), "x3_similarity")
+    return sim[:, :m, :n].contiguous(), None
+
+
+def _assign_input_grads(lib, st, sim, dz0, dz1, x0, x1, fp_w, m_w, md, mdp, Lp, counts):
+    """Backward of MatchAssignment (lightglue.py:272-288) from d sim [B,m,n] (in sim) and the matchability logits'
+    gradients dz0 [B,m] / dz1 [B,n] to (d desc0, d desc1, d final_proj.weight, d final_proj.bias, d matchability.weight,
+    d matchability.bias).  md / mdp as returned by / given to _assign_similarity; counts: rows past them get 0."""
+    B, m, n = sim.shape
+    dev = sim.device
+    f32 = torch.float32
+    if md is not None and md[0].dtype == torch.bfloat16:
+        md0, md1 = md
+        s16 = sim.to(torch.bfloat16)
+        dmd0 = torch.bmm(s16, md1, out_dtype=f32)
+        dmd1 = torch.bmm(s16.transpose(1, 2), md0, out_dtype=f32)
+    elif mdp is None:
+        md0, md1 = md
+        dmd0 = torch.bmm(sim, md1)
+        dmd1 = torch.bmm(sim.transpose(1, 2), md0)
+    else:  # three fp16 tensor-core products per GEMM, as _Kern.mm3
+        sp = torch.empty(2, B, m, n, device=dev, dtype=torch.float16)
+        inv = torch.empty(2, device=dev, dtype=torch.float32)
+        check(lib.lgb200_split_dynamic(ptr(sim), sim.numel(), ptr(sp), ptr(inv), 0, None, 0, st), "lgb200_split_dynamic")
+        mv = mdp.view(2, B, 2, Lp, 256)
+        mp0, mp1 = mv[:, :, 0, :m], mv[:, :, 1, :n]
+        dmd0 = bmm3(sp, mp1, inv[0] * AI)
+        dmd1 = bmm3(sp.transpose(2, 3), mp0, inv[0] * AI)
+    if counts is not None:  # rows past the counts: no matchability gradient (their z is not a keypoint's)
+        v0 = torch.arange(m, device=dev)[None] < counts[0::2, None]
+        v1 = torch.arange(n, device=dev)[None] < counts[1::2, None]
+        dz0, dz1 = torch.where(v0, dz0, 0.0), torch.where(v1, dz1, 0.0)
+    mw = m_w.reshape(1, 1, 256)
+    gx0 = 0.25 * (dmd0 @ fp_w) + dz0[..., None] * mw
+    gx1 = 0.25 * (dmd1 @ fp_w) + dz1[..., None] * mw
+    if counts is not None:
+        gx0, gx1 = torch.where(v0[..., None], gx0, 0.0), torch.where(v1[..., None], gx1, 0.0)
+    g_fp_w = 0.25 * (dmd0.reshape(-1, 256).t() @ x0.reshape(-1, 256) + dmd1.reshape(-1, 256).t() @ x1.reshape(-1, 256))
+    g_fp_b = 0.25 * (dmd0.sum((0, 1)) + dmd1.sum((0, 1)))
+    g_m_w = ((dz0[..., None] * x0).sum((0, 1)) + (dz1[..., None] * x1).sum((0, 1))).reshape(m_w.shape)
+    g_m_b = (dz0.sum() + dz1.sum()).reshape(1)
+    return gx0, gx1, g_fp_w, g_fp_b, g_m_w, g_m_b
+
+
+class LogAssignFn(torch.autograd.Function):
+    """The training forward's tail: MatchAssignment `layer` (lightglue.py:272-288) and filter_matches (:294-319) on the
+    last layer's descriptors d0 / d1 -> (log_assignment [B,m+1,n+1], matches0, matches1, matching_scores0,
+    matching_scores1), with the kernels and arguments the step used before it had a graph, so the values are the same
+    bits.  log_assignment and the matching scores are differentiable w.r.t. d0, d1 and the final_proj / matchability
+    parameters; the matches are not.  counts (device int32 [2B] or None): per-pair valid counts of a padded batch.
+
+    Backward: G = d loss / d log_assignment, plus the matching-score terms as autograd differentiates the reference's
+    filter_matches -- ms0_i = exp(la[i, m0_i]) on mutual rows, ms1_j = exp(la[m1_j, j]) on mutual columns (below the
+    threshold too), 0 elsewhere -- then lgb200_assign_bwd on the recomputed similarity, then AssignFn's tail.  The
+    forward keeps z, lse, the filter workspace (the packed row / column maxima) and what the similarity is recomputed
+    from (AssignFn's choice); nothing runs unless the loss reads these outputs."""
+
+    @staticmethod
+    def forward(ctx, model, layer: int, counts, d0, d1, fp_w, fp_b, m_w, m_b):
+        lib = _abi.load()
+        keep: Dict = {}
+        bf = model._train_bf16()
+        if bf:
+            scores, m0, m1, ms0, ms1 = model._assign_match_bf16(lib, d0, d1, layer, counts, keep=keep)
+        else:
+            # (fp32-accurate tensor-core kernels, as the rest of the training forward; CUDA cores with
+            # LGB200_TRAIN_SIMT_LINEAR=1)
+            dev = d0.device
+            B, m, _ = d0.shape
+            n = d1.shape[1]
+            model._log_assignment_of(lib, F32 if _SIMT_LINEAR else F32X3, d0, d1, layer, None, keep=keep, counts=counts)
+            scores = keep["scores"]
+            m0 = torch.empty(B, m, device=dev, dtype=torch.int64)
+            m1 = torch.empty(B, n, device=dev, dtype=torch.int64)
+            ms0 = torch.empty(B, m, device=dev, dtype=torch.float32)
+            ms1 = torch.empty(B, n, device=dev, dtype=torch.float32)
+            keep["fm_ws"] = torch.empty(B * (m + n + 2), device=dev, dtype=torch.int64)
+            st = torch.cuda.current_stream(dev).cuda_stream
+            check(lib.lgb200_filter_matches(ptr(scores), B, m + 1, n + 1, ptr(keep["lens"]),
+                                            float(model.conf.filter_threshold), None, None, 0, m, n, ptr(m0), ptr(m1),
+                                            ptr(ms0), ptr(ms1), ptr(keep["fm_ws"]), 0, st), "filter_matches")
+        ctx.save_for_backward(d0, d1, fp_w, fp_b, m_w, keep["z"], keep["lse"], keep["fm_ws"])
+        ctx.counts, ctx.Lp = counts, keep["Lp"]
+        ctx.md_planes, ctx.lens = (None, keep["lens"]) if (_SGEMM or bf) else (keep["md_planes"], keep["lens"])
+        ctx.md16 = keep["md16"] if bf else None
+        ctx.mark_non_differentiable(m0, m1)
+        return scores, m0, m1, ms0, ms1
+
+    @staticmethod
+    def backward(ctx, g_la, _g_m0, _g_m1, g_ms0, g_ms1):
+        d0, d1, fp_w, fp_b, m_w, z, lse, fm_ws = ctx.saved_tensors
+        lib = _abi.load()
+        B, m, _ = d0.shape
+        n = d1.shape[1]
+        Lp, counts = ctx.Lp, ctx.counts
+        dev = d0.device
+        st = torch.cuda.current_stream(dev).cuda_stream
+        G = torch.zeros(B, m + 1, n + 1, device=dev, dtype=torch.float32)
+        if g_la is not None:
+            G.copy_(g_la)
+        if g_ms0 is not None or g_ms1 is not None:
+            # the raw mutual pairs: lgb200_filter_matches again on the packed maxima the forward left in fm_ws, with a
+            # threshold below every score (scores are >= 0), so every mutual pair is a match
+            mm0 = torch.empty(B, m, device=dev, dtype=torch.int64)
+            mm1 = torch.empty(B, n, device=dev, dtype=torch.int64)
+            ms0 = torch.empty(B, m, device=dev, dtype=torch.float32)
+            ms1 = torch.empty(B, n, device=dev, dtype=torch.float32)
+            check(lib.lgb200_filter_matches(None, B, m + 1, n + 1, ptr(ctx.lens), -1.0, None, None, 0, m, n, ptr(mm0),
+                                            ptr(mm1), ptr(ms0), ptr(ms1), ptr(fm_ws), 1, st), "filter_matches")
+            bi = torch.arange(B, device=dev)[:, None]
+            # rows, then columns: two index_put_ calls, each with distinct indices, so sums into one entry of G have a
+            # fixed order (a row / column without a mutual pair adds an exact 0)
+            if g_ms0 is not None:
+                ii = torch.arange(m, device=dev)[None].expand(B, m)
+                G.index_put_((bi.expand(B, m), ii, mm0.clamp(min=0)), torch.where(mm0 >= 0, g_ms0 * ms0, 0.0),
+                             accumulate=True)
+            if g_ms1 is not None:
+                jj = torch.arange(n, device=dev)[None].expand(B, n)
+                G.index_put_((bi.expand(B, n), mm1.clamp(min=0), jj), torch.where(mm1 >= 0, g_ms1 * ms1, 0.0),
+                             accumulate=True)
+        x0, x1 = d0.to(torch.float32), d1.to(torch.float32)
+        sim, md = _assign_similarity(lib, st, x0, x1, fp_w, fp_b, ctx.md_planes, ctx.md16, ctx.lens, Lp)
+        dz0 = torch.empty(B, m, device=dev, dtype=torch.float32)
+        dz1 = torch.empty(B, n, device=dev, dtype=torch.float32)
+        n_ws = C.c_longlong(0)
+        check(lib.lgb200_assign_bwd_workspace(B, m, n, C.byref(n_ws)), "lgb200_assign_bwd_workspace")
+        ws = torch.empty(n_ws.value, device=dev, dtype=torch.float32)
+        check(lib.lgb200_assign_bwd(ptr(G), ptr(sim), B, m, n, ptr(lse), Lp, ptr(counts), ptr(z), ptr(dz0), ptr(dz1),
+                                    ptr(ws), st), "lgb200_assign_bwd")
+        return (None, None, None,
+                *_assign_input_grads(lib, st, sim, dz0, dz1, x0, x1, fp_w, m_w, md, ctx.md_planes, Lp, counts))
 
 
 def wants_grad(model, data=None) -> bool:
@@ -818,4 +950,5 @@ def wants_grad(model, data=None) -> bool:
     if any(p.requires_grad for p in model.parameters()):
         return True
     return data is not None and any(
-        isinstance(data.get(kk), torch.Tensor) and data[kk].requires_grad for kk in ("descriptors0", "descriptors1"))
+        isinstance(data.get(kk), torch.Tensor) and data[kk].requires_grad
+        for kk in ("descriptors0", "descriptors1", "keypoints0", "keypoints1", "scales0", "scales1", "oris0", "oris1"))

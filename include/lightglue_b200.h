@@ -367,6 +367,28 @@ int lgb200_assign_dsim(float* sim, int B, int m, int n, const float* lse, int Lp
 int lgb200_assign_dsim_ragged(float* sim, int B, int m, int n, const float* lse, int Lp, const int32_t* lens,
                               const uint8_t* gt_assignment, const float* g_pos, const float* r, const float* c,
                               void* stream);
+/* lgb200_assign_bwd: backward of sigmoid_log_double_softmax (lightglue.py:257-269) for ANY upstream gradient
+ *   G [B,m+1,n+1] fp32 = d loss / d log_assignment in the forward's layout (dustbin column n, dustbin row m).  Pair b
+ *   uses rows i < n0 = lens[2b] and columns j < n1 = lens[2b+1] (lens NULL: n0 = m, n1 = n; an empty side is allowed);
+ *   R_i / C_j are the row / column sums of G over that block.  sim [B,m,n] (the recomputed similarity) is replaced in
+ *   place by d sim = 2 G_ij - R_i exp(sim_ij - lse0_i) - C_j exp(sim_ij - lse1_j) inside the block and exactly 0
+ *   outside it; lse as written by lgb200_assign_lse ([S,Lp]: rows of image 0, columns of image 1).  z [S,Lp]
+ *   (matchability logits, nullable): then dz0 [B,m] = R_i sigmoid(-z0_i) - G_{i,n} sigmoid(z0_i) and dz1 [B,n] =
+ *   C_j sigmoid(-z1_j) - G_{m,j} sigmoid(z1_j), 0 past the counts.  Nothing outside the valid block (and its
+ *   dustbin entries) is read.  No atomics: bit-reproducible.  workspace: lgb200_assign_bwd_workspace(B, m, n) floats.
+ * lgb200_assign_bwd_workspace: *n_floats = B m + B n + B ceil(m / 32) n (row sums, column sums, per-warp column
+ *   partials). */
+int lgb200_assign_bwd(const float* G, float* sim, int B, int m, int n, const float* lse, int Lp, const int32_t* lens,
+                      const float* z, float* dz0, float* dz1, float* workspace, void* stream);
+int lgb200_assign_bwd_workspace(int B, int m, int n, long long* n_floats);
+/* lgb200_posenc_bwd: gradient w.r.t. the keypoints of lgb200_posenc with the same kpts / B / n / kdim / size / Wr /
+ *   lens / img / Lp.  dtheta [S,Lp,32] = gradient of the rotary angles (what lgb200_heads_bwd accumulates);
+ *   dkpts [B,n,kdim] receives d kpts: through normalize_keypoints (lightglue.py:28-40) on the two coordinates -- with
+ *   size NULL also through the extent 1 + max - min of the valid points, to the first arg-maximum / arg-minimum (torch's
+ *   tie rule; the x extent wins a tie between W and H) -- and unchanged on scale / orientation.  Rows >= lens[2b+img]
+ *   are 0.  Gradients w.r.t. size are not formed. */
+int lgb200_posenc_bwd(const float* kpts, int B, int n, int kdim, const float* size, const float* Wr,
+                      const int32_t* lens, int img, int Lp, const float* dtheta, float* dkpts, void* stream);
 
 #ifdef __cplusplus
 }
