@@ -1,15 +1,10 @@
 // Backward kernels of the training path (SURVEY.md 8(f) rank 2: "training forward + loss", the part the reference
-// gets from autograd, lightglue.py:484-498, 588-637).  Everything is fp32-accurate; the training step is not the
-// benchmarked path, what counts here is that the fused forward ops have fused backward ops (nothing N x M is materialised
-// by the attention backward either) and that gradients agree with the reference's autograd.  The attention backward that
-// ships is the tcgen05 kernel of lg_x3_attn_bwd.cu (lgb200_attention_bwd dispatches to it); the kernels in this file are
-// its predecessors, kept as cross-checks: 3xTF32 warp MMAs (`*_tc_kernel`, LGB200_ATTN_BWD_MMASYNC=1) and CUDA cores
-// (LGB200_ATTN_BWD_SIMT=1).  Plain GEMMs of the backward (dX = dY.W, dW = dY^T.X) are left to cuBLAS on the host side
-// (glue_factory_colon_b200/train.py: three fp16 tensor-core GEMMs on split planes).
+// gets from autograd, lightglue.py:484-498, 588-637).  What counts here is that the fused forward ops have fused
+// backward ops (nothing N x M is materialised by the attention backward either) and that gradients agree with the
+// reference's autograd.  The attention backward is the tcgen05 kernel of lg_x3_attn_bwd.cu: lgb200_attention_bwd runs
+// its fp32-accurate split-fp16 instantiation, lgb200_attention_bwd_bf16 its bf16 one.  Plain GEMMs of the backward
+// (dX = dY.W, dW = dY^T.X) are left to cuBLAS on the host side (glue_factory_colon_b200/train.py).
 //
-//   attn_bwd_stats_kernel   per query row: lse (log2 domain) and delta = <dO, O>          (flash-attention backward,
-//   attn_bwd_kernel<false>  dQ for 64 queries, sweeping the keys                           recomputing S tile by tile)
-//   attn_bwd_kernel<true>   dK, dV for 64 keys, sweeping the queries that attend to them
 //   heads_bwd_kernel        head-major dq/dk/dv -> token-major d(qkv) incl. the transposed rotary embedding and the
 //                           gradient of the rotary angles (-> posenc.Wr)                   lightglue.py:43-50, 157-161
 //   ln_gelu_bwd_kernel      GELU(erf)' . LayerNorm backward, d gamma / d beta partials     lightglue.py:144-149
@@ -18,462 +13,8 @@
 //   posenc_bwd_kernel       d keypoints through normalize_keypoints and posenc.Wr            lightglue.py:28-40, 61-66
 #include "lg_common.cuh"
 #include "lg_internal.cuh"
-#include <stdlib.h>
 
 namespace {
-
-constexpr int AB_T = 64;          // rows per tile on both sides
-constexpr int AB_LD = AB_T + 4;   // padded leading dimension (keeps float4 alignment, spreads banks)
-constexpr float LN2 = 0.69314718055994530942f;
-
-// 6 x 17 KB + 512 B = 102.5 KB: two CTAs (16 warps) per SM.  The transposed other-tiles Yt / Wt are dead once the two
-// score products are in registers; dS^T and P^T are written over them (one extra barrier per tile) -- with separate
-// buffers (139 KB, one CTA per SM) the kernels ran at 28 TFLOP/s of fp32 FMA.
-struct AbSmem {
-  float Xt[LG_DH][AB_LD];  // own X   [d][row]
-  float Ut[LG_DH][AB_LD];  // own U   [d][row]
-  float Yt[LG_DH][AB_LD];  // other Y [d][n]; then dS^T [n][m]
-  float Wt[LG_DH][AB_LD];  // other W [d][n]; then P^T  [n][m] (dK/dV only)
-  float Ys[AB_T][AB_LD];   // other Y [n][d]
-  float Ws[AB_T][AB_LD];   // other W [n][d]   (dK/dV only)
-  float lse[AB_T], dlt[AB_T];  // statistics of the query rows of the current other-tile (dK/dV only)
-};
-static_assert(LG_DH == AB_T, "dS^T / P^T reuse the [d][n] buffers");
-
-// 64 rows x 64 floats -> transposed [d][row] and (optionally) row-major [row][d]
-__device__ __forceinline__ void ab_load(const float* __restrict__ src, size_t row_stride, float (*T_)[AB_LD],
-                                        float (*R_)[AB_LD]) {
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int idx = threadIdx.x + 256 * i, m = idx >> 4, d4 = (idx & 15) * 4;
-    const float4 v = *reinterpret_cast<const float4*>(src + (size_t)m * row_stride + d4);
-    T_[d4 + 0][m] = v.x; T_[d4 + 1][m] = v.y; T_[d4 + 2][m] = v.z; T_[d4 + 3][m] = v.w;
-    if (R_) *reinterpret_cast<float4*>(&R_[m][d4]) = v;
-  }
-}
-
-// c[i][j] += sum_d A[d][ty*4+i] * B[d][tx*4+j]
-__device__ __forceinline__ void ab_mma_t(const float (*A)[AB_LD], const float (*B)[AB_LD], int ty, int tx,
-                                         float c[4][4]) {
-#pragma unroll 8
-  for (int d = 0; d < LG_DH; ++d) {
-    const float4 a = *reinterpret_cast<const float4*>(&A[d][ty * 4]);
-    const float4 b = *reinterpret_cast<const float4*>(&B[d][tx * 4]);
-    const float av[4] = {a.x, a.y, a.z, a.w}, bv[4] = {b.x, b.y, b.z, b.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) c[i][j] = fmaf(av[i], bv[j], c[i][j]);
-  }
-}
-
-__global__ void __launch_bounds__(256, 2) attn_bwd_stats_kernel(const float* __restrict__ Q, const float* __restrict__ K,
-                                                             const float* __restrict__ O, const float* __restrict__ dO,
-                                                             int Lp, const int32_t* __restrict__ lens, int kv_xor,
-                                                             float* __restrict__ lse2, float* __restrict__ dlt) {
-  extern __shared__ __align__(16) unsigned char ab_raw[];
-  AbSmem& sm = *reinterpret_cast<AbSmem*>(ab_raw);
-  const int s = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * AB_T;
-  const int nq = lens ? lens[s] : Lp;
-  if (q0 >= nq) return;
-  const int skv = s ^ kv_xor;
-  const int nk = lens ? lens[skv] : Lp;
-  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  ab_load(Q + (((size_t)s * LG_HEADS + h) * Lp + q0) * LG_DH, LG_DH, sm.Xt, nullptr);
-  const float* Kh = K + ((size_t)skv * LG_HEADS + h) * Lp * LG_DH;
-  float mrow[4], lrow[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { mrow[i] = -INFINITY; lrow[i] = 0.f; }
-  for (int n0 = 0; n0 < nk; n0 += AB_T) {
-    __syncthreads();
-    ab_load(Kh + (size_t)n0 * LG_DH, LG_DH, sm.Yt, nullptr);
-    __syncthreads();
-    float sc[4][4] = {};
-    ab_mma_t(sm.Xt, sm.Yt, ty, tx, sc);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      float mx = -INFINITY;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        if (n0 + tx * 4 + j >= nk) sc[i][j] = -INFINITY;
-        mx = fmaxf(mx, sc[i][j]);
-      }
-      for (int ofs = 8; ofs; ofs >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, ofs));
-      const float mnew = fmaxf(mrow[i], mx);
-      const float msafe = mnew == -INFINITY ? 0.f : mnew;
-      float rs = 0.f;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) rs += exp2f(sc[i][j] - msafe);
-      for (int ofs = 8; ofs; ofs >>= 1) rs += __shfl_xor_sync(0xffffffffu, rs, ofs);
-      lrow[i] = lrow[i] * exp2f(mrow[i] - msafe) + rs;
-      mrow[i] = mnew;
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int l = q0 + ty * 4 + i;
-    const size_t off = ((size_t)s * Lp + l) * LG_D + h * LG_DH + tx * 4;
-    const float4 o = *reinterpret_cast<const float4*>(O + off);
-    const float4 g = *reinterpret_cast<const float4*>(dO + off);
-    float d = o.x * g.x + o.y * g.y + o.z * g.z + o.w * g.w;
-    for (int ofs = 8; ofs; ofs >>= 1) d += __shfl_xor_sync(0xffffffffu, d, ofs);
-    if (tx == 0) {
-      const size_t r = ((size_t)s * LG_HEADS + h) * Lp + l;
-      lse2[r] = lrow[i] > 0.f ? mrow[i] + log2f(lrow[i]) : INFINITY;  // no keys: every probability is 0
-      dlt[r] = d;
-    }
-  }
-}
-
-// DKV = false: own rows = queries of sequence s (X = Q, U = dO), other rows = keys of s ^ kv_xor (Y = K, W = V);
-//              out1 = dQ.
-// DKV = true:  own rows = keys of sequence s (X = K, U = V), other rows = the queries of s ^ kv_xor, which are the
-//              ones that attend to these keys (Y = Q, W = dO); out1 = dK, out2 = dV.
-// With logits a = ln2 . <q', k'> (q' carries log2(e)/sqrt(d)): P = exp2(<q',k'> - lse2[query]),
-// dS = P (<dO, v> - delta[query]), dq' = ln2 . dS k', dk' = ln2 . dS^T q', dv = P^T dO.
-template <bool DKV>
-__global__ void __launch_bounds__(256, 2) attn_bwd_kernel(const float* __restrict__ Q, const float* __restrict__ K,
-                                                       const float* __restrict__ V, const float* __restrict__ dO,
-                                                       int Lp, const int32_t* __restrict__ lens, int kv_xor,
-                                                       const float* __restrict__ lse2, const float* __restrict__ dlt,
-                                                       float* __restrict__ out1, float* __restrict__ out2) {
-  extern __shared__ __align__(16) unsigned char ab_raw[];
-  AbSmem& sm = *reinterpret_cast<AbSmem*>(ab_raw);
-  const int s = blockIdx.z, h = blockIdx.y, r0 = blockIdx.x * AB_T;
-  const int so = s ^ kv_xor;
-  const int n_own = lens ? lens[s] : Lp, n_oth = lens ? lens[so] : Lp;
-  if (r0 >= n_own) return;  // (outputs are zero-filled by the caller)
-  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  const size_t own_h = (((size_t)s * LG_HEADS + h) * Lp + r0) * LG_DH;   // head-major offset of the own tile
-  const size_t own_t = ((size_t)s * Lp + r0) * LG_D + h * LG_DH;         // token-major offset of the own tile
-  const size_t oth_h = ((size_t)so * LG_HEADS + h) * Lp * LG_DH;
-  const size_t oth_t = (size_t)so * Lp * LG_D + h * LG_DH;
-  if (!DKV) {
-    ab_load(Q + own_h, LG_DH, sm.Xt, nullptr);
-    ab_load(dO + own_t, LG_D, sm.Ut, nullptr);
-  } else {
-    ab_load(K + own_h, LG_DH, sm.Xt, nullptr);
-    ab_load(V + own_h, LG_DH, sm.Ut, nullptr);
-  }
-  float lse_own[4], dlt_own[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    lse_own[i] = dlt_own[i] = 0.f;
-    if (!DKV && r0 + ty * 4 + i < n_own) {
-      const size_t r = ((size_t)s * LG_HEADS + h) * Lp + r0 + ty * 4 + i;
-      lse_own[i] = lse2[r];
-      dlt_own[i] = dlt[r];
-    }
-  }
-  float acc1[4][4] = {}, acc2[4][4] = {};
-  for (int n0 = 0; n0 < n_oth; n0 += AB_T) {
-    __syncthreads();  // the previous tile is fully consumed (also orders the own-tile stores on iteration 0)
-    if (!DKV) {
-      ab_load(K + oth_h + (size_t)n0 * LG_DH, LG_DH, sm.Yt, sm.Ys);
-      ab_load(V + oth_h + (size_t)n0 * LG_DH, LG_DH, sm.Wt, nullptr);
-    } else {
-      ab_load(Q + oth_h + (size_t)n0 * LG_DH, LG_DH, sm.Yt, sm.Ys);
-      ab_load(dO + oth_t + (size_t)n0 * LG_D, LG_D, sm.Wt, sm.Ws);
-      if (tid < AB_T) {
-        const bool ok = n0 + tid < n_oth;
-        const size_t r = ((size_t)so * LG_HEADS + h) * Lp + n0 + tid;
-        sm.lse[tid] = ok ? lse2[r] : INFINITY;
-        sm.dlt[tid] = ok ? dlt[r] : 0.f;
-      }
-    }
-    __syncthreads();
-    float sc[4][4] = {}, dp[4][4] = {};
-    ab_mma_t(sm.Xt, sm.Yt, ty, tx, sc);
-    ab_mma_t(sm.Ut, sm.Wt, ty, tx, dp);
-    float (*Dt)[AB_LD] = sm.Yt;  // dS^T [n][m]
-    float (*Pt)[AB_LD] = sm.Wt;  // P^T  [n][m]
-    __syncthreads();             // every thread has read Yt / Wt
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const bool valid = (r0 + ty * 4 + i < n_own) && (n0 + tx * 4 + j < n_oth);
-        const float lq = DKV ? sm.lse[tx * 4 + j] : lse_own[i];
-        const float dq = DKV ? sm.dlt[tx * 4 + j] : dlt_own[i];
-        const float p = valid ? exp2f(sc[i][j] - lq) : 0.f;
-        const float ds = valid ? p * (dp[i][j] - dq) : 0.f;
-        Dt[tx * 4 + j][ty * 4 + i] = ds;
-        if (DKV) Pt[tx * 4 + j][ty * 4 + i] = p;
-      }
-    __syncthreads();
-#pragma unroll 8
-    for (int n = 0; n < AB_T; ++n) {
-      const float4 a = *reinterpret_cast<const float4*>(&Dt[n][ty * 4]);
-      const float4 b = *reinterpret_cast<const float4*>(&sm.Ys[n][tx * 4]);
-      const float av[4] = {a.x, a.y, a.z, a.w}, bv[4] = {b.x, b.y, b.z, b.w};
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc1[i][j] = fmaf(av[i], bv[j], acc1[i][j]);
-      if (DKV) {
-        const float4 p = *reinterpret_cast<const float4*>(&Pt[n][ty * 4]);
-        const float4 w = *reinterpret_cast<const float4*>(&sm.Ws[n][tx * 4]);
-        const float pv[4] = {p.x, p.y, p.z, p.w}, wv[4] = {w.x, w.y, w.z, w.w};
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) acc2[i][j] = fmaf(pv[i], wv[j], acc2[i][j]);
-      }
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const size_t off = own_h + (size_t)(ty * 4 + i) * LG_DH + tx * 4;
-    *reinterpret_cast<float4*>(out1 + off) =
-        make_float4(acc1[i][0] * LN2, acc1[i][1] * LN2, acc1[i][2] * LN2, acc1[i][3] * LN2);
-    if (DKV) *reinterpret_cast<float4*>(out2 + off) = make_float4(acc2[i][0], acc2[i][1], acc2[i][2], acc2[i][3]);
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// Tensor-core variant of the three attention-backward kernels: the four 64 x 64 x 64 products of a tile pair run as
-// 3xTF32 warp MMAs (mma.sync m16n8k8: x = hi + lo with hi = tf32(x); lo.hi + hi.lo + hi.hi accumulated in fp32, the
-// dropped lo.lo term is 2^-22 relative), i.e. fp32-accurate like the forward's split-fp16 tcgen05 kernels -- the
-// kernel-level gradient tests keep their 2e-5 bound.  All operands stay ROW-major [row][64] in shared memory (leading
-// dimension 68): with the contraction over d both fragments are read as [row g][k t] (bank 4g + t: conflict-free),
-// with the contraction over the other rows the B fragment is read as [k t][column g] of the same tile, so no
-// transposed copies exist and dS / P get buffers of their own (one block barrier less per tile).
-// 8 warps = 4 row blocks of 16 x 2 column halves of 32; 6 x 17 KB + 512 B of shared memory, two CTAs per SM.
-// LGB200_ATTN_BWD_SIMT=1 selects the CUDA-core kernels above (kept for A/B timing and as a cross-check).
-constexpr int TB_LD = AB_T + 4;
-struct TbSmem {
-  float X[AB_T][TB_LD];  // own rows:   Q (dQ kernel, statistics) | K (dK/dV kernel)
-  float U[AB_T][TB_LD];  // own rows:   dO                        | V
-  float Y[AB_T][TB_LD];  // other rows: K                         | Q
-  float W[AB_T][TB_LD];  // other rows: V                         | dO
-  float D[AB_T][TB_LD];  // dS [own][other]
-  float P[AB_T][TB_LD];  // P  [own][other]   (dK/dV kernel)
-  float lse[AB_T], dlt[AB_T];
-};
-
-__device__ __forceinline__ void tf32_split(float x, uint32_t& hi, uint32_t& lo) {
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hi) : "f"(x));
-  lo = __float_as_uint(x - __uint_as_float(hi));  // exact; the MMA reads its upper 19 bits
-}
-
-__device__ __forceinline__ void mma_tf32(float c[4], const uint32_t a[4], const uint32_t b[2]) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
-}
-
-// c[nt] (rows m0 + g, m0 + g + 8; columns n0 + 8 nt + 2t, + 1) += sum_k A[m][k] . B(k, n), k = 0..63.
-// BT: B is stored [n][k] (contraction over the columns of both tiles); !BT: B is stored [k][n].
-template <bool BT>
-__device__ __forceinline__ void tb_gemm(const float (*A)[TB_LD], int m0, const float (*B)[TB_LD], int n0, int g, int t,
-                                        float c[4][4]) {
-#pragma unroll
-  for (int k0 = 0; k0 < AB_T; k0 += 8) {
-    uint32_t ah[4], al[4];
-    tf32_split(A[m0 + g][k0 + t], ah[0], al[0]);
-    tf32_split(A[m0 + g + 8][k0 + t], ah[1], al[1]);
-    tf32_split(A[m0 + g][k0 + t + 4], ah[2], al[2]);
-    tf32_split(A[m0 + g + 8][k0 + t + 4], ah[3], al[3]);
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt) {
-      const int n = n0 + nt * 8 + g;
-      uint32_t bh[2], bl[2];
-      tf32_split(BT ? B[n][k0 + t] : B[k0 + t][n], bh[0], bl[0]);
-      tf32_split(BT ? B[n][k0 + t + 4] : B[k0 + t + 4][n], bh[1], bl[1]);
-      mma_tf32(c[nt], al, bh);
-      mma_tf32(c[nt], ah, bl);
-      mma_tf32(c[nt], ah, bh);
-    }
-  }
-}
-
-// 64 rows x 64 floats, row-major; rows >= n_valid are zero-filled (padding rows of the activations are not defined)
-__device__ __forceinline__ void tb_load(const float* __restrict__ src, size_t row_stride, int n_valid,
-                                        float (*R_)[TB_LD]) {
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int idx = threadIdx.x + 256 * i, m = idx >> 4, d4 = (idx & 15) * 4;
-    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (m < n_valid) v = *reinterpret_cast<const float4*>(src + (size_t)m * row_stride + d4);
-    *reinterpret_cast<float4*>(&R_[m][d4]) = v;
-  }
-}
-
-__global__ void __launch_bounds__(256, 2) attn_bwd_stats_tc_kernel(const float* __restrict__ Q, const float* __restrict__ K,
-                                                                const float* __restrict__ O, const float* __restrict__ dO,
-                                                                int Lp, const int32_t* __restrict__ lens, int kv_xor,
-                                                                float* __restrict__ lse2, float* __restrict__ dlt) {
-  extern __shared__ __align__(16) unsigned char ab_raw[];
-  TbSmem& sm = *reinterpret_cast<TbSmem*>(ab_raw);
-  const int s = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * AB_T;
-  const int nq = lens ? lens[s] : Lp;
-  if (q0 >= nq) return;
-  const int skv = s ^ kv_xor;
-  const int nk = lens ? lens[skv] : Lp;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-  const int mb = (warp & 3) * 16, nb = (warp >> 2) * 32;
-  tb_load(Q + (((size_t)s * LG_HEADS + h) * Lp + q0) * LG_DH, LG_DH, nq - q0, sm.X);
-  const float* Kh = K + ((size_t)skv * LG_HEADS + h) * Lp * LG_DH;
-  // online (max, sum) per thread over ITS columns of rows mb + g and mb + g + 8: partial states merge associatively, so
-  // the four lanes of a row and the two column-half warps are only combined once, after the sweep
-  float mrow[2] = {-INFINITY, -INFINITY}, lrow[2] = {0.f, 0.f};
-  for (int n0 = 0; n0 < nk; n0 += AB_T) {
-    __syncthreads();
-    tb_load(Kh + (size_t)n0 * LG_DH, LG_DH, nk - n0, sm.Y);
-    __syncthreads();
-    float sc[4][4] = {};
-    tb_gemm<true>(sm.X, mb, sm.Y, nb, g, t, sc);
-#pragma unroll
-    for (int r = 0; r < 2; ++r) {
-      float mx = -INFINITY;
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          if (n0 + nb + nt * 8 + 2 * t + c >= nk) sc[nt][2 * r + c] = -INFINITY;
-          mx = fmaxf(mx, sc[nt][2 * r + c]);
-        }
-      const float mnew = fmaxf(mrow[r], mx);
-      const float msafe = mnew == -INFINITY ? 0.f : mnew;
-      float rs = 0.f;
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt) rs += exp2f(sc[nt][2 * r] - msafe) + exp2f(sc[nt][2 * r + 1] - msafe);
-      lrow[r] = lrow[r] * exp2f(mrow[r] - msafe) + rs;
-      mrow[r] = mnew;
-    }
-  }
-#pragma unroll
-  for (int r = 0; r < 2; ++r) {
-#pragma unroll
-    for (int ofs = 1; ofs <= 2; ofs <<= 1) {
-      const float mo = __shfl_xor_sync(0xffffffffu, mrow[r], ofs), lo = __shfl_xor_sync(0xffffffffu, lrow[r], ofs);
-      const float mnew = fmaxf(mrow[r], mo);
-      const float msafe = mnew == -INFINITY ? 0.f : mnew;
-      lrow[r] = lrow[r] * exp2f(mrow[r] - msafe) + lo * exp2f(mo - msafe);
-      mrow[r] = mnew;
-    }
-  }
-  __syncthreads();  // every warp is done with sm.Y: its first rows carry the (max, sum) of the two column halves
-  float* comb = &sm.Y[0][0];  // [column half][row][max, sum]
-  if (t == 0) {
-#pragma unroll
-    for (int r = 0; r < 2; ++r) {
-      comb[(warp >> 2) * 2 * AB_T + 2 * (mb + g + 8 * r)] = mrow[r];
-      comb[(warp >> 2) * 2 * AB_T + 2 * (mb + g + 8 * r) + 1] = lrow[r];
-    }
-  }
-  __syncthreads();
-  const int ty = tid >> 4, tx = tid & 15;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int row = ty * 4 + i, l = q0 + row;
-    const size_t off = ((size_t)s * Lp + l) * LG_D + h * LG_DH + tx * 4;
-    float d = 0.f;
-    if (l < nq) {
-      const float4 o = *reinterpret_cast<const float4*>(O + off);
-      const float4 gr = *reinterpret_cast<const float4*>(dO + off);
-      d = o.x * gr.x + o.y * gr.y + o.z * gr.z + o.w * gr.w;
-    }
-    for (int ofs = 8; ofs; ofs >>= 1) d += __shfl_xor_sync(0xffffffffu, d, ofs);
-    if (tx == 0) {
-      const float m0 = comb[2 * row], l0 = comb[2 * row + 1], m1 = comb[2 * AB_T + 2 * row], l1 = comb[2 * AB_T + 2 * row + 1];
-      const float mnew = fmaxf(m0, m1);
-      const float msafe = mnew == -INFINITY ? 0.f : mnew;
-      const float lsum = l0 * exp2f(m0 - msafe) + l1 * exp2f(m1 - msafe);
-      const size_t r = ((size_t)s * LG_HEADS + h) * Lp + l;
-      lse2[r] = lsum > 0.f ? mnew + log2f(lsum) : INFINITY;  // no keys: every probability is 0
-      dlt[r] = d;
-    }
-  }
-}
-
-// Same contract as attn_bwd_kernel<DKV> above (own / other tiles, out1 / out2).
-template <bool DKV>
-__global__ void __launch_bounds__(256, 2) attn_bwd_tc_kernel(const float* __restrict__ Q, const float* __restrict__ K,
-                                                          const float* __restrict__ V, const float* __restrict__ dO,
-                                                          int Lp, const int32_t* __restrict__ lens, int kv_xor,
-                                                          const float* __restrict__ lse2, const float* __restrict__ dlt,
-                                                          float* __restrict__ out1, float* __restrict__ out2) {
-  extern __shared__ __align__(16) unsigned char ab_raw[];
-  TbSmem& sm = *reinterpret_cast<TbSmem*>(ab_raw);
-  const int s = blockIdx.z, h = blockIdx.y, r0 = blockIdx.x * AB_T;
-  const int so = s ^ kv_xor;
-  const int n_own = lens ? lens[s] : Lp, n_oth = lens ? lens[so] : Lp;
-  if (r0 >= n_own) return;  // (outputs are zero-filled by the caller)
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-  const int mb = (warp & 3) * 16, nb = (warp >> 2) * 32;
-  const size_t own_h = (((size_t)s * LG_HEADS + h) * Lp + r0) * LG_DH;   // head-major offset of the own tile
-  const size_t own_t = ((size_t)s * Lp + r0) * LG_D + h * LG_DH;         // token-major offset of the own tile
-  const size_t oth_h = ((size_t)so * LG_HEADS + h) * Lp * LG_DH;
-  const size_t oth_t = (size_t)so * Lp * LG_D + h * LG_DH;
-  if (!DKV) {
-    tb_load(Q + own_h, LG_DH, n_own - r0, sm.X);
-    tb_load(dO + own_t, LG_D, n_own - r0, sm.U);
-  } else {
-    tb_load(K + own_h, LG_DH, n_own - r0, sm.X);
-    tb_load(V + own_h, LG_DH, n_own - r0, sm.U);
-  }
-  float lse_own[2] = {0.f, 0.f}, dlt_own[2] = {0.f, 0.f};
-#pragma unroll
-  for (int r = 0; r < 2; ++r) {
-    const int m = r0 + mb + g + 8 * r;
-    if (!DKV && m < n_own) {
-      const size_t ri = ((size_t)s * LG_HEADS + h) * Lp + m;
-      lse_own[r] = lse2[ri];
-      dlt_own[r] = dlt[ri];
-    }
-  }
-  float acc1[4][4] = {}, acc2[4][4] = {};
-  for (int n0 = 0; n0 < n_oth; n0 += AB_T) {
-    __syncthreads();  // the previous tile is fully consumed (also orders the own-tile stores on iteration 0)
-    if (!DKV) {
-      tb_load(K + oth_h + (size_t)n0 * LG_DH, LG_DH, n_oth - n0, sm.Y);
-      tb_load(V + oth_h + (size_t)n0 * LG_DH, LG_DH, n_oth - n0, sm.W);
-    } else {
-      tb_load(Q + oth_h + (size_t)n0 * LG_DH, LG_DH, n_oth - n0, sm.Y);
-      tb_load(dO + oth_t + (size_t)n0 * LG_D, LG_D, n_oth - n0, sm.W);
-      if (tid < AB_T) {
-        const bool ok = n0 + tid < n_oth;
-        const size_t ri = ((size_t)so * LG_HEADS + h) * Lp + n0 + tid;
-        sm.lse[tid] = ok ? lse2[ri] : INFINITY;
-        sm.dlt[tid] = ok ? dlt[ri] : 0.f;
-      }
-    }
-    __syncthreads();
-    float sc[4][4] = {}, dp[4][4] = {};
-    tb_gemm<true>(sm.X, mb, sm.Y, nb, g, t, sc);  // <x, y> over d
-    tb_gemm<true>(sm.U, mb, sm.W, nb, g, t, dp);  // <u, w> over d
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-      for (int r = 0; r < 2; ++r) {
-        const int m = mb + g + 8 * r, n = nb + nt * 8 + 2 * t;
-        float pv[2], dv[2];
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          const bool valid = (r0 + m < n_own) && (n0 + n + c < n_oth);
-          const float lq = DKV ? sm.lse[n + c] : lse_own[r];
-          const float dq = DKV ? sm.dlt[n + c] : dlt_own[r];
-          pv[c] = valid ? exp2f(sc[nt][2 * r + c] - lq) : 0.f;
-          dv[c] = valid ? pv[c] * (dp[nt][2 * r + c] - dq) : 0.f;
-        }
-        *reinterpret_cast<float2*>(&sm.D[m][n]) = make_float2(dv[0], dv[1]);
-        if (DKV) *reinterpret_cast<float2*>(&sm.P[m][n]) = make_float2(pv[0], pv[1]);
-      }
-    __syncthreads();
-    tb_gemm<false>(sm.D, mb, sm.Y, nb, g, t, acc1);          // dS . y over the other rows (columns nb.. of d)
-    if (DKV) tb_gemm<false>(sm.P, mb, sm.W, nb, g, t, acc2);  // P . w
-  }
-#pragma unroll
-  for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-    for (int r = 0; r < 2; ++r) {
-      const size_t off = own_h + (size_t)(mb + g + 8 * r) * LG_DH + nb + nt * 8 + 2 * t;
-      *reinterpret_cast<float2*>(out1 + off) = make_float2(acc1[nt][2 * r] * LN2, acc1[nt][2 * r + 1] * LN2);
-      if (DKV) *reinterpret_cast<float2*>(out2 + off) = make_float2(acc2[nt][2 * r], acc2[nt][2 * r + 1]);
-    }
-}
 
 // One thread per (token, 4 consecutive head dimensions), looping over the 4 heads.
 // n_parts == 3 (self block): out [T,768] = [s0 R^T(dq') | s1 R^T(dk') | s2 dv], column part*256 + head*64 + d -- the
@@ -913,28 +454,7 @@ extern "C" int lgb200_attention_bwd(const float* Q, const float* K, const float*
   if ((e = cudaMemsetAsync(dQ, 0, nb, st)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(dK, 0, nb, st)) != cudaSuccess) return (int)e;
   if ((e = cudaMemsetAsync(dV, 0, nb, st)) != cudaSuccess) return (int)e;
-  static const int simt = getenv("LGB200_ATTN_BWD_SIMT") ? atoi(getenv("LGB200_ATTN_BWD_SIMT")) : 0;
-  // default: tcgen05 kernels on split-fp16 planes (lg_x3_attn_bwd.cu).  LGB200_ATTN_BWD_MMASYNC=1 selects the 3xTF32
-  // warp-MMA kernels below, LGB200_ATTN_BWD_SIMT=1 the CUDA-core ones (both kept as cross-checks).
-  static const int mmasync = getenv("LGB200_ATTN_BWD_MMASYNC") ? atoi(getenv("LGB200_ATTN_BWD_MMASYNC")) : 0;
-  if (!simt && !mmasync) return lg_x3_attention_bwd(Q, K, V, ctx, dctx, S, Lp, lens, kv_xor, dQ, dK, dV, workspace, st);
-  const int smem = simt ? (int)sizeof(AbSmem) : (int)sizeof(TbSmem);
-  auto k_stats = simt ? attn_bwd_stats_kernel : attn_bwd_stats_tc_kernel;
-  auto k_dq = simt ? attn_bwd_kernel<false> : attn_bwd_tc_kernel<false>;
-  auto k_dkv = simt ? attn_bwd_kernel<true> : attn_bwd_tc_kernel<true>;
-  if ((e = cudaFuncSetAttribute(k_stats, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return (int)e;
-  if ((e = cudaFuncSetAttribute(k_dq, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return (int)e;
-  if ((e = cudaFuncSetAttribute(k_dkv, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return (int)e;
-  float* lse2 = workspace;
-  float* dlt = workspace + (size_t)S * LG_HEADS * Lp;
-  dim3 grid(Lp / AB_T, LG_HEADS, S);
-  k_stats<<<grid, 256, smem, st>>>(Q, K, ctx, dctx, Lp, lens, kv_xor, lse2, dlt);
-  LG_LAUNCH_CHECK();
-  k_dq<<<grid, 256, smem, st>>>(Q, K, V, dctx, Lp, lens, kv_xor, lse2, dlt, dQ, nullptr);
-  LG_LAUNCH_CHECK();
-  k_dkv<<<grid, 256, smem, st>>>(Q, K, V, dctx, Lp, lens, kv_xor, lse2, dlt, dK, dV);
-  LG_LAUNCH_CHECK();
-  return LGB200_OK;
+  return lg_x3_attention_bwd(Q, K, V, ctx, dctx, S, Lp, lens, kv_xor, dQ, dK, dV, workspace, st);
 }
 
 extern "C" int lgb200_attention_bwd_workspace(int S, int Lp, long long* n_floats) {

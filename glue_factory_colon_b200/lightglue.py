@@ -33,6 +33,14 @@ from ._abi import BF16, EPI_HEADS, EPI_LN_GELU, EPI_ROWMAJOR, F32, F32X3, check,
 LOG2E = 1.4426950408889634
 
 
+def weight_planes(t: torch.Tensor) -> torch.Tensor:
+    """Split-fp16 planes [2][N][K] of a weight matrix, the W operand of the F32X3 kernels: 256 w = hi + lo (LG_X3_EW in
+    csrc/lg_internal.cuh: the power of two keeps the low plane a normal fp16 number; undone in the epilogues)."""
+    t = t.detach().to(torch.float32) * 256.0
+    hi = t.to(torch.float16)
+    return torch.stack([hi, (t - hi.to(torch.float32)).to(torch.float16)]).contiguous()
+
+
 class _Conf(dict):
     """Minimal attribute dict (the reference uses OmegaConf; not a dependency here)."""
 
@@ -419,10 +427,10 @@ class LightGlue(nn.Module):
         The dense [B,M+1,N+1] work -- MatchAssignment of every collected layer, the NLL sums of weight_loss
         (models/utils/losses.py:6-26), row_norm and the arg-maxima of TokenConfidence.loss (:82-95) -- runs in the
         library's kernels; what is left here is arithmetic on [B] and [B,N] vectors.  with_grad: every layer's
-        MatchAssignment goes through train.AssignFn (fp32; backward = lgb200_assign_dsim + cuBLAS GEMMs), the vector
-        arithmetic below is tracked by autograd, and the token-confidence logits are a torch matrix-vector product on
-        the detached descriptors (lightglue.py:83-84), so `losses["total"].mean().backward()` reaches every parameter
-        the reference's does.
+        MatchAssignment goes through train.AssignFn (in conf.train_precision; backward = lgb200_assign_dsim + cuBLAS
+        GEMMs), the vector arithmetic below is tracked by autograd, and the token-confidence logits are a torch
+        matrix-vector product on the detached descriptors (lightglue.py:83-84), so `losses["total"].mean().backward()`
+        reaches every parameter the reference's does.
         With data["num_keypoints0/1"] every entry of `losses` and `metrics` is, per pair, that of the pair un-padded:
         ground truth outside the valid block is ignored (padded rows of gt_matches count as -2), means over an empty
         side are 0 (row_norm, the token-confidence BCE)."""
@@ -435,8 +443,6 @@ class LightGlue(nn.Module):
         B, N, m, _ = r0.shape
         n = r1.shape[2]
         prec = self._precision()
-        if with_grad:  # (train.AssignFn picks the fp32-accurate kernels itself)
-            prec = F32
         st = torch.cuda.current_stream(dev).cuda_stream
         L = conf.n_layers
         gt = data["gt_assignment"].to(dev).to(torch.bool).contiguous()
@@ -573,12 +579,7 @@ class LightGlue(nn.Module):
 
         def W(t):
             t = t.detach().to(device=device, dtype=torch.float32)
-            if prec == F32X3:  # split planes [2][N][K] fp16: 256 w = hi + lo (LG_X3_EW in csrc/lg_internal.cuh:
-                t = t * 256.0   # the power of two keeps the low plane a normal fp16 number; undone in the epilogues)
-                hi = t.to(torch.float16)
-                lo = (t - hi.to(torch.float32)).to(torch.float16)
-                return torch.stack([hi, lo]).contiguous()
-            return t.to(wdt).contiguous()
+            return weight_planes(t) if prec == F32X3 else t.to(wdt).contiguous()
 
         def Fp(t):
             return t.detach().to(device=device, dtype=torch.float32).contiguous()
@@ -652,15 +653,15 @@ class LightGlue(nn.Module):
 
     def _forward_train(self, data: dict) -> dict:
         """Training step (module in training mode, autograd on): the transformer stack runs through
-        train.TransformerFn -- fp32 kernels forward, hand-written backward kernels + cuBLAS GEMMs backward -- so that
-        `ref_descriptors0/1` carry an autograd graph to the descriptors and to every parameter
+        train.TransformerFn -- the library's kernels forward, hand-written backward kernels + cuBLAS GEMMs backward, in
+        conf.train_precision ("fp32": the fp32-accurate tensor-core mode; "bf16": the bf16 inference kernels and bf16
+        products) -- so that `ref_descriptors0/1` carry an autograd graph to the descriptors and to every parameter
         (lightglue.py:484-498, :546-547).  conf.checkpointed (:485-494) selects recomputation of the attention
         operands in the backward pass instead of keeping them.  The last layer's MatchAssignment and filter_matches run
         through train.LogAssignFn, so that `log_assignment` and `matching_scores0/1` carry a graph too (as in the
         reference: a loss may read them; LightGlue.loss reads log_assignment detached, :606, :625-630).  The staged
         keypoints (with scales / orientations when add_scale_ori) are inputs of the transformer Function: keypoints0/1,
         scales0/1 and oris0/1 that require grad receive their gradient through the positional encoding.
-        conf.train_precision = "bf16" runs train.TransformerBf16Fn and the bf16 assignment kernels instead.
         data["num_keypoints0/1"] (padded batches): every kernel reads the per-pair counts, the padding's descriptors and
         keypoints are replaced by zeros, and the outputs take the layout of the no-grad forward with the same counts."""
         from . import train as _train
@@ -702,10 +703,7 @@ class LightGlue(nn.Module):
         assert desc0.shape[-1] == conf.input_dim and desc1.shape[-1] == conf.input_dim
         params = [p for _, p in _train.transformer_params(self)]
         L = conf.n_layers
-        if self._train_bf16():  # mixed precision: the bf16 inference kernels forward (conf.train_precision)
-            r0, r1 = _train.TransformerBf16Fn.apply(self, geom, desc0, desc1, k0, k1, *params)
-        else:
-            r0, r1 = _train.TransformerFn.apply(self, geom, desc0, desc1, k0, k1, *params)
+        r0, r1 = _train.TransformerFn.apply(self, geom, desc0, desc1, k0, k1, *params)
         a = self.log_assignment[L - 1]
         scores, m0, m1, ms0, ms1 = _train.LogAssignFn.apply(
             self, L - 1, counts, r0[:, -1], r1[:, -1], a.final_proj.weight, a.final_proj.bias, a.matchability.weight,

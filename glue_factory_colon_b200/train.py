@@ -2,38 +2,38 @@
 
 The reference trains through `LightGlue.forward` / `LightGlue.loss` with autograd (lightglue.py:484-498 collects every
 layer's descriptors in training mode, :588-637 turns them into the deep-supervision NLL; train.py calls
-`loss.backward()`).  Here the same contract is met by two `torch.autograd.Function`s whose backward is written by hand:
+`loss.backward()`).  Here the same contract is met by `torch.autograd.Function`s whose backward is written by hand:
 
   * `TransformerFn`  descriptors (+ every transformer / posenc / input_proj parameter) -> ref_descriptors0/1
-    [B, n_layers, N, 256].  Forward = the library's fp32-accurate tensor-core kernels (linear layers and attention in the
-    split-fp16 / three-MMA mode of lg_x3.cu / lg_x3_attn.cu; LGB200_TRAIN_SIMT_LINEAR=1 selects the CUDA-core fp32 linear
-    kernels), keeping the two block inputs of every layer plus -- unless conf.checkpointed
-    (lightglue.py:485-494) -- q / k / v / context / message; with conf.checkpointed those are recomputed in the
+    [B, n_layers, N, 256].  It keeps the two block inputs of every layer plus -- unless conf.checkpointed
+    (lightglue.py:485-494) -- q / k / v / context (/ message); with conf.checkpointed those are recomputed in the
     backward pass with the same kernels.  The pre-LayerNorm activations are always recomputed (one GEMM).  Backward =
-    the hand-written kernels of csrc/lg_bwd.cu:
-    flash-attention backward (lgb200_attention_bwd), rotary / head-split backward incl. the gradient of the rotary
-    angles (lgb200_heads_bwd), GELU . LayerNorm backward (lgb200_ln_gelu_bwd).
+    the hand-written kernels of csrc/lg_bwd.cu: flash-attention backward (lgb200_attention_bwd /
+    lgb200_attention_bwd_bf16), rotary / head-split backward incl. the gradient of the rotary angles
+    (lgb200_heads_bwd), GELU . LayerNorm backward (lgb200_ln_gelu_bwd).  The layer loop, the keep / recompute policy
+    and the posenc / input_proj tail are shared; the kernels and GEMMs of each block come from `_F32Blocks` or
+    `_Bf16Blocks` (conf.train_precision).
   * `AssignFn`       MatchAssignment of one layer (lightglue.py:272-288) reduced to what NLLLoss reads
     (losses.py:6-26: the sum of log_assignment over the ground-truth matches and the two dustbin vectors).  Forward =
     the library's assignment + reduction kernels; backward = lgb200_assign_dsim (d similarity of the double softmax).
   * `LogAssignFn`    the training forward's log_assignment / matches / matching_scores of the last layer (lightglue.py:
     272-288, 294-319) with a graph for losses that read them; backward = lgb200_assign_bwd (any upstream gradient).
-The staged keypoints are inputs of the transformer Functions: with keypoints (scales, orientations) that require grad,
+The staged keypoints are inputs of TransformerFn: with keypoints (scales, orientations) that require grad,
 lgb200_posenc_bwd turns the rotary-angle gradient into their gradient (lightglue.py:28-40, 61-66).
 
-Plain GEMMs of the backward pass (dX = dY.W, dW = dY^T.X) go to cuBLAS -- they are library GEMMs with nothing to fuse --
-as three fp16 tensor-core GEMMs on split planes with fp32 accumulation (_Kern.mm3; LGB200_TRAIN_SGEMM=1: one fp32
-sgemm on the CUDA cores).  Gradients span a range (1e-8 ... 1e-2) that a fixed plane scaling does not cover, so
-lgb200_split_dynamic scales every gradient tensor by its own power of two first.  That is the default,
-conf.train_precision = "fp32": fp32-accurate whatever conf.precision says.
+conf.train_precision = "fp32" (the default): fp32-accurate whatever conf.precision says.  Forward = the library's
+tensor-core kernels in the split-fp16 / three-MMA mode (lg_x3.cu / lg_x3_attn.cu).  Plain GEMMs of the backward pass
+(dX = dY.W, dW = dY^T.X) go to cuBLAS -- they are library GEMMs with nothing to fuse -- as three fp16 tensor-core GEMMs
+on split planes with fp32 accumulation (_Kern.mm3).  Gradients span a range (1e-8 ... 1e-2) that a fixed plane scaling
+does not cover, so lgb200_split_dynamic scales every gradient tensor by its own power of two first.
 
-conf.train_precision = "bf16" (mixed precision, the counterpart of the reference under torch.autocast(bfloat16)):
-`TransformerBf16Fn` runs the bf16 inference kernels forward exactly as the no-grad forward with precision="bf16" does
-(bf16 weight pack with out_proj / to_out folded into the first FFN matrix, bf16 residual stream, rot16), so the training
-forward's outputs are bit-equal to it; the backward recomputes the pre-LayerNorm activations in fp32 from the bf16
-operands, runs lgb200_ln_gelu_bwd, the bf16 attention backward (lgb200_attention_bwd_bf16: one bf16 tcgen05 MMA per
-product) and lgb200_heads_bwd, and does every plain GEMM as ONE bf16 cuBLAS product with fp32 output.  Gradients of the
-folded weights follow by the chain rule (see _ffn_bwd16).  `AssignFn` uses the bf16 assignment kernels.
+conf.train_precision = "bf16" (mixed precision, the counterpart of the reference under torch.autocast(bfloat16)): the
+forward runs the bf16 inference kernels exactly as the no-grad forward with precision="bf16" does (bf16 weight pack with
+out_proj / to_out folded into the first FFN matrix, bf16 residual stream, rot16), so the training forward's outputs are
+bit-equal to it; the backward recomputes the pre-LayerNorm activations in fp32 from the bf16 operands, runs the bf16
+attention backward (one bf16 tcgen05 MMA per product) and does every plain GEMM as ONE bf16 cuBLAS product with fp32
+output.  Gradients of the folded weights follow by the chain rule (see _Bf16Blocks.ffn_bwd).  `AssignFn` uses the bf16
+assignment kernels.
 
 Padded batches (data["num_keypoints0/1"], the counts padding.py produces): every kernel of the stack reads the
 per-pair counts from the device `lens`, the staged descriptor and keypoint rows past the counts are zeroed (so the
@@ -46,7 +46,6 @@ from __future__ import annotations
 
 import ctypes as C
 import math
-import os
 from typing import Dict, List, Tuple
 
 import numpy as np
@@ -55,26 +54,13 @@ from torch import nn
 
 from . import _abi
 from ._abi import BF16, EPI_HEADS, EPI_LN_GELU, EPI_ROWMAJOR, F32, F32X3, check, ptr
+from .lightglue import weight_planes
 
 LOG2E = 1.4426950408889634
 Q_SCALE = LOG2E / math.sqrt(64.0)   # folded into q: the attention kernels work in the log2 domain
 C_SCALE = math.sqrt(Q_SCALE)        # cross block: to_qk feeds both sides (lightglue.py:208)
 AI, WI = 1.0 / 64.0, 1.0 / 256.0       # inverse plane scalings of activations / weights (LG_X3_EA, LG_X3_EW)
 N_PARTIALS = 296                    # CTAs of lgb200_ln_gelu_bwd (2 per SM)
-_SIMT_ATTN = os.environ.get("LGB200_TRAIN_SIMT_ATTN", "0") == "1"
-_SIMT_LINEAR = os.environ.get("LGB200_TRAIN_SIMT_LINEAR", "0") == "1"
-# plain GEMMs of the backward pass: 1 = cuBLAS fp32 (sgemm on the CUDA cores), default = three fp16 tensor-core GEMMs on
-# split planes with fp32 accumulation (the same hi.hi + hi.lo + lo.hi scheme as the forward's lg_x3.cu kernels)
-def _has_mm_out_dtype() -> bool:
-    """torch.mm / addmm / bmm with out_dtype (fp16 operands, fp32 accumulation AND fp32 output) exist from PyTorch 2.8 on."""
-    try:
-        a = torch.empty(1, 1, device="meta", dtype=torch.float16)
-        return torch.mm(a, a, out_dtype=torch.float32).dtype == torch.float32
-    except (TypeError, RuntimeError, NotImplementedError):
-        return False
-
-
-_SGEMM = os.environ.get("LGB200_TRAIN_SGEMM", "0") == "1" or _SIMT_LINEAR or not _has_mm_out_dtype()
 _X3_WEIGHTS = ("qkv_w", "so_w", "sf0_w", "sf3_w", "cqv_w", "co_w", "cf0_w", "cf3_w")
 # packed Wqkv row r holds reference row _PERM[r] (lightglue.py:158: head*192 + d*3 + part -> part*256 + head*64 + d)
 _PERM = torch.arange(768).view(4, 64, 3).permute(2, 0, 1).reshape(-1)
@@ -175,20 +161,10 @@ class _Kern:
         torch.addmm(r, A[0], B[0], out_dtype=f32, out=r)
         return r.mul_(scale)
 
-    def attention(self, q, k, v, kv_xor, ctx):
+    def attention(self, qp, kp, vp, kv_xor, ctx):
         """Forward attention on the tensor cores in the fp32-accurate mode (lg_x3_attn.cu: split-fp16 operands, three
-        tcgen05 MMAs per product, fp32 softmax) -- 12x faster than the CUDA-core fp32 kernel at 2048 keypoints, same
-        1e-6-level agreement with float64.  LGB200_TRAIN_SIMT_ATTN=1 selects the CUDA-core kernel."""
-        if _SIMT_ATTN:
-            check(self.lib.lgb200_attention(F32, ptr(q), ptr(k), ptr(v), self.S, self.Lp, ptr(self.lens), kv_xor, ptr(ctx),
-                                            self.st), "lgb200_attention")
-            return
-        if q.dtype == torch.float16:  # already split planes (x3 projections)
-            qp, kp, vp = q, k, v
-        else:
-            qp = self.split(q)
-            kp = qp if k is q else self.split(k)
-            vp = self.split(v)
+        tcgen05 MMAs per product, fp32 softmax) on the planes of the x3 projections -> the context's planes; ctx
+        [T,256] receives it in fp32."""
         cp = torch.zeros(2, self.T, 256, device=self.dev, dtype=torch.float16)
         check(self.lib.lgb200_attention(F32X3, ptr(qp), ptr(kp), ptr(vp), self.S, self.Lp, ptr(self.lens), kv_xor, ptr(cp),
                                         self.st), "lgb200_attention")
@@ -196,12 +172,15 @@ class _Kern:
         return cp
 
     def attention_bwd(self, q, k, v, ctx, dctx, kv_xor):
+        """Flash-attention backward, fp32 dctx -> fp32 dq, dk, dv: lgb200_attention_bwd on fp32 q / k / v / ctx, or
+        lgb200_attention_bwd_bf16 on the bf16 ones the bf16 forward kept."""
+        name = "lgb200_attention_bwd_bf16" if q.dtype == torch.bfloat16 else "lgb200_attention_bwd"
         dq, dk, dv = self.empty(self.T * 256), self.empty(self.T * 256), self.empty(self.T * 256)
         n_ws = C.c_longlong(0)
-        check(self.lib.lgb200_attention_bwd_workspace(self.S, self.Lp, C.byref(n_ws)), "lgb200_attention_bwd_workspace")
+        check(getattr(self.lib, name + "_workspace")(self.S, self.Lp, C.byref(n_ws)), name + "_workspace")
         ws = self.empty(n_ws.value)
-        check(self.lib.lgb200_attention_bwd(ptr(q), ptr(k), ptr(v), ptr(ctx), ptr(dctx), self.S, self.Lp, ptr(self.lens),
-                                            kv_xor, ptr(dq), ptr(dk), ptr(dv), ptr(ws), self.st), "lgb200_attention_bwd")
+        check(getattr(self.lib, name)(ptr(q), ptr(k), ptr(v), ptr(ctx), ptr(dctx), self.S, self.Lp, ptr(self.lens),
+                                      kv_xor, ptr(dq), ptr(dk), ptr(dv), ptr(ws), self.st), name)
         return dq, dk, dv
 
     # ---- bf16 mixed-precision training (conf.train_precision = "bf16") ----
@@ -223,18 +202,6 @@ class _Kern:
                                         self.st), "lgb200_attention (bf16)")
         return ctx
 
-    def attention_bwd16(self, q, k, v, ctx, dctx, kv_xor):
-        """lgb200_attention_bwd_bf16: bf16 q / k / v / ctx of the forward, fp32 dctx -> fp32 dq, dk, dv."""
-        dq, dk, dv = self.empty(self.T * 256), self.empty(self.T * 256), self.empty(self.T * 256)
-        n_ws = C.c_longlong(0)
-        check(self.lib.lgb200_attention_bwd_bf16_workspace(self.S, self.Lp, C.byref(n_ws)),
-              "lgb200_attention_bwd_bf16_workspace")
-        ws = self.empty(n_ws.value)
-        check(self.lib.lgb200_attention_bwd_bf16(ptr(q), ptr(k), ptr(v), ptr(ctx), ptr(dctx), self.S, self.Lp,
-                                                 ptr(self.lens), kv_xor, ptr(dq), ptr(dk), ptr(dv), ptr(ws), self.st),
-              "lgb200_attention_bwd_bf16")
-        return dq, dk, dv
-
     def heads_bwd(self, dq, dk, dv, q, k, rot, n_parts, scales, dtheta):
         out = self.empty(self.T, 256 * n_parts)
         check(self.lib.lgb200_heads_bwd(ptr(dq), ptr(dk), ptr(dv), ptr(q), ptr(k), ptr(rot), self.S, self.Lp,
@@ -248,17 +215,16 @@ class _Kern:
                                           ptr(act), ptr(part), N_PARTIALS, self.st), "lgb200_ln_gelu_bwd")
         return dh, act, part.sum(0)
 
-    def pack(self, src, img, dst):
-        """src [B, cnt, dim] -> rows of sequences 2b + img of dst [T, dim] (rows past cnt zero-filled)."""
-        src = src.to(torch.float32).contiguous()
-        check(self.lib.lgb200_pack_rows(ptr(src), self.B, src.shape[1], src.shape[2], img, self.Lp, ptr(dst), None,
-                                        self.st), "lgb200_pack_rows")
-
-    def pack2(self, a0, a1):
-        """[B, m, dim] / [B, n, dim] -> [T, dim], rows past the padded sizes and the per-pair counts zero."""
-        dst = self.zeros(self.T, a0.shape[-1])
-        self.pack(a0, 0, dst)
-        self.pack(a1, 1, dst)
+    def pack2(self, a0, a1, dtype=torch.float32):
+        """[B, m, dim] / [B, n, dim] -> [T, dim] fp32 or bf16 (image img of pair b in the rows of sequence 2b + img),
+        rows past the padded sizes and the per-pair counts zero."""
+        dst = torch.zeros(self.T, a0.shape[-1], device=self.dev, dtype=dtype)
+        f32 = dtype == torch.float32
+        for img, src in ((0, a0), (1, a1)):
+            src = src.to(torch.float32).contiguous()
+            check(self.lib.lgb200_pack_rows(ptr(src), self.B, src.shape[1], src.shape[2], img, self.Lp,
+                                            ptr(dst) if f32 else None, None if f32 else ptr(dst), self.st),
+                  "lgb200_pack_rows")
         return self.mask_rows(dst)
 
     def unpack(self, x):
@@ -351,101 +317,86 @@ def transformer_params(model) -> List[Tuple[object, nn.Parameter]]:
     return out
 
 
-# ---- one transformer layer, forward pieces (lightglue.py:151-164, 193-222) ---------------------------------------
+# ---- the transformer stack (lightglue.py:151-164, 193-222, 456-498) ------------------------------------------------
+# _F32Blocks / _Bf16Blocks hold what depends on conf.train_precision -- the weight pack, the staging, the positional
+# encoding and the kernels and GEMMs of one block forward and backward -- behind the same methods; TransformerFn owns
+# the layer loop, the keep / recompute policy of conf.checkpointed and the posenc / input_proj tail.  A block's saved
+# tuple starts with the attention operands (q, k, v, ctx) of the self block, (qk, v, ctx) of the cross block.
 
 
-def x3_weights(w: Dict) -> Dict:
-    """Split-fp16 planes [2][N][K] of a layer's weight matrices (256 w = hi + lo, the operand format of lg_x3.cu)."""
-    out = {}
-    for name in _X3_WEIGHTS:
-        t = w[name].detach().float() * 256.0
-        hi = t.to(torch.float16)
-        out[name] = torch.stack([hi, (t - hi.float()).to(torch.float16)]).contiguous()
-    return out
+class _F32Blocks:
+    """conf.train_precision = "fp32": the fp32-accurate tensor-core kernels on split-fp16 planes forward (lg_x3.cu /
+    lg_x3_attn.cu), three fp16 tensor-core GEMMs on split planes for every plain GEMM of the backward (_Kern.mm3);
+    fp32 residual stream.  Saved tuples end with the message: (q, k, v, ctx, msg) / (qk, v, ctx, msg), q / k / v fp32
+    or None (not kept)."""
 
+    def __init__(self, k: _Kern, model):
+        self.k, self.model = k, model
+        self.W = model._pack(F32, k.dev)
+        for w in self.W["layers"]:  # split-fp16 planes of the weight matrices, cached with the pack (rebuilt with it)
+            if "x3" not in w:
+                w["x3"] = {name: weight_planes(w[name]) for name in _X3_WEIGHTS}
 
-def _self_attend(k: _Kern, w: Dict, x, rot, fp32_heads: bool = True):
-    """-> (q, k, v, ctx, msg); with the tensor-core linears q / k / v are None unless `fp32_heads` (the backward kernels
-    read them in fp32)."""
-    T = k.T
-    if _SIMT_LINEAR:
-        q, kk, v = k.zeros(T * 256), k.zeros(T * 256), k.zeros(T * 256)
-        k.linear(EPI_HEADS, x, w["qkv_w"], w["qkv_b"], 768, 256, scale=(Q_SCALE, 1.0, 1.0), rot=rot, n_rot=2,
-                 outp=(q, kk, v))
+    def stage(self, desc0, desc1):
+        """-> (x [T,256]: the first block input, the staged input of input_proj or None)"""
+        k = self.k
+        x = k.pack2(desc0, desc1)
+        if not isinstance(self.model.input_proj, nn.Linear):
+            return x, None
+        out = k.zeros(k.T, 256)
+        k.linear(EPI_ROWMAJOR, x, self.W["in_w"], self.W["in_b"], 256, x.shape[1], out=out)
+        return out, x
+
+    def posenc(self, geom):
+        """self.rot: rotary angles [T,64] fp32 from the staged keypoints."""
+        self.rot = self.k.zeros(self.k.T, 64)
+        self.k.posenc(geom, self.W["wr"], self.rot)
+
+    def self_attend(self, w, x, heads: bool = True):
+        """-> (q, k, v, ctx, msg); q / k / v None unless `heads` (the backward kernels read them in fp32)."""
+        k, T, wx = self.k, self.k.T, w["x3"]
+        qp, kp, vp = k.planes(T * 256), k.planes(T * 256), k.planes(T * 256)
+        k.linear3(EPI_HEADS, k.split(x), wx["qkv_w"], w["qkv_b"], 768, 256, scale=(Q_SCALE, 1.0, 1.0), rot=self.rot,
+                  n_rot=2, outp=(qp, kp, vp))
         ctx = k.zeros(T, 256)
-        k.attention(q, kk, v, 0, ctx)
+        cp = k.attention(qp, kp, vp, 0, ctx)
         msg = k.zeros(T, 256)
-        k.linear(EPI_ROWMAJOR, ctx, w["so_w"], w["so_b"], 256, 256, out=msg)
-        return q, kk, v, ctx, msg
-    wx = w["x3"]
-    qp, kp, vp = k.planes(T * 256), k.planes(T * 256), k.planes(T * 256)
-    k.linear3(EPI_HEADS, k.split(x), wx["qkv_w"], w["qkv_b"], 768, 256, scale=(Q_SCALE, 1.0, 1.0), rot=rot, n_rot=2,
-              outp=(qp, kp, vp))
-    ctx = k.zeros(T, 256)
-    cp = k.attention(qp, kp, vp, 0, ctx)
-    msg = k.zeros(T, 256)
-    k.linear3(EPI_ROWMAJOR, cp, wx["so_w"], w["so_b"], 256, 256, out32=msg)
-    if not fp32_heads:
-        return None, None, None, ctx, msg
-    return k.unsplit(qp, T * 256), k.unsplit(kp, T * 256), k.unsplit(vp, T * 256), ctx, msg
+        k.linear3(EPI_ROWMAJOR, cp, wx["so_w"], w["so_b"], 256, 256, out32=msg)
+        if not heads:
+            return None, None, None, ctx, msg
+        return k.unsplit(qp, T * 256), k.unsplit(kp, T * 256), k.unsplit(vp, T * 256), ctx, msg
 
-
-def _cross_attend(k: _Kern, w: Dict, x, fp32_heads: bool = True):
-    T = k.T
-    if _SIMT_LINEAR:
-        qk, v = k.zeros(T * 256), k.zeros(T * 256)
-        k.linear(EPI_HEADS, x, w["cqv_w"], w["cqv_b"], 512, 256, scale=(C_SCALE, 1.0, 1.0), n_rot=0, outp=(qk, v, None))
+    def cross_attend(self, w, x, heads: bool = True):
+        k, T, wx = self.k, self.k.T, w["x3"]
+        qp, vp = k.planes(T * 256), k.planes(T * 256)
+        k.linear3(EPI_HEADS, k.split(x), wx["cqv_w"], w["cqv_b"], 512, 256, scale=(C_SCALE, 1.0, 1.0), n_rot=0,
+                  outp=(qp, vp, None))
         ctx = k.zeros(T, 256)
-        k.attention(qk, qk, v, 1, ctx)
+        cp = k.attention(qp, qp, vp, 1, ctx)
         msg = k.zeros(T, 256)
-        k.linear(EPI_ROWMAJOR, ctx, w["co_w"], w["co_b"], 256, 256, out=msg)
-        return qk, v, ctx, msg
-    wx = w["x3"]
-    qp, vp = k.planes(T * 256), k.planes(T * 256)
-    k.linear3(EPI_HEADS, k.split(x), wx["cqv_w"], w["cqv_b"], 512, 256, scale=(C_SCALE, 1.0, 1.0), n_rot=0,
-              outp=(qp, vp, None))
-    ctx = k.zeros(T, 256)
-    cp = k.attention(qp, qp, vp, 1, ctx)
-    msg = k.zeros(T, 256)
-    k.linear3(EPI_ROWMAJOR, cp, wx["co_w"], w["co_b"], 256, 256, out32=msg)
-    if not fp32_heads:
-        return None, None, ctx, msg
-    return k.unsplit(qp, T * 256), k.unsplit(vp, T * 256), ctx, msg
+        k.linear3(EPI_ROWMAJOR, cp, wx["co_w"], w["co_b"], 256, 256, out32=msg)
+        if not heads:
+            return None, None, ctx, msg
+        return k.unsplit(qp, T * 256), k.unsplit(vp, T * 256), ctx, msg
 
-
-def _ffn(k: _Kern, w: Dict, pre: str, x, msg):
-    """x + ffn(cat[x, msg]) (lightglue.py:164, 220-221)."""
-    out = k.zeros(k.T, 256)
-    if _SIMT_LINEAR:
-        hid = k.zeros(k.T, 512)
-        k.linear(EPI_LN_GELU, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=msg, K0=256, gamma=w[pre + "ln_g"],
-                 beta=w[pre + "ln_b"], out=hid)
-        k.linear(EPI_ROWMAJOR, hid, w[pre + "f3_w"], w[pre + "f3_b"], 256, 512, resid=x, out=out)
+    def ffn(self, w, pre: str, x, s):
+        """x + ffn(cat[x, msg]) (lightglue.py:164, 220-221), msg = s[-1]."""
+        k, wx = self.k, w["x3"]
+        out = k.zeros(k.T, 256)
+        hp = k.planes(k.T, 512)
+        k.linear3(EPI_LN_GELU, k.split(x), wx[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=k.split(s[-1]), K0=256,
+                  gamma=w[pre + "ln_g"], beta=w[pre + "ln_b"], out=hp)
+        k.linear3(EPI_ROWMAJOR, hp, wx[pre + "f3_w"], w[pre + "f3_b"], 256, 512, resid=x, out32=out)
         return out
-    wx = w["x3"]
-    hp = k.planes(k.T, 512)
-    k.linear3(EPI_LN_GELU, k.split(x), wx[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=k.split(msg), K0=256,
-              gamma=w[pre + "ln_g"], beta=w[pre + "ln_b"], out=hp)
-    k.linear3(EPI_ROWMAJOR, hp, wx[pre + "f3_w"], w[pre + "f3_b"], 256, 512, resid=x, out32=out)
-    return out
 
-
-def _ffn_bwd(k: _Kern, w: Dict, pre: str, x, msg, dy):
-    """Backward of y = ffn(cat[x, msg]) given dy [T,256]: (d x, d msg, parameter gradients)."""
-    h = k.zeros(k.T, 512)  # pre-LayerNorm activations, recomputed
-    if _SIMT_LINEAR:
-        k.linear(EPI_ROWMAJOR, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=msg, K0=256, out=h)
-    else:
-        k.linear3(EPI_ROWMAJOR, k.split(x), w["x3"][pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=k.split(msg), K0=256,
+    def ffn_bwd(self, i: int, w, pre: str, x, s, dy):
+        """Backward of y = ffn(cat[x, out_proj(ctx)]) given dy [T,256] and the block's saved tuple s: (d x through the
+        ffn, d ctx, parameter gradients incl. those of out_proj / to_out)."""
+        k, wx = self.k, w["x3"]
+        c, msg = s[-2:]
+        h = k.zeros(k.T, 512)  # pre-LayerNorm activations, recomputed
+        k.linear3(EPI_ROWMAJOR, k.split(x), wx[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=k.split(msg), K0=256,
                   out32=h)
-    if _SGEMM:
-        da = dy @ w[pre + "f3_w"]
-        dh, act, gsum = k.ln_gelu_bwd(h, w[pre + "ln_g"], w[pre + "ln_b"], da)
-        g3, g0 = dy.t() @ act, torch.cat([dh.t() @ x, dh.t() @ msg], 1)
-        dcat = dh @ w[pre + "f0_w"]
-        b3, b0 = dy.sum(0), dh.sum(0)
-    else:
-        wx = w["x3"]
         dyp, dyi, b3 = k.gsplit(dy, colsum=True)
         da = k.mm3(dyp, wx[pre + "f3_w"], dyi * WI)
         dh, act, gsum = k.ln_gelu_bwd(h, w[pre + "ln_g"], w[pre + "ln_b"], da)
@@ -454,123 +405,26 @@ def _ffn_bwd(k: _Kern, w: Dict, pre: str, x, msg, dy):
         dht = dhp.transpose(1, 2)
         g0 = torch.cat([k.mm3(dht, k.asplit(x), dhi * AI), k.mm3(dht, k.asplit(msg), dhi * AI)], 1)
         dcat = k.mm3(dhp, wx[pre + "f0_w"], dhi * WI)
-    g = {
-        pre + "f3_w": g3, pre + "f3_b": b3,
-        pre + "ln_g": gsum[:512], pre + "ln_b": gsum[512:],
-        pre + "f0_w": g0, pre + "f0_b": b0,
-    }
-    return dcat[:, :256], dcat[:, 256:].contiguous(), g
+        del h, dyp, dyi, da, dh, act, dhp, dhi, dht  # not held across the out_proj backward: keeps the peak memory down
+        po = "so" if pre == "s" else "co"
+        gw, gb, dc = self.proj_bwd(w, po + "_w", dcat[:, 256:].contiguous(), c)
+        g = {
+            pre + "f3_w": g3, pre + "f3_b": b3,
+            pre + "ln_g": gsum[:512], pre + "ln_b": gsum[512:],
+            pre + "f0_w": g0, pre + "f0_b": b0,
+            po + "_w": gw, po + "_b": gb,
+        }
+        return dcat[:, :256], dc, g
 
+    def proj_bwd(self, w, name: str, dy, x):
+        """Backward of y = x W^T + b for the weight `name` ([N, K], planes in w["x3"]): (dy^T x, dy^T 1, dy W)."""
+        k = self.k
+        dyp, dyi, db = k.gsplit(dy, colsum=True)
+        return k.mm3(dyp.transpose(1, 2), k.asplit(x), dyi * AI), db, k.mm3(dyp, w["x3"][name], dyi * WI)
 
-def _proj_bwd(k: _Kern, w: Dict, name: str, dy, x):
-    """Backward of y = x W^T + b for the weight `name` ([N, K], planes in w["x3"]): (dy^T x, dy^T 1, dy W)."""
-    if _SGEMM:
-        return dy.t() @ x, dy.sum(0), dy @ w[name]
-    dyp, dyi, db = k.gsplit(dy, colsum=True)
-    return k.mm3(dyp.transpose(1, 2), k.asplit(x), dyi * AI), db, k.mm3(dyp, w["x3"][name], dyi * WI)
-
-
-class TransformerFn(torch.autograd.Function):
-    """ref_descriptors0/1 = all layers' outputs of the transformer stack (lightglue.py:456-498)."""
-
-    @staticmethod
-    def forward(ctx, model, geom: Dict, desc0, desc1, k0, k1, *params):
-        """k0 / k1 [B, m / n, kdim]: the staged keypoint rows (coordinates, plus scale and orientation with
-        add_scale_ori) -- inputs, so that their gradient reaches whatever the caller built them from."""
-        dev = desc0.device
-        B, m, _ = desc0.shape
-        n = desc1.shape[1]
-        geom = dict(geom, k0=k0, k1=k1)
-        k = _Kern(dev, B, m, n, geom.get("counts"))
-        W = model._pack(F32, dev)
-        L = model.conf.n_layers
-        if not _SIMT_LINEAR:  # split-fp16 planes of the weight matrices, cached with the pack (rebuilt when a weight changes)
-            for w in W["layers"]:
-                if "x3" not in w:
-                    w["x3"] = x3_weights(w)
-        xin = None
-        if isinstance(model.input_proj, nn.Linear):
-            din = model.conf.input_dim
-            xin = k.pack2(desc0, desc1)
-            x = k.zeros(k.T, 256)
-            k.linear(EPI_ROWMAJOR, xin, W["in_w"], W["in_b"], 256, din, out=x)
-        else:
-            x = k.pack2(desc0, desc1)
-        rot = k.zeros(k.T, 64)
-        k.posenc(geom, W["wr"], rot)
-        # conf.checkpointed (lightglue.py:485-494): keep only the block inputs and recompute q / k / v / context /
-        # message in the backward pass (26 x T KB per layer less); otherwise they are kept, as autograd would
-        keep = not bool(model.conf.checkpointed)
-        xs_in, xs_mid, outs, kept = [], [], [], []
-        for i in range(L):
-            w = W["layers"][i]
-            xs_in.append(x)
-            sa = _self_attend(k, w, x, rot, fp32_heads=keep)
-            x = _ffn(k, w, "s", x, sa[-1])
-            xs_mid.append(x)
-            ca = _cross_attend(k, w, x, fp32_heads=keep)
-            x = _ffn(k, w, "c", x, ca[-1])
-            outs.append(x)
-            kept.append((sa, ca) if keep else None)
-        ctx.k, ctx.W, ctx.geom, ctx.model = k, W, geom, model
-        ctx.xs_in, ctx.xs_mid, ctx.rot, ctx.xin, ctx.kept = xs_in, xs_mid, rot, xin, kept
-        ctx.keys = [key for key, _ in transformer_params(model)]
-        r0 = torch.stack([k.unpack(o)[0] for o in outs], 1)
-        r1 = torch.stack([k.unpack(o)[1] for o in outs], 1)
-        return r0, r1
-
-    @staticmethod
-    def backward(ctx, g0, g1):
-        k, W, geom = ctx.k, ctx.W, ctx.geom
-        L = len(ctx.xs_in)
-        rot = ctx.rot
-        dx = k.zeros(k.T, 256)
-        dtheta = k.zeros(k.T, 32)
-        grads: Dict[object, torch.Tensor] = {}
-        for i in reversed(range(L)):
-            w = W["layers"][i]
-            dx = dx + k.pack2(g0[:, i], g1[:, i])
-            x_in, x_mid = ctx.xs_in[i], ctx.xs_mid[i]
-            # ---- cross block (lightglue.py:193-222) ----
-            qk, v, c, msg = ctx.kept[i][1] if ctx.kept[i] is not None else _cross_attend(k, w, x_mid)
-            dxa, dmsg, g = _ffn_bwd(k, w, "c", x_mid, msg, dx)
-            for name, val in g.items():
-                grads[(i, name)] = val
-            grads[(i, "co_w")], grads[(i, "co_b")], dc = _proj_bwd(k, w, "co_w", dmsg, c)
-            dq, dk, dv = k.attention_bwd(qk, qk, v, c, dc, 1)
-            dqv = k.heads_bwd(dq, dk, dv, None, None, None, 2, (C_SCALE, 1.0, 1.0), None)
-            gw, gb, dxp = _proj_bwd(k, w, "cqv_w", dqv, x_mid)
-            grads[(i, "cqk_w")], grads[(i, "cv_w")] = gw[:256], gw[256:]
-            grads[(i, "cqk_b")], grads[(i, "cv_b")] = gb[:256], gb[256:]
-            dxm = dx + dxa + dxp
-            # ---- self block (lightglue.py:151-164) ----
-            q, kk, v, c, msg = ctx.kept[i][0] if ctx.kept[i] is not None else _self_attend(k, w, x_in, rot)
-            ctx.kept[i] = None
-            dxa, dmsg, g = _ffn_bwd(k, w, "s", x_in, msg, dxm)
-            for name, val in g.items():
-                grads[(i, name)] = val
-            grads[(i, "so_w")], grads[(i, "so_b")], dc = _proj_bwd(k, w, "so_w", dmsg, c)
-            dq, dk, dv = k.attention_bwd(q, kk, v, c, dc, 0)
-            dqkv = k.heads_bwd(dq, dk, dv, q, kk, rot, 3, (Q_SCALE, 1.0, 1.0), dtheta)
-            perm = _PERM.to(dqkv.device)
-            gw = torch.empty(768, 256, device=dqkv.device, dtype=torch.float32)
-            gb = torch.empty(768, device=dqkv.device, dtype=torch.float32)
-            gw[perm], gb[perm], dxp = _proj_bwd(k, w, "qkv_w", dqkv, x_in)
-            grads[(i, "qkv_w")], grads[(i, "qkv_b")] = gw, gb
-            dx = dxm + dxa + dxp
-        # positional encoding: theta = Wr . normalised keypoints (lightglue.py:61-66)
-        grads["wr"] = dtheta.t() @ _posenc_rows(k, geom)
-        need = ctx.needs_input_grad
-        gk0, gk1 = k.posenc_bwd(geom, W["wr"], dtheta, need[4:6])
-        if ctx.xin is not None:  # input_proj (lightglue.py:464-465)
-            grads["in_w"], grads["in_b"] = dx.t() @ ctx.xin, dx.sum(0)
-            dx = dx @ W["in_w"]
-        gd0, gd1 = k.unpack(k.mask_rows(dx))
-        return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None, gk0, gk1,
-                *[grads[key] if need[6 + j] else None for j, key in enumerate(ctx.keys)])
-
-
-# ---- bf16 mixed-precision training (conf.train_precision = "bf16") ------------------------------------------------
+    def input_proj_bwd(self, dx, xin):
+        """(d input_proj.weight, d input_proj.bias, d its input) from dx [T,256] (lightglue.py:464-465)."""
+        return dx.t() @ xin, dx.sum(0), dx @ self.W["in_w"]
 
 
 def _mm16(a, b):
@@ -578,110 +432,130 @@ def _mm16(a, b):
     return torch.mm(a.to(torch.bfloat16), b.to(torch.bfloat16), out_dtype=torch.float32)
 
 
-def _self_attend16(k: _Kern, w: Dict, x, rot16):
-    """Self block up to the context, as the no-grad bf16 forward runs it: (q, k, v, ctx), all bf16."""
-    q, kk, v = k.zeros16(k.T * 256), k.zeros16(k.T * 256), k.zeros16(k.T * 256)
-    k.linear16(EPI_HEADS, x, w["qkv_w"], w["qkv_b"], 768, 256, scale=(Q_SCALE, 1.0, 1.0), rot16=rot16, n_rot=2,
-               outp=(q, kk, v))
-    return q, kk, v, k.attention16(q, kk, v, 0)
+class _Bf16Blocks:
+    """conf.train_precision = "bf16": the bf16 inference kernels forward, with the arguments of the no-grad forward with
+    precision="bf16" (bf16 pack with out_proj / to_out folded into the first FFN matrix, bf16 residual stream, rot16),
+    one bf16 tensor-core GEMM with fp32 output for every plain GEMM of the backward.  Saved tuples: (q, k, v, ctx) /
+    (qk, v, ctx), bf16."""
+
+    def __init__(self, k: _Kern, model):
+        self.k, self.model = k, model
+        self.W = model._pack(BF16, k.dev)
+
+    def stage(self, desc0, desc1):
+        """-> (x [T,256] bf16: the first block input, the staged input of input_proj or None)"""
+        k = self.k
+        x = k.pack2(desc0, desc1, torch.bfloat16)
+        if not isinstance(self.model.input_proj, nn.Linear):
+            return x, None
+        out = k.zeros16(k.T, 256)
+        k.linear16(EPI_ROWMAJOR, x, self.W["in_w"], self.W["in_b"], 256, x.shape[1], out=out, lens=False)
+        return out, x
+
+    def posenc(self, geom):
+        """self.rot: fp32 angles [T,64] for lgb200_heads_bwd; self.rot16 [T,32]: packed fp16 cos / sin for the
+        forward's QKV epilogue (one call)."""
+        k = self.k
+        self.rot = k.zeros(k.T, 64)
+        self.rot16 = torch.zeros(k.T, 32, device=k.dev, dtype=torch.int32)
+        k.posenc(geom, self.W["wr"], self.rot, self.rot16)
+
+    def self_attend(self, w, x, heads: bool = True):
+        """Self block up to the context, as the no-grad bf16 forward runs it: (q, k, v, ctx), kept whatever `heads`."""
+        k = self.k
+        q, kk, v = k.zeros16(k.T * 256), k.zeros16(k.T * 256), k.zeros16(k.T * 256)
+        k.linear16(EPI_HEADS, x, w["qkv_w"], w["qkv_b"], 768, 256, scale=(Q_SCALE, 1.0, 1.0), rot16=self.rot16, n_rot=2,
+                   outp=(q, kk, v))
+        return q, kk, v, k.attention16(q, kk, v, 0)
+
+    def cross_attend(self, w, x, heads: bool = True):
+        k = self.k
+        qk, v = k.zeros16(k.T * 256), k.zeros16(k.T * 256)
+        k.linear16(EPI_HEADS, x, w["cqv_w"], w["cqv_b"], 512, 256, scale=(C_SCALE, 1.0, 1.0), rot16=self.rot16, n_rot=0,
+                   outp=(qk, v, None))
+        return qk, v, k.attention16(qk, qk, v, 1)
+
+    def ffn(self, w, pre: str, x, s):
+        """x + ffn(cat[x, out_proj(ctx)]) with out_proj folded into the first FFN matrix, ctx = s[-1]: a new bf16
+        tensor."""
+        k = self.k
+        hid = k.zeros16(k.T, 512)
+        k.linear16(EPI_LN_GELU, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=s[-1], K0=256, gamma=w[pre + "ln_g"],
+                   beta=w[pre + "ln_b"], out=hid)
+        out = x.clone()  # (the no-grad forward updates its residual stream in place; the block input is kept here)
+        k.linear16(EPI_ROWMAJOR, hid, w[pre + "f3_w"], w[pre + "f3_b"], 256, 512, resid=out, out=out)
+        return out
+
+    def ffn_bwd(self, i: int, w, pre: str, x, s, dy):
+        """Backward of y = ffn(cat[x, proj(c)]) in the folded form h = [W1x | W1m.Wo].cat[x, c] + (b1 + W1m.bo), given
+        dy [T,256] and the saved tuple s (c = s[-1]): (d x through the ffn, d c, parameter gradients incl. those of
+        proj).  With G = dh^T c (the [512,256] block of d W1') and gb = sum dh: dW1m = G Wo^T + gb bo^T (W1m enters the
+        folded bias too), dWo = W1m^T G, dbo = W1m^T gb, db1 = gb."""
+        k, c = self.k, s[-1]
+        blk = self.model.transformers[i]
+        ffn0, proj = (blk.self_attn.ffn[0], blk.self_attn.out_proj) if pre == "s" else \
+            (blk.cross_attn.ffn[0], blk.cross_attn.to_out)
+        h = k.empty(k.T, 512)  # pre-LayerNorm activations, recomputed in fp32 from the same bf16 operands
+        k.linear16(EPI_ROWMAJOR, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=c, K0=256, out32=h)
+        dy16 = dy.to(torch.bfloat16)
+        da = _mm16(dy16, w[pre + "f3_w"])
+        dh, act, gsum = k.ln_gelu_bwd(h, w[pre + "ln_g"], w[pre + "ln_b"], da)
+        dh16 = dh.to(torch.bfloat16)
+        g3 = _mm16(dy16.t(), act)
+        gx, G = _mm16(dh16.t(), x), _mm16(dh16.t(), c)
+        dcat = _mm16(dh16, w[pre + "f0_w"])
+        gb = dh.sum(0)
+        d = proj.weight.shape[0]
+        w1m, wo, bo = ffn0.weight.detach()[:, d:], proj.weight.detach(), proj.bias.detach()
+        po = "so" if pre == "s" else "co"
+        g = {
+            pre + "f3_w": g3, pre + "f3_b": dy.sum(0),
+            pre + "ln_g": gsum[:512], pre + "ln_b": gsum[512:],
+            pre + "f0_w": torch.cat([gx, G @ wo.t() + torch.outer(gb, bo)], 1), pre + "f0_b": gb,
+            po + "_w": w1m.t() @ G, po + "_b": w1m.t() @ gb,
+        }
+        return dcat[:, :256], dcat[:, 256:].contiguous(), g
+
+    def proj_bwd(self, w, name: str, dy, x):
+        """Backward of y = x W^T + b with bf16 x / W = w[name]: (dy^T x, dy^T 1, dy W)."""
+        dy16 = dy.to(torch.bfloat16)
+        return _mm16(dy16.t(), x), dy.sum(0), _mm16(dy16, w[name])
+
+    def input_proj_bwd(self, dx, xin):
+        """(d input_proj.weight, d input_proj.bias, d its input) from dx [T,256] (lightglue.py:464-465)."""
+        return dx.t() @ xin.float(), dx.sum(0), dx @ self.model.input_proj.weight.detach()
 
 
-def _cross_attend16(k: _Kern, w: Dict, x, rot16):
-    qk, v = k.zeros16(k.T * 256), k.zeros16(k.T * 256)
-    k.linear16(EPI_HEADS, x, w["cqv_w"], w["cqv_b"], 512, 256, scale=(C_SCALE, 1.0, 1.0), rot16=rot16, n_rot=0,
-               outp=(qk, v, None))
-    return qk, v, k.attention16(qk, qk, v, 1)
-
-
-def _ffn16(k: _Kern, w: Dict, pre: str, x, c):
-    """x + ffn(cat[x, out_proj(c)]) with out_proj folded into the first FFN matrix (bf16 pack): a new bf16 tensor."""
-    hid = k.zeros16(k.T, 512)
-    k.linear16(EPI_LN_GELU, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=c, K0=256, gamma=w[pre + "ln_g"],
-               beta=w[pre + "ln_b"], out=hid)
-    out = x.clone()  # (the no-grad forward updates its residual stream in place; the block input is kept here)
-    k.linear16(EPI_ROWMAJOR, hid, w[pre + "f3_w"], w[pre + "f3_b"], 256, 512, resid=out, out=out)
-    return out
-
-
-def _ffn_bwd16(k: _Kern, w: Dict, pre: str, ffn0: nn.Linear, proj: nn.Linear, x, c, dy):
-    """Backward of y = x + ffn(cat[x, proj(c)]) in the bf16 forward's folded form h = [W1x | W1m.Wo].cat[x, c] +
-    (b1 + W1m.bo), given dy [T,256]: (d x through the ffn, d c, parameter gradients incl. those of proj).  With
-    G = dh^T c (the [512,256] block of d W1') and gb = sum dh: dW1m = G Wo^T + gb bo^T (W1m enters the folded bias
-    too), dWo = W1m^T G, dbo = W1m^T gb, db1 = gb."""
-    h = k.empty(k.T, 512)  # pre-LayerNorm activations, recomputed in fp32 from the same bf16 operands
-    k.linear16(EPI_ROWMAJOR, x, w[pre + "f0_w"], w[pre + "f0_b"], 512, 512, A1=c, K0=256, out32=h)
-    dy16 = dy.to(torch.bfloat16)
-    da = _mm16(dy16, w[pre + "f3_w"])
-    dh, act, gsum = k.ln_gelu_bwd(h, w[pre + "ln_g"], w[pre + "ln_b"], da)
-    dh16 = dh.to(torch.bfloat16)
-    g3 = _mm16(dy16.t(), act)
-    gx, G = _mm16(dh16.t(), x), _mm16(dh16.t(), c)
-    dcat = _mm16(dh16, w[pre + "f0_w"])
-    gb = dh.sum(0)
-    d = proj.weight.shape[0]
-    w1m, wo, bo = ffn0.weight.detach()[:, d:], proj.weight.detach(), proj.bias.detach()
-    po = "so" if pre == "s" else "co"
-    g = {
-        pre + "f3_w": g3, pre + "f3_b": dy.sum(0),
-        pre + "ln_g": gsum[:512], pre + "ln_b": gsum[512:],
-        pre + "f0_w": torch.cat([gx, G @ wo.t() + torch.outer(gb, bo)], 1), pre + "f0_b": gb,
-        po + "_w": w1m.t() @ G, po + "_b": w1m.t() @ gb,
-    }
-    return dcat[:, :256], dcat[:, 256:].contiguous(), g
-
-
-def _proj_bwd16(dy, x, w16):
-    """Backward of y = x W^T + b with bf16 x / W: (dy^T x, dy^T 1, dy W)."""
-    dy16 = dy.to(torch.bfloat16)
-    return _mm16(dy16.t(), x), dy.sum(0), _mm16(dy16, w16)
-
-
-class TransformerBf16Fn(torch.autograd.Function):
-    """TransformerFn for conf.train_precision = "bf16": ref_descriptors0/1 (bf16, as the no-grad bf16 forward returns
-    them) with the bf16 inference kernels forward and bf16 tensor-core products backward."""
+class TransformerFn(torch.autograd.Function):
+    """ref_descriptors0/1 = all layers' outputs of the transformer stack (lightglue.py:456-498) in conf.train_precision:
+    fp32, or bf16 as the no-grad bf16 forward returns them."""
 
     @staticmethod
     def forward(ctx, model, geom: Dict, desc0, desc1, k0, k1, *params):
-        dev = desc0.device
+        """k0 / k1 [B, m / n, kdim]: the staged keypoint rows (coordinates, plus scale and orientation with
+        add_scale_ori) -- inputs, so that their gradient reaches whatever the caller built them from."""
         B, m, _ = desc0.shape
         n = desc1.shape[1]
         geom = dict(geom, k0=k0, k1=k1)
-        k = _Kern(dev, B, m, n, geom.get("counts"))
-        W = model._pack(BF16, dev)
-        L = model.conf.n_layers
-        xin = None
-        if isinstance(model.input_proj, nn.Linear):
-            din = model.conf.input_dim
-            xin = k.zeros16(k.T, din)
-            x = k.zeros16(k.T, 256)
-            for img, dsc, cnt in ((0, desc0, m), (1, desc1, n)):
-                check(k.lib.lgb200_pack_rows(ptr(dsc.contiguous()), B, cnt, din, img, k.Lp, None, ptr(xin), k.st),
-                      "lgb200_pack_rows")
-            k.mask_rows(xin)
-            k.linear16(EPI_ROWMAJOR, xin, W["in_w"], W["in_b"], 256, din, out=x, lens=False)
-        else:
-            x = k.zeros16(k.T, 256)
-            for img, dsc, cnt in ((0, desc0, m), (1, desc1, n)):
-                check(k.lib.lgb200_pack_rows(ptr(dsc.contiguous()), B, cnt, 256, img, k.Lp, None, ptr(x), k.st),
-                      "lgb200_pack_rows")
-            k.mask_rows(x)
-        rot = k.zeros(k.T, 64)  # fp32 angles for lgb200_heads_bwd, rot16 for the forward's QKV epilogue (one call)
-        rot16 = torch.zeros(k.T, 32, device=dev, dtype=torch.int32)
-        k.posenc(geom, W["wr"], rot, rot16)
+        k = _Kern(desc0.device, B, m, n, geom.get("counts"))
+        P = (_Bf16Blocks if model._train_bf16() else _F32Blocks)(k, model)
+        x, xin = P.stage(desc0, desc1)
+        P.posenc(geom)
+        # conf.checkpointed (lightglue.py:485-494): keep only the block inputs and recompute q / k / v / context /
+        # message in the backward pass (26 x T KB per layer less in fp32); otherwise they are kept, as autograd would
         keep = not bool(model.conf.checkpointed)
         xs_in, xs_mid, outs, kept = [], [], [], []
-        for i in range(L):
-            w = W["layers"][i]
+        for w in P.W["layers"]:
             xs_in.append(x)
-            sa = _self_attend16(k, w, x, rot16)
-            x = _ffn16(k, w, "s", x, sa[-1])
+            sa = P.self_attend(w, x, heads=keep)
+            x = P.ffn(w, "s", x, sa)
             xs_mid.append(x)
-            ca = _cross_attend16(k, w, x, rot16)
-            x = _ffn16(k, w, "c", x, ca[-1])
+            ca = P.cross_attend(w, x, heads=keep)
+            x = P.ffn(w, "c", x, ca)
             outs.append(x)
             kept.append((sa, ca) if keep else None)
-        ctx.k, ctx.W, ctx.geom, ctx.model = k, W, geom, model
-        ctx.xs_in, ctx.xs_mid, ctx.rot, ctx.rot16, ctx.xin, ctx.kept = xs_in, xs_mid, rot, rot16, xin, kept
+        ctx.P, ctx.geom = P, geom
+        ctx.xs_in, ctx.xs_mid, ctx.xin, ctx.kept = xs_in, xs_mid, xin, kept
         ctx.keys = [key for key, _ in transformer_params(model)]
         r0 = torch.stack([k.unpack(o)[0] for o in outs], 1)
         r1 = torch.stack([k.unpack(o)[1] for o in outs], 1)
@@ -689,49 +563,48 @@ class TransformerBf16Fn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g0, g1):
-        k, W, geom, model = ctx.k, ctx.W, ctx.geom, ctx.model
-        L = len(ctx.xs_in)
-        rot, rot16 = ctx.rot, ctx.rot16
+        P, geom = ctx.P, ctx.geom
+        k, rot = P.k, P.rot
         dx = k.zeros(k.T, 256)
         dtheta = k.zeros(k.T, 32)
         grads: Dict[object, torch.Tensor] = {}
         perm = _PERM.to(dx.device)
-        for i in reversed(range(L)):
-            w = W["layers"][i]
-            sa_m, ca_m = model.transformers[i].self_attn, model.transformers[i].cross_attn
+        for i in reversed(range(len(ctx.xs_in))):
+            w = P.W["layers"][i]
             dx = dx + k.pack2(g0[:, i], g1[:, i])
             x_in, x_mid = ctx.xs_in[i], ctx.xs_mid[i]
             # ---- cross block (lightglue.py:193-222) ----
-            qk, v, c = ctx.kept[i][1] if ctx.kept[i] is not None else _cross_attend16(k, w, x_mid, rot16)
-            dxa, dc, g = _ffn_bwd16(k, w, "c", ca_m.ffn[0], ca_m.to_out, x_mid, c, dx)
+            s = ctx.kept[i][1] if ctx.kept[i] is not None else P.cross_attend(w, x_mid)
+            qk, v, c = s[:3]  # (unpacked here: releases the previous block's v / c before the FFN backward)
+            dxa, dc, g = P.ffn_bwd(i, w, "c", x_mid, s, dx)
             for name, val in g.items():
                 grads[(i, name)] = val
-            dq, dk, dv = k.attention_bwd16(qk, qk, v, c, dc, 1)
+            dq, dk, dv = k.attention_bwd(qk, qk, v, c, dc, 1)
             dqv = k.heads_bwd(dq, dk, dv, None, None, None, 2, (C_SCALE, 1.0, 1.0), None)
-            gw, gb, dxp = _proj_bwd16(dqv, x_mid, w["cqv_w"])
+            gw, gb, dxp = P.proj_bwd(w, "cqv_w", dqv, x_mid)
             grads[(i, "cqk_w")], grads[(i, "cv_w")] = gw[:256], gw[256:]
             grads[(i, "cqk_b")], grads[(i, "cv_b")] = gb[:256], gb[256:]
             dxm = dx + dxa + dxp
             # ---- self block (lightglue.py:151-164) ----
-            q, kk, v, c = ctx.kept[i][0] if ctx.kept[i] is not None else _self_attend16(k, w, x_in, rot16)
+            s = ctx.kept[i][0] if ctx.kept[i] is not None else P.self_attend(w, x_in)
             ctx.kept[i] = None
-            dxa, dc, g = _ffn_bwd16(k, w, "s", sa_m.ffn[0], sa_m.out_proj, x_in, c, dxm)
+            q, kk, v, c = s[:4]
+            dxa, dc, g = P.ffn_bwd(i, w, "s", x_in, s, dxm)
             for name, val in g.items():
                 grads[(i, name)] = val
-            dq, dk, dv = k.attention_bwd16(q, kk, v, c, dc, 0)
+            dq, dk, dv = k.attention_bwd(q, kk, v, c, dc, 0)
             dqkv = k.heads_bwd(dq, dk, dv, q.float(), kk.float(), rot, 3, (Q_SCALE, 1.0, 1.0), dtheta)
             gw = torch.empty(768, 256, device=dqkv.device, dtype=torch.float32)
             gb = torch.empty(768, device=dqkv.device, dtype=torch.float32)
-            gw[perm], gb[perm], dxp = _proj_bwd16(dqkv, x_in, w["qkv_w"])
+            gw[perm], gb[perm], dxp = P.proj_bwd(w, "qkv_w", dqkv, x_in)
             grads[(i, "qkv_w")], grads[(i, "qkv_b")] = gw, gb
             dx = dxm + dxa + dxp
         # positional encoding: theta = Wr . normalised keypoints (lightglue.py:61-66)
         grads["wr"] = dtheta.t() @ _posenc_rows(k, geom)
         need = ctx.needs_input_grad
-        gk0, gk1 = k.posenc_bwd(geom, W["wr"], dtheta, need[4:6])
+        gk0, gk1 = k.posenc_bwd(geom, P.W["wr"], dtheta, need[4:6])
         if ctx.xin is not None:  # input_proj (lightglue.py:464-465)
-            grads["in_w"], grads["in_b"] = dx.t() @ ctx.xin.float(), dx.sum(0)
-            dx = dx @ model.input_proj.weight.detach()
+            grads["in_w"], grads["in_b"], dx = P.input_proj_bwd(dx, ctx.xin)
         gd0, gd1 = k.unpack(k.mask_rows(dx))
         return (None, None, gd0.contiguous() if need[2] else None, gd1.contiguous() if need[3] else None, gk0, gk1,
                 *[grads[key] if need[6 + j] else None for j, key in enumerate(ctx.keys)])
@@ -748,23 +621,20 @@ class AssignFn(torch.autograd.Function):
     def forward(ctx, model, layer: int, gt, counts, d0, d1, fp_w, fp_b, m_w, m_b):
         lib = _abi.load()
         keep: Dict = {}
-        bf = model._train_bf16()
-        prec = BF16 if bf else (F32 if _SIMT_LINEAR else F32X3)
         pos_sum, pos_cnt, row_exp, row_arg, col_arg, dust0, dust1, _ = model._log_assignment_of(
-            lib, prec, d0, d1, layer, gt, keep=keep, counts=counts)
-        ctx.save_for_backward(d0, d1, fp_w, fp_b, m_w, gt, keep["z"], keep["lse"])
+            lib, BF16 if model._train_bf16() else F32X3, d0, d1, layer, gt, keep=keep, counts=counts)
+        ctx.save_for_backward(d0, d1, fp_w, m_w, gt, keep["z"], keep["lse"])
         ctx.counts = counts
         ctx.Lp = keep["Lp"]
-        # x3 mode: the split planes of final_proj(desc) / 4 (33 MB at 8 x 2048) -- the backward recomputes the similarity
-        # from them on tcgen05 instead of redoing final_proj and the N x M product in fp32 on the CUDA cores
-        ctx.md_planes, ctx.lens = (None, None) if (_SGEMM or bf) else (keep["md_planes"], keep["lens"])
-        ctx.md16 = keep["md16"] if bf else None  # bf16: final_proj(desc) / 4 as the forward's kernels computed it
+        # what the backward recomputes the similarity from: x3 mode, the split planes of final_proj(desc) / 4 (33 MB at
+        # 8 x 2048, recomputed on tcgen05); bf16, final_proj(desc) / 4 as the forward's kernels computed it
+        ctx.md_planes, ctx.md16, ctx.lens = keep["md_planes"], keep["md16"], keep["lens"]
         ctx.mark_non_differentiable(pos_cnt, row_exp, row_arg, col_arg)
         return pos_sum, dust0.contiguous(), dust1.contiguous(), pos_cnt, row_exp, row_arg, col_arg
 
     @staticmethod
     def backward(ctx, g_pos, g_d0, g_d1, *_):
-        d0, d1, fp_w, fp_b, m_w, gt, z, lse = ctx.saved_tensors
+        d0, d1, fp_w, m_w, gt, z, lse = ctx.saved_tensors
         lib = _abi.load()
         B, m, _ = d0.shape
         n = d1.shape[1]
@@ -772,7 +642,7 @@ class AssignFn(torch.autograd.Function):
         dev = d0.device
         x0, x1 = d0.to(torch.float32), d1.to(torch.float32)
         st = torch.cuda.current_stream(dev).cuda_stream
-        sim, md = _assign_similarity(lib, st, x0, x1, fp_w, fp_b, ctx.md_planes, ctx.md16, ctx.lens, Lp)
+        sim, md = _assign_similarity(lib, st, x0, x1, ctx.md_planes, ctx.md16, ctx.lens, Lp)
         g = (g_pos if g_pos is not None else torch.zeros(B, device=dev)).to(torch.float32).contiguous()
         r = (g[:, None] * gt.sum(2)).contiguous()
         c = (g[:, None] * gt.sum(1)).contiguous()
@@ -794,10 +664,10 @@ class AssignFn(torch.autograd.Function):
                 *_assign_input_grads(lib, st, sim, dz0, dz1, x0, x1, fp_w, m_w, md, ctx.md_planes, Lp, counts))
 
 
-def _assign_similarity(lib, st, x0, x1, fp_w, fp_b, mdp, md16, lens, Lp):
+def _assign_similarity(lib, st, x0, x1, mdp, md16, lens, Lp):
     """The similarity [B,m,n] fp32 of MatchAssignment (lightglue.py:281-284) recomputed for a backward pass from what
-    the forward kept -> (sim, (md0, md1)); (md0, md1) = final_proj(desc) / 4 for the d md products (None with the
-    split planes mdp of the x3 mode).  md16: the bf16 forward's md."""
+    the forward kept -- the split planes mdp of final_proj(desc) / 4 in the x3 mode, or md16 = final_proj(desc) / 4 of the
+    bf16 forward -> (sim, md); md = (md0, md1) of the bf16 forward for the d md products, None in the x3 mode."""
     B, m, _ = x0.shape
     n = x1.shape[1]
     f32 = torch.float32
@@ -805,10 +675,6 @@ def _assign_similarity(lib, st, x0, x1, fp_w, fp_b, mdp, md16, lens, Lp):
         mv = md16.view(B, 2, Lp, 256)
         md0, md1 = mv[:, 0, :m], mv[:, 1, :n]
         return torch.bmm(md0, md1.transpose(1, 2), out_dtype=f32).contiguous(), (md0, md1)
-    if mdp is None:
-        md0 = torch.addmm(fp_b, x0.reshape(-1, 256), fp_w.t()).view(B, m, 256) * 0.25  # lightglue.py:281-283
-        md1 = torch.addmm(fp_b, x1.reshape(-1, 256), fp_w.t()).view(B, n, 256) * 0.25
-        return torch.bmm(md0, md1.transpose(1, 2)).contiguous(), (md0, md1)
     sim = torch.empty(B, Lp, Lp, device=x0.device, dtype=f32)
     check(lib.lgb200_x3_similarity(ptr(mdp), B, Lp, ptr(lens), ptr(sim), st), "x3_similarity")
     return sim[:, :m, :n].contiguous(), None
@@ -821,15 +687,11 @@ def _assign_input_grads(lib, st, sim, dz0, dz1, x0, x1, fp_w, m_w, md, mdp, Lp, 
     B, m, n = sim.shape
     dev = sim.device
     f32 = torch.float32
-    if md is not None and md[0].dtype == torch.bfloat16:
+    if md is not None:  # bf16
         md0, md1 = md
         s16 = sim.to(torch.bfloat16)
         dmd0 = torch.bmm(s16, md1, out_dtype=f32)
         dmd1 = torch.bmm(s16.transpose(1, 2), md0, out_dtype=f32)
-    elif mdp is None:
-        md0, md1 = md
-        dmd0 = torch.bmm(sim, md1)
-        dmd1 = torch.bmm(sim.transpose(1, 2), md0)
     else:  # three fp16 tensor-core products per GEMM, as _Kern.mm3
         sp = torch.empty(2, B, m, n, device=dev, dtype=torch.float16)
         inv = torch.empty(2, device=dev, dtype=torch.float32)
@@ -871,16 +733,13 @@ class LogAssignFn(torch.autograd.Function):
     def forward(ctx, model, layer: int, counts, d0, d1, fp_w, fp_b, m_w, m_b):
         lib = _abi.load()
         keep: Dict = {}
-        bf = model._train_bf16()
-        if bf:
+        if model._train_bf16():
             scores, m0, m1, ms0, ms1 = model._assign_match_bf16(lib, d0, d1, layer, counts, keep=keep)
-        else:
-            # (fp32-accurate tensor-core kernels, as the rest of the training forward; CUDA cores with
-            # LGB200_TRAIN_SIMT_LINEAR=1)
+        else:  # (the fp32-accurate tensor-core kernels, as the rest of the training forward)
             dev = d0.device
             B, m, _ = d0.shape
             n = d1.shape[1]
-            model._log_assignment_of(lib, F32 if _SIMT_LINEAR else F32X3, d0, d1, layer, None, keep=keep, counts=counts)
+            model._log_assignment_of(lib, F32X3, d0, d1, layer, None, keep=keep, counts=counts)
             scores = keep["scores"]
             m0 = torch.empty(B, m, device=dev, dtype=torch.int64)
             m1 = torch.empty(B, n, device=dev, dtype=torch.int64)
@@ -891,16 +750,15 @@ class LogAssignFn(torch.autograd.Function):
             check(lib.lgb200_filter_matches(ptr(scores), B, m + 1, n + 1, ptr(keep["lens"]),
                                             float(model.conf.filter_threshold), None, None, 0, m, n, ptr(m0), ptr(m1),
                                             ptr(ms0), ptr(ms1), ptr(keep["fm_ws"]), 0, st), "filter_matches")
-        ctx.save_for_backward(d0, d1, fp_w, fp_b, m_w, keep["z"], keep["lse"], keep["fm_ws"])
+        ctx.save_for_backward(d0, d1, fp_w, m_w, keep["z"], keep["lse"], keep["fm_ws"])
         ctx.counts, ctx.Lp = counts, keep["Lp"]
-        ctx.md_planes, ctx.lens = (None, keep["lens"]) if (_SGEMM or bf) else (keep["md_planes"], keep["lens"])
-        ctx.md16 = keep["md16"] if bf else None
+        ctx.md_planes, ctx.md16, ctx.lens = keep["md_planes"], keep["md16"], keep["lens"]
         ctx.mark_non_differentiable(m0, m1)
         return scores, m0, m1, ms0, ms1
 
     @staticmethod
     def backward(ctx, g_la, _g_m0, _g_m1, g_ms0, g_ms1):
-        d0, d1, fp_w, fp_b, m_w, z, lse, fm_ws = ctx.saved_tensors
+        d0, d1, fp_w, m_w, z, lse, fm_ws = ctx.saved_tensors
         lib = _abi.load()
         B, m, _ = d0.shape
         n = d1.shape[1]
@@ -931,7 +789,7 @@ class LogAssignFn(torch.autograd.Function):
                 G.index_put_((bi.expand(B, n), mm1.clamp(min=0), jj), torch.where(mm1 >= 0, g_ms1 * ms1, 0.0),
                              accumulate=True)
         x0, x1 = d0.to(torch.float32), d1.to(torch.float32)
-        sim, md = _assign_similarity(lib, st, x0, x1, fp_w, fp_b, ctx.md_planes, ctx.md16, ctx.lens, Lp)
+        sim, md = _assign_similarity(lib, st, x0, x1, ctx.md_planes, ctx.md16, ctx.lens, Lp)
         dz0 = torch.empty(B, m, device=dev, dtype=torch.float32)
         dz1 = torch.empty(B, n, device=dev, dtype=torch.float32)
         n_ws = C.c_longlong(0)

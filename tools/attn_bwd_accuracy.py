@@ -1,5 +1,5 @@
 """Attention backward (lgb200_attention_bwd) against float64 autograd at long sequences: relative error (norm-wise and
-largest entry) of dQ / dK / dV.  usage: attn_bwd_accuracy.py [S] [Lp]   (LGB200_ATTN_BWD_MMASYNC=1: the warp-MMA kernels)"""
+largest entry) of dQ / dK / dV.  usage: attn_bwd_accuracy.py [S] [Lp]"""
 import ctypes
 import math
 import sys

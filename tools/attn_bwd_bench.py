@@ -2,8 +2,7 @@
 inputs: the fp32 entry lgb200_attention_bwd (csrc/lg_bwd.cu -> the x3 tcgen05 kernel) and the bf16 entry
 lgb200_attention_bwd_bf16 (the same kernel template on bf16 operands, fed by the bf16 forward).  Prints ms per call and
 the useful TFLOP/s on one product count for both (8 tile products of 2.Lp^2.64 per head: 1 statistics + 3 dQ +
-4 dK/dV), and the card's name and power limit.  Usage: python tools/attn_bwd_bench.py [S] [Lp] [reps]
-(LGB200_ATTN_BWD_SIMT=1: CUDA-core kernels in the fp32 arm)"""
+4 dK/dV), and the card's name and power limit.  Usage: python tools/attn_bwd_bench.py [S] [Lp] [reps]"""
 import ctypes
 import sys
 from pathlib import Path

@@ -8,12 +8,14 @@ untouched.  One JSON line per measurement, plus the card's name and power limit.
    own process, the two alternating (--parent DIR: a copy of the parent commit's package, e.g. exported with
    `git archive HEAD~1 glue_factory_colon_b200 | tar -x -C DIR`, built with its own build.py):
      "today"  LightGlue.loss's total, descriptors requiring grad (the step both versions run): ms per step, peak
-              memory, launches per step; the losses and every gradient of one seeded step are dumped by both versions
-              and compared bit for bit;
+              memory, launches per step;
      "extra"  the same plus sum W.log_assignment + sum v.matching_scores0 + sum u.matching_scores1 (this version only),
               with and without keypoints that require grad.
+   Both versions also run one seeded step of every case in DUMP_CASES and dump a digest of its losses, forward outputs,
+   parameter gradients and input gradients; the digests are compared per case (bit_equal_to_parent).
 The dumps go to a temporary directory.  Usage: python tools/la_grad_bench.py [--parent DIR] [--steps K] [--rounds R]"""
 import argparse
+import hashlib
 import json
 import os
 import shutil
@@ -26,6 +28,28 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parents[1]
 HBM_BYTES_PER_S = 7.7e12
 CONFIGS = ((32, 512), (8, 2048))
+# name -> (conf over the timed model's, make_pairs arguments, counts, inputs that require grad, loss mode).  counts:
+# num_keypoints0/1 below the padded size, and an empty side in the last pair.
+KPTS = ("keypoints0", "keypoints1", "scales0", "scales1", "oris0", "oris1")
+DUMP_CASES = {
+    "today": ({}, {}, False, (), "today"),
+    "checkpointed": ({"checkpointed": True}, {}, False, (), "today"),
+    "padded_counts": ({}, {}, True, (), "extra"),
+    "dim128_scale_ori": ({"input_dim": 128, "add_scale_ori": True}, {"dim": 128, "scale_ori": True}, False, KPTS,
+                         "extra"),
+    "extra": ({}, {}, False, (), "extra"),
+}
+OUTPUTS = ("ref_descriptors0", "ref_descriptors1", "log_assignment", "matches0", "matches1", "matching_scores0",
+           "matching_scores1")
+
+
+def digest(t):
+    """dtype, shape and SHA-256 of the bytes of t: equal digests are equal bits."""
+    import torch
+
+    t = t.detach().contiguous()
+    h = hashlib.sha256(t.reshape(-1).view(torch.uint8).cpu().numpy().tobytes()).hexdigest()
+    return f"{t.dtype} {tuple(t.shape)} {h}"
 
 
 def card():
@@ -106,9 +130,10 @@ def worker(args):
     W = torch.randn(B, N + 1, N + 1, device=dev, generator=g) * 1e-3
     v, u = torch.randn(B, N, device=dev, generator=g) * 0.1, torch.randn(B, N, device=dev, generator=g) * 0.1
 
-    def step(mode):
+    def step(mode, model=model, data=data, leaves=()):
         d = dict(data)
-        for k in ("descriptors0", "descriptors1") + (("keypoints0", "keypoints1") if mode == "extra_kpts" else ()):
+        leaves = ("descriptors0", "descriptors1") + leaves + (("keypoints0", "keypoints1") if mode == "extra_kpts" else ())
+        for k in leaves:
             d[k] = data[k].clone().requires_grad_(True)
         model.zero_grad(set_to_none=True)
         pred = model(d)
@@ -118,13 +143,25 @@ def worker(args):
             loss = loss + (W * pred["log_assignment"]).sum() + (v * pred["matching_scores0"]).sum() + \
                 (u * pred["matching_scores1"]).sum()
         loss.backward()
-        return losses, d
+        return losses, d, pred, leaves
 
     if args.dump:
-        losses, d = step("today")
-        out = {"loss." + k: t.detach().cpu() for k, t in losses.items()}
-        out.update({"grad." + k: p.grad.cpu() for k, p in model.named_parameters() if p.grad is not None})
-        out.update({"grad." + k: d[k].grad.cpu() for k in ("descriptors0", "descriptors1")})
+        out = {}
+        for case, (conf, kw, counts, leaves, mode) in DUMP_CASES.items():
+            torch.manual_seed(0)
+            m_ = LightGlue({"n_layers": 9, "filter_threshold": 0.1, "train_precision": args.prec, **conf}).to(dev).train()
+            d_ = to_device(make_pairs(B=B, n0=N, n1=N, seed=3, with_gt=True, **kw), dev)
+            if counts:
+                c0, c1 = [N - (61 * b) % N for b in range(B)], [N - (97 * b) % N for b in range(B)]
+                c1[-1] = 0
+                d_["num_keypoints0"], d_["num_keypoints1"] = torch.tensor(c0), torch.tensor(c1)
+            losses, d, pred, leaves = step(mode, m_, d_, leaves)
+            ts = {"loss." + k: t for k, t in losses.items()}
+            ts.update({"out." + k: pred[k] for k in OUTPUTS})
+            ts.update({"grad." + k: p.grad for k, p in m_.named_parameters() if p.grad is not None})
+            ts.update({"grad." + k: d[k].grad for k in leaves})
+            out.update({f"{case}/{k}": digest(t) for k, t in ts.items()})
+            del m_, d_, losses, d, pred, ts
         torch.save(out, args.dump)
     for mode in args.modes.split(","):
         for _ in range(2):
@@ -177,9 +214,12 @@ def main():
 
                 a = torch.load(out / f"branch_{B}x{N}_{prec}.pt")
                 b = torch.load(out / f"parent_{B}x{N}_{prec}.pt")
-                diff = sorted(k for k in set(a) | set(b) if k not in a or k not in b or not torch.equal(a[k], b[k]))
-                print(json.dumps({"B": B, "N": N, "train_precision": prec, "tensors_compared": len(a),
-                                  "bit_equal_to_parent": not diff, "differing": diff[:10]}), flush=True)
+                for case in DUMP_CASES:
+                    keys = {k for k in set(a) | set(b) if k.startswith(case + "/")}
+                    diff = sorted(k for k in keys if a.get(k) != b.get(k))
+                    print(json.dumps({"B": B, "N": N, "train_precision": prec, "case": case,
+                                      "tensors_compared": len(keys), "bit_equal_to_parent": not diff,
+                                      "differing": diff[:10]}), flush=True)
     shutil.rmtree(out)
 
 
