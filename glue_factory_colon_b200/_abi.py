@@ -17,6 +17,15 @@ ABI_VERSION = 8
 
 _p, _i, _f = C.c_void_p, C.c_int, C.c_float
 
+
+class MatchConfig(C.Structure):
+    """lgb200_match_config (the whole-matcher entry points)."""
+    _fields_ = [("precision", C.c_int), ("n_layers", C.c_int), ("input_dim", C.c_int), ("kdim", C.c_int),
+                ("filter_threshold", C.c_float)]
+
+
+_cfg = C.POINTER(MatchConfig)
+
 # name -> argtypes, exactly as declared in include/lightglue_b200.h
 SIGNATURES = {
     "lgb200_abi_version": [],
@@ -56,6 +65,11 @@ SIGNATURES = {
     "lgb200_assign_bwd": [_p, _p, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p, _p],
     "lgb200_assign_bwd_workspace": [_i, _i, _i, _p],
     "lgb200_posenc_bwd": [_p, _i, _i, _i, _p, _p, _p, _i, _i, _p, _p, _p],
+    "lgb200_weight_table_size": [_cfg, _p, _p],
+    "lgb200_pack_weights": [_cfg, _i, _p, _p, _p, C.c_longlong, _p, _p],
+    "lgb200_match_workspace": [_cfg, _i, _i, _i, _p],
+    "lgb200_match": [_cfg, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p,
+                     C.c_longlong, _p],
     "lgb200_prune_compact": [_p, _p, _f, _f, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
 }
 

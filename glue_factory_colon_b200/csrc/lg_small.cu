@@ -28,6 +28,7 @@ extern "C" const char* lgb200_error_string(int code) {
     case LGB200_ERR_PRECISION: return "unknown precision or epilogue";
     case LGB200_ERR_DRIVER: return "cuTensorMapEncodeTiled unavailable or failed";
     case LGB200_ERR_ARCH: return "device is not sm_100";
+    case LGB200_ERR_WEIGHTS: return "required weight missing";
     default: return code > 0 ? cudaGetErrorString((cudaError_t)code) : "unknown error";
   }
 }

@@ -9,7 +9,7 @@ CPU tensors written with the zipfile serializer (tools/convert_weights/official_
 from __future__ import annotations
 
 from pathlib import Path
-from typing import Dict, Mapping, Union
+from typing import Dict, List, Mapping, Tuple, Union
 
 import torch
 
@@ -67,3 +67,23 @@ def export_plain_state_dict(model: torch.nn.Module, path: Union[str, Path]) -> D
 def to_pipeline_state_dict(state: Mapping[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
     """`transformers.0...` -> `matcher.transformers.0...` (what `TwoViewPipeline.load_state_dict` expects)."""
     return {f"matcher.{k}": v for k, v in strip_prefixes(state).items()}
+
+
+# entry order of the packed-weight table of lgb200_match (include/lightglue_b200.h, "whole matcher")
+NATIVE_LAYER_ENTRIES = ("qkv_w", "qkv_b", "sf0_w", "sf0_b", "sln_g", "sln_b", "sf3_w", "sf3_b",
+                        "cqv_w", "cqv_b", "cf0_w", "cf0_b", "cln_g", "cln_b", "cf3_w", "cf3_b")
+
+
+def native_table(model: torch.nn.Module, prec: int) -> Tuple[object, List[torch.Tensor]]:
+    """The packed-weight table of lgb200_match built from `model._pack(prec)` on the model's device (prec = _abi.BF16
+    or _abi.F32X3): (ctypes array of device pointers, the tensors they point into).  The tensors must outlive every
+    call that uses the table."""
+    import ctypes
+
+    packed = model._pack(prec, next(model.parameters()).device)
+    tensors = [lyr[k] for lyr in packed["layers"] for k in NATIVE_LAYER_ENTRIES]
+    a = packed["assign"][-1]  # only the last layer's MatchAssignment runs in the forward
+    tensors += [packed["wr"], a["fp_w"], a["fp_b"], a["m_w"], a["m_b"]]
+    if "in_w" in packed:
+        tensors += [packed["in_w"], packed["in_b"]]
+    return (ctypes.c_void_p * len(tensors))(*[t.data_ptr() for t in tensors]), tensors

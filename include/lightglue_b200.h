@@ -5,8 +5,10 @@
  * of gluefactory/models/matchers/lightglue.py is a PyTorch library call.  Each
  * entry point below replaces the library call sites of one kernel family; the
  * reference file:line it replaces is cited per function (paths relative to the
- * reference checkout).  The only caller is the Python host mirror
- * glue_factory_colon_b200/lightglue.py (ctypes; see INTEGRATION.md).
+ * reference checkout).  The Python host mirror glue_factory_colon_b200/lightglue.py
+ * calls the kernel entry points (ctypes; see INTEGRATION.md); a native caller can
+ * run the whole matcher with lgb200_pack_weights + lgb200_match ("whole matcher",
+ * at the end; tools/native_match_demo.cpp uses nothing but this header).
  *
  * Conventions
  *   - All pointers are DEVICE pointers unless stated otherwise.  No entry point
@@ -48,7 +50,8 @@ enum {
   LGB200_ERR_NULL = -2,      /* required pointer missing                  */
   LGB200_ERR_PRECISION = -3, /* unknown precision / epilogue enum         */
   LGB200_ERR_DRIVER = -4,    /* cuTensorMapEncodeTiled unavailable/failed */
-  LGB200_ERR_ARCH = -5       /* device is not sm_100                      */
+  LGB200_ERR_ARCH = -5,      /* device is not sm_100                      */
+  LGB200_ERR_WEIGHTS = -6    /* required weight missing (lgb200_pack_weights) */
 };
 
 /* epilogues of lgb200_linear */
@@ -389,6 +392,94 @@ int lgb200_assign_bwd_workspace(int B, int m, int n, long long* n_floats);
  *   are 0.  Gradients w.r.t. size are not formed. */
 int lgb200_posenc_bwd(const float* kpts, int B, int n, int kdim, const float* size, const float* Wr,
                       const int32_t* lens, int img, int Lp, const float* dtheta, float* dkpts, void* stream);
+
+/* ---- whole matcher ------------------------------------------------------------------------------------------------
+ * The no-grad forward of LightGlue in eval mode with depth_confidence <= 0 and width_confidence <= 0 (lightglue.py:
+ * 422-553) behind two calls, for callers without the Python package (a C++ / LibTorch consumer of the plain-dict
+ * state dict, weights.py).  lgb200_match makes exactly the calls of LightGlue._forward_impl in the same order, with the
+ * same arguments, so its outputs are bit-equal to LightGlue.forward with the same weights, precision and counts. */
+typedef struct {
+  int precision;          /* LGB200_BF16 or LGB200_F32X3 (LightGlue precision "bf16" / "fp32"); else LGB200_ERR_PRECISION */
+  int n_layers;           /* >= 1 */
+  int input_dim;          /* 256, or the input_proj width: a positive multiple of 64 */
+  int kdim;               /* 2, or 4 with add_scale_ori (scale, orientation appended to the keypoints) */
+  float filter_threshold;
+} lgb200_match_config;
+
+/* Packed-weight table for `cfg`: *entries = 16 n_layers + 5 (+ 2 when input_dim != 256) and *pack_bytes = the device
+ * bytes lgb200_pack_weights fills (every entry starts on a 256-byte boundary).
+ *
+ * Entry order -- per layer l = 0 .. n_layers-1, at 16 l + j (the names of LightGlue._pack):
+ *    j  0 qkv_w  W [768][256]  Wqkv.weight, rows permuted head*192 + d*3 + part -> part*256 + head*64 + d
+ *       1 qkv_b  F [768]       Wqkv.bias, same permutation
+ *       2 sf0_w  W [512][512]  [W1x | W1m Wo]: self ffn.0 with out_proj folded in (float64, rounded to fp32 once)
+ *       3 sf0_b  F [512]       b1 + W1m bo
+ *       4 sln_g  F [512]       self ffn.1.weight       5 sln_b  F [512]  ffn.1.bias
+ *       6 sf3_w  W [256][512]  self ffn.3.weight       7 sf3_b  F [256]  ffn.3.bias
+ *       8 cqv_w  W [512][256]  to_qk.weight | to_v.weight (rows concatenated)
+ *       9 cqv_b  F [512]       to_qk.bias | to_v.bias
+ *      10 cf0_w  W [512][512]  cross ffn.0 with to_out folded in      11 cf0_b  F [512]
+ *      12 cln_g  F [512]       13 cln_b  F [512]       14 cf3_w  W [256][512]       15 cf3_b  F [256]
+ * then the tail, at t = 16 n_layers + j:
+ *    j  0 wr     F [32][kdim]  posenc.Wr.weight
+ *       1 fp_w   W [256][256]  log_assignment.{n_layers-1}.final_proj.weight     2 fp_b  F [256]
+ *       3 m_w    F [256]       log_assignment.{n_layers-1}.matchability.weight   4 m_b   F [1]
+ *       5 in_w   W [256][input_dim]  input_proj.weight (input_dim != 256 only)   6 in_b  F [256]
+ * W = weight matrix in the operand format of the precision: LGB200_BF16 bf16 [N][K]; LGB200_F32X3 fp16 planes
+ * [2][N][K] with 256 w = hi + lo (hi = fp16(256 w), lo = fp16(256 w - hi)).  F = fp32, copied as it is. */
+int lgb200_weight_table_size(const lgb200_match_config* cfg, int* entries, long long* pack_bytes);
+
+/* Packs the weights: tensors[i] (fp32, contiguous, DEVICE, the reference's shapes, which are not checked) is the
+ * state-dict tensor called names[i] (host strings, the keys of LightGlue.state_dict() with prefixes stripped as
+ * weights.strip_prefixes does).  Names not listed below are ignored; a missing one returns LGB200_ERR_WEIGHTS and a
+ * NULL tensor of a required name LGB200_ERR_NULL, before anything is launched.  Required names:
+ * BEGIN REQUIRED WEIGHTS
+ *   transformers.{l}.self_attn.Wqkv.weight          transformers.{l}.self_attn.Wqkv.bias
+ *   transformers.{l}.self_attn.out_proj.weight      transformers.{l}.self_attn.out_proj.bias
+ *   transformers.{l}.self_attn.ffn.0.weight         transformers.{l}.self_attn.ffn.0.bias
+ *   transformers.{l}.self_attn.ffn.1.weight         transformers.{l}.self_attn.ffn.1.bias
+ *   transformers.{l}.self_attn.ffn.3.weight         transformers.{l}.self_attn.ffn.3.bias
+ *   transformers.{l}.cross_attn.to_qk.weight        transformers.{l}.cross_attn.to_qk.bias
+ *   transformers.{l}.cross_attn.to_v.weight         transformers.{l}.cross_attn.to_v.bias
+ *   transformers.{l}.cross_attn.to_out.weight       transformers.{l}.cross_attn.to_out.bias
+ *   transformers.{l}.cross_attn.ffn.0.weight        transformers.{l}.cross_attn.ffn.0.bias
+ *   transformers.{l}.cross_attn.ffn.1.weight        transformers.{l}.cross_attn.ffn.1.bias
+ *   transformers.{l}.cross_attn.ffn.3.weight        transformers.{l}.cross_attn.ffn.3.bias
+ *   posenc.Wr.weight
+ *   log_assignment.{L-1}.final_proj.weight          log_assignment.{L-1}.final_proj.bias
+ *   log_assignment.{L-1}.matchability.weight        log_assignment.{L-1}.matchability.bias
+ *   input_proj.weight                               input_proj.bias              (input_dim != 256 only)
+ * END REQUIRED WEIGHTS
+ * for every layer l < L = n_layers.  (token_confidence and the other layers' log_assignment serve adaptive depth /
+ * width and the loss only.)  Writes the table's entries into pack_buf (pack_bytes from lgb200_weight_table_size) and
+ * the HOST array table[entries] with device pointers into pack_buf (256-byte aligned).  Runs on `stream`; no allocation, no
+ * synchronisation: the source tensors must stay valid until the stream has run the packing. */
+int lgb200_pack_weights(const lgb200_match_config* cfg, int n, const char* const* names,
+                        const float* const* tensors, void* pack_buf, long long pack_bytes,
+                        const void** table, void* stream);
+
+/* *bytes = the workspace of lgb200_match for B pairs of capacity m x n (it does not depend on the counts). */
+int lgb200_match_workspace(const lgb200_match_config* cfg, int B, int m, int n, long long* bytes);
+
+/* The forward.  table = the table filled by lgb200_pack_weights (or the same layouts built elsewhere).  Inputs fp32
+ * contiguous: kpts0/1 [B,m|n,kdim], desc0/1 [B,m|n,input_dim], size0/1 [B,2] (W,H) or NULL (extent of the valid
+ * points), counts0/1 DEVICE int32 [B] or NULL: per-pair valid counts of a padded batch (num_keypoints0/1), clamped to
+ * [0, m] / [0, n] on the device.  Outputs (every pointer non-NULL, also when m or n is 0, except desc_out0/1):
+ * matches0/1 int64 [B,m|n], scores0/1 fp32 [B,m|n] (matching_scores), log_assignment fp32 [B,m+1,n+1] (dustbin column
+ * n, dustbin row m: the padded layout of LightGlue.forward), desc_out0/1 (nullable) [B,m|n,256] in the activation dtype
+ * (bf16 / fp32) = the last layer's ref_descriptors.  workspace: lgb200_match_workspace bytes, 256-byte aligned.
+ * Kernel launches: those of LightGlue.forward with the same inputs, plus one (device-side lens and attention launch
+ * order) unless counts are NULL and m == n == Lp (Lp = max(m, n) rounded up to 128 in bf16, 256 in fp32, at least
+ * that granule: lens is then NULL, as in the Python forward); besides, cudaMemsetAsync where
+ * the Python forward allocates zeros and cudaMemcpy2DAsync for desc_out0/1.  No allocation, no synchronisation, no
+ * host read of device data, every operation on `stream`: a call can be captured into a CUDA graph at a capacity m x n
+ * and replayed with other inputs and counts written into the same buffers. */
+int lgb200_match(const lgb200_match_config* cfg, const void* const* table, int B, int m, int n,
+                 const float* kpts0, const float* kpts1, const float* desc0, const float* desc1,
+                 const float* size0, const float* size1, const int32_t* counts0, const int32_t* counts1,
+                 int64_t* matches0, int64_t* matches1, float* scores0, float* scores1,
+                 float* log_assignment, void* desc_out0, void* desc_out1,
+                 void* workspace, long long workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
