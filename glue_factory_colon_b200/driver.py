@@ -104,14 +104,14 @@ def collate_pairs(pairs: Sequence[dict], bucket: int = 128, pin: bool = False) -
 
 
 def crop_log_assignment(scores: torch.Tensor, n0: int, n1: int) -> torch.Tensor:
-    """[R, C] padded score matrix of one pair (valid block, dustbin column C-1, dustbin row R-1) -> the
-    [n0+1, n1+1] matrix the reference would have produced for the un-padded pair."""
-    R, C = scores.shape
-    out = scores.new_empty(n0 + 1, n1 + 1)
-    out[:n0, :n1] = scores[:n0, :n1]
-    out[:n0, n1] = scores[:n0, C - 1]
-    out[n0, :n1] = scores[R - 1, :n1]
-    out[n0, n1] = scores[R - 1, C - 1]
+    """[..., R, C] padded score matrices (valid block, dustbin column C-1, dustbin row R-1; leading dimensions, such as
+    a batch, are kept) -> the [..., n0+1, n1+1] matrices the reference would have produced for the un-padded pairs."""
+    R, C = scores.shape[-2:]
+    out = scores.new_empty(*scores.shape[:-2], n0 + 1, n1 + 1)
+    out[..., :n0, :n1] = scores[..., :n0, :n1]
+    out[..., :n0, n1] = scores[..., :n0, C - 1]
+    out[..., n0, :n1] = scores[..., R - 1, :n1]
+    out[..., n0, n1] = scores[..., R - 1, C - 1]
     return out
 
 

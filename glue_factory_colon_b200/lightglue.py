@@ -19,7 +19,10 @@ PyTorch fallback: CPU inputs raise.
 """
 from __future__ import annotations
 
+import ctypes
+import gc
 import math
+import numbers
 import os
 from typing import Dict, Optional
 
@@ -28,7 +31,9 @@ import torch
 from torch import nn
 
 from . import _abi
-from ._abi import BF16, EPI_HEADS, EPI_LN_GELU, EPI_ROWMAJOR, F32, F32X3, check, ptr
+from ._abi import BF16, EPI_HEADS, EPI_LN_GELU, EPI_ROWMAJOR, F32, F32X3, MatchConfig, check, ptr
+from .driver import crop_log_assignment
+from .weights import native_table
 
 LOG2E = 1.4426950408889634
 
@@ -39,6 +44,21 @@ def weight_planes(t: torch.Tensor) -> torch.Tensor:
     t = t.detach().to(torch.float32) * 256.0
     hi = t.to(torch.float16)
     return torch.stack([hi, (t - hi.to(torch.float32)).to(torch.float16)]).contiguous()
+
+
+def _capture(graph: "torch.cuda.CUDAGraph", fn):
+    """fn() captured into `graph` -> what fn returns.  The cyclic garbage collector is off during the capture: a
+    collection there can destroy another module's graphs (an adaptive entry's tail closure refers back to its module,
+    so a dropped module is cyclic garbage, and torch.cuda.graph no longer collects before capturing), and destroying a
+    graph during a capture invalidates the capture."""
+    enabled = gc.isenabled()
+    gc.disable()
+    try:
+        with torch.cuda.graph(graph):
+            return fn()
+    finally:
+        if enabled:
+            gc.enable()
 
 
 class _Conf(dict):
@@ -156,6 +176,12 @@ class LightGlue(nn.Module):
         # with cuda_graph: return the graph's own output buffers (valid until the next call) instead of copies --
         # saves the 16.8 MB-per-pair copy of log_assignment at 2048 keypoints
         "graph_static_outputs": False,
+        # B200 extension: with cuda_graph, an int K captures the forward once at K keypoints per image (lgb200_match at
+        # B x K x K) and replays that graph for every input with max(m, n) <= K, zero-padded, with the counts
+        # (num_keypoints0/1 or m / n) on the device: one capture serves a stream of varying keypoint counts.  bf16 / fp32
+        # without adaptive depth / width; anything else takes the path it takes without this key.  A replay at K costs
+        # a little more than one at the exact size, so streams of one fixed size are better served without it
+        "graph_capacity": None,
         # B200 extension: arithmetic of a training step (module in training mode, autograd on; the no-grad forward
         # follows `precision`).  "fp32" = the fp32-accurate tensor-core mode; "bf16" = mixed precision: the bf16
         # inference kernels forward (outputs bit-equal to the no-grad forward with precision="bf16"), bf16 tensor-core
@@ -169,6 +195,9 @@ class LightGlue(nn.Module):
         super().__init__()
         self.conf = conf = _merge_conf(self.default_conf, conf)
         self._train_bf16()  # (validates conf.train_precision)
+        cap = conf.graph_capacity
+        if cap is not None and (isinstance(cap, bool) or not isinstance(cap, numbers.Integral) or cap <= 0):
+            raise ValueError(f"graph_capacity must be None or a positive int, got {cap!r}")
         d = conf.descriptor_dim
         if d != 256 or conf.num_heads != 4:
             raise NotImplementedError("the B200 kernels are specialised for descriptor_dim=256, num_heads=4")
@@ -718,17 +747,19 @@ class LightGlue(nn.Module):
         for key in self.required_data_keys:
             assert key in data, f"Missing key {key} in data"
         conf = self.conf
-        graphable = (
-            conf.cuda_graph and not self.training
-            and "num_keypoints0" not in data and "num_keypoints1" not in data and data["keypoints0"].is_cuda
-        )
-        if not graphable:
+        if not (conf.cuda_graph and not self.training and data["keypoints0"].is_cuda):
             return self._forward_impl(data)
         # adaptive depth / width: the transformer stack (all layers; the kernels skip finished pairs and pruned rows
         # from device-side counts) is captured, the data-dependent tail -- one host read of the exit layers and the
         # pruned counts, MatchAssignment of the exit layer at the pruned shape, filter_matches -- runs eagerly behind
         # every replay (lightglue.py:501-536)
         adaptive = conf.depth_confidence > 0 or conf.width_confidence > 0
+        cap = conf.get("graph_capacity")
+        if (cap is not None and not adaptive and self._precision() in (BF16, F32X3)
+                and max(data["keypoints0"].shape[1], data["keypoints1"].shape[1]) <= cap):
+            return self._forward_capacity(data, int(cap))
+        if "num_keypoints0" in data or "num_keypoints1" in data:
+            return self._forward_impl(data)
         # ---- CUDA-graph path: static copies of the inputs, one captured forward per input signature ----
         ins = {k: data[k] for k in self._GRAPH_INPUTS if isinstance(data.get(k), torch.Tensor)}
         for v in ("view0", "view1"):
@@ -755,8 +786,7 @@ class LightGlue(nn.Module):
                 warm()
             torch.cuda.synchronize(dev)
             graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                out = self._forward_impl(as_data(), static=adaptive)  # adaptive: the tail closure
+            out = _capture(graph, lambda: self._forward_impl(as_data(), static=adaptive))  # adaptive: the tail closure
             if len(self._graphs) >= 8:  # a handful of signatures at most; drop the oldest
                 self._graphs.pop(next(iter(self._graphs)))
             # the captured launches carry raw device pointers (and TMA tensor maps) into the weight pack: the entry
@@ -771,6 +801,25 @@ class LightGlue(nn.Module):
         if conf.get("graph_static_outputs", False):  # caller consumes the results before the next call: no copies
             return dict(out)
         return {k: v.clone() for k, v in out.items()}  # the graph's output buffers are overwritten by the next replay
+
+    def _forward_capacity(self, data: dict, cap: int) -> dict:
+        """conf.graph_capacity: one CUDA graph of lgb200_match at B x cap x cap per (precision, weights, B, which image
+        sizes are given) serves every input with max(m, n) <= cap.  The outputs are bit-equal to the eager forward of
+        the input zero-padded to cap with the same counts, cropped to this input's shapes.  A call reads nothing back
+        and makes no library call: it copies the pair in, replays and crops."""
+        dev = data["keypoints0"].device
+        B = data["keypoints0"].shape[0]
+        prec = self._precision()
+        self._pack(prec, dev)
+        sizes = [data[v].get("image_size") if v in data else None for v in ("view0", "view1")]
+        key = (prec, self._pack_key, B, cap, sizes[0] is not None, sizes[1] is not None)
+        entry = self._graphs.get(key)
+        if entry is None:
+            entry = _CapacityGraph(self, prec, B, cap, data, sizes)
+            if len(self._graphs) >= 8:  # shares the per-signature captures' limit: drop the oldest
+                self._graphs.pop(next(iter(self._graphs)))
+            self._graphs[key] = entry
+        return entry(data, sizes, self.conf.get("graph_static_outputs", False))
 
     def _forward_impl(self, data: dict, static: bool = False):
         lib = _abi.load()
@@ -1144,5 +1193,109 @@ class LightGlue(nn.Module):
 
 
         return tail if static else tail()
+
+
+class _CapacityGraph:
+    """The forward captured at a keypoint capacity K (conf.graph_capacity): one lgb200_match call at B x K x K on static
+    inputs, device counts, a workspace and output buffers.  lgb200_match allocates nothing, synchronises nothing and
+    reads no count on the host, so the graph serves any input of at most K keypoints per image.  The entry owns the
+    packed weights its launches point into: a precision switch replaces the module's pack but cannot free them."""
+
+    def __init__(self, model: LightGlue, prec: int, B: int, K: int, data: dict, sizes: list):
+        conf = model.conf
+        dev = data["keypoints0"].device
+        self.B, self.K, self.n_layers = B, K, conf.n_layers
+        kdim = 4 if conf.add_scale_ori else 2
+        self.cfg = MatchConfig(prec, conf.n_layers, conf.input_dim, kdim, float(conf.filter_threshold))
+        self.table, self.weights = native_table(model, prec)
+        f32, i64 = dict(device=dev, dtype=torch.float32), dict(device=dev, dtype=torch.int64)
+        self.kpts = [torch.zeros(B, K, kdim, **f32) for _ in range(2)]
+        self.desc = [torch.zeros(B, K, conf.input_dim, **f32) for _ in range(2)]
+        self.rows = [0, 0]  # rows of kpts / desc that may hold something other than zeros
+        self.size = [None if s is None else torch.empty(B, 2, **f32) for s in sizes]
+        self.counts = torch.empty(2, B, device=dev, dtype=torch.int32)
+        lib = _abi.load()
+        nb = ctypes.c_longlong(0)
+        check(lib.lgb200_match_workspace(ctypes.byref(self.cfg), B, K, K, ctypes.byref(nb)), "match_workspace")
+        self.ws = torch.empty(nb.value, device=dev, dtype=torch.uint8)
+        act = torch.bfloat16 if prec == BF16 else torch.float32
+        self.out = {
+            "matches0": torch.empty(B, K, **i64), "matches1": torch.empty(B, K, **i64),
+            "matching_scores0": torch.empty(B, K, **f32), "matching_scores1": torch.empty(B, K, **f32),
+            "ref_descriptors0": torch.empty(B, K, 256, device=dev, dtype=act),
+            "ref_descriptors1": torch.empty(B, K, 256, device=dev, dtype=act),
+            "log_assignment": torch.empty(B, K + 1, K + 1, **f32),
+        }
+        self._load(data, sizes)
+        self._launch(lib)  # outside the capture: lazy initialisation
+        torch.cuda.synchronize(dev)
+        self.graph = torch.cuda.CUDAGraph()
+        _capture(self.graph, lambda: self._launch(lib))
+
+    def _launch(self, lib) -> None:
+        o = self.out
+        check(lib.lgb200_match(
+            ctypes.byref(self.cfg), self.table, self.B, self.K, self.K, ptr(self.kpts[0]), ptr(self.kpts[1]),
+            ptr(self.desc[0]), ptr(self.desc[1]), ptr(self.size[0]), ptr(self.size[1]), ptr(self.counts[0]),
+            ptr(self.counts[1]), ptr(o["matches0"]), ptr(o["matches1"]), ptr(o["matching_scores0"]),
+            ptr(o["matching_scores1"]), ptr(o["log_assignment"]), ptr(o["ref_descriptors0"]),
+            ptr(o["ref_descriptors1"]), ptr(self.ws), self.ws.numel(),
+            torch.cuda.current_stream(self.ws.device).cuda_stream), "lgb200_match")
+
+    def _load(self, data: dict, sizes: list) -> None:
+        """The pair into the static inputs: its rows, zeros over the rows a larger earlier input left (so every row past
+        m / n is zero and the result cannot depend on an earlier call), the counts min(num_keypoints, m) or m, the image
+        sizes.  Copies only: nothing is read back."""
+        B = self.B
+        for i in (0, 1):
+            kp, dsc, k, d = data[f"keypoints{i}"], data[f"descriptors{i}"], self.kpts[i], self.desc[i]
+            c = kp.shape[1]
+            assert dsc.shape[-1] == d.shape[-1]
+            k[:, :c, :2].copy_(kp, non_blocking=True)
+            if k.shape[2] == 4:  # add_scale_ori (lightglue.py:436-454)
+                k[:, :c, 2].copy_(data[f"scales{i}"].reshape(B, c), non_blocking=True)
+                k[:, :c, 3].copy_(data[f"oris{i}"].reshape(B, c), non_blocking=True)
+            d[:, :c].copy_(dsc, non_blocking=True)
+            if self.rows[i] > c:
+                k[:, c:self.rows[i]].zero_()
+                d[:, c:self.rows[i]].zero_()
+            self.rows[i] = c
+            cnt = data.get(f"num_keypoints{i}")
+            if cnt is None:
+                self.counts[i].fill_(c)
+            else:
+                self.counts[i].copy_(torch.as_tensor(cnt).reshape(-1).clamp(max=c), non_blocking=True)
+            if sizes[i] is not None:
+                self.size[i].copy_(torch.as_tensor(sizes[i]).reshape(-1, 2), non_blocking=True)
+
+    def __call__(self, data: dict, sizes: list, static_outputs: bool) -> dict:
+        """Load, replay, and fresh outputs in the shapes of the eager forward for this input: log_assignment cropped
+        to [B, m+1, n+1] with the dustbins moved to row m and column n.  static_outputs: the graph's own buffers (valid
+        until the next call) when they already have those shapes: m == n == K and no counts given."""
+        B, K = self.B, self.K
+        m, n = data["keypoints0"].shape[1], data["keypoints1"].shape[1]
+        self._load(data, sizes)
+        self.graph.replay()
+        o = self.out
+        dev = self.ws.device
+        prune0 = torch.full((B, m), float(self.n_layers), device=dev, dtype=torch.float32)
+        prune1 = torch.full((B, n), float(self.n_layers), device=dev, dtype=torch.float32)
+        if static_outputs and m == n == K and "num_keypoints0" not in data and "num_keypoints1" not in data:
+            return {
+                "matches0": o["matches0"], "matches1": o["matches1"],
+                "matching_scores0": o["matching_scores0"], "matching_scores1": o["matching_scores1"],
+                "ref_descriptors0": o["ref_descriptors0"][:, None], "ref_descriptors1": o["ref_descriptors1"][:, None],
+                "log_assignment": o["log_assignment"], "prune0": prune0, "prune1": prune1,
+            }
+        return {
+            "matches0": o["matches0"][:, :m].clone(), "matches1": o["matches1"][:, :n].clone(),
+            "matching_scores0": o["matching_scores0"][:, :m].clone(),
+            "matching_scores1": o["matching_scores1"][:, :n].clone(),
+            "ref_descriptors0": o["ref_descriptors0"][:, None, :m].clone(),
+            "ref_descriptors1": o["ref_descriptors1"][:, None, :n].clone(),
+            "log_assignment": crop_log_assignment(o["log_assignment"], m, n),
+            "prune0": prune0, "prune1": prune1,
+        }
+
 
 __main_model__ = LightGlue
