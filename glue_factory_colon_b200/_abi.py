@@ -24,7 +24,13 @@ class MatchConfig(C.Structure):
                 ("filter_threshold", C.c_float)]
 
 
+class AdaptiveConfig(C.Structure):
+    """lgb200_adaptive_config (lgb200_match_adaptive): a confidence <= 0 turns its mode off."""
+    _fields_ = [("depth_confidence", C.c_float), ("width_confidence", C.c_float)]
+
+
 _cfg = C.POINTER(MatchConfig)
+_acfg = C.POINTER(AdaptiveConfig)
 
 # name -> argtypes, exactly as declared in include/lightglue_b200.h
 SIGNATURES = {
@@ -70,6 +76,10 @@ SIGNATURES = {
     "lgb200_match_workspace": [_cfg, _i, _i, _i, _p],
     "lgb200_match": [_cfg, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p,
                      C.c_longlong, _p],
+    "lgb200_adaptive_table_size": [_cfg, _p, _p],
+    "lgb200_pack_weights_adaptive": [_cfg, _i, _p, _p, _p, C.c_longlong, _p, _p],
+    "lgb200_match_adaptive_workspace": [_cfg, _i, _i, _i, _p],
+    "lgb200_match_adaptive": [_cfg, _acfg, _p, _i, _i, _i] + [_p] * 19 + [_p, C.c_longlong, _p],
     "lgb200_prune_compact": [_p, _p, _f, _f, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
 }
 

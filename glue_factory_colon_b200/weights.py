@@ -74,10 +74,11 @@ NATIVE_LAYER_ENTRIES = ("qkv_w", "qkv_b", "sf0_w", "sf0_b", "sln_g", "sln_b", "s
                         "cqv_w", "cqv_b", "cf0_w", "cf0_b", "cln_g", "cln_b", "cf3_w", "cf3_b")
 
 
-def native_table(model: torch.nn.Module, prec: int) -> Tuple[object, List[torch.Tensor]]:
+def native_table(model: torch.nn.Module, prec: int, adaptive: bool = False) -> Tuple[object, List[torch.Tensor]]:
     """The packed-weight table of lgb200_match built from `model._pack(prec)` on the model's device (prec = _abi.BF16
     or _abi.F32X3): (ctypes array of device pointers, the tensors they point into).  The tensors must outlive every
-    call that uses the table."""
+    call that uses the table.  adaptive=True: the table of lgb200_match_adaptive, with the MatchAssignment and the
+    token-confidence head of every layer but the last appended (fp_w, fp_b, m_w, m_b, tk_w, tk_b per layer)."""
     import ctypes
 
     packed = model._pack(prec, next(model.parameters()).device)
@@ -86,4 +87,7 @@ def native_table(model: torch.nn.Module, prec: int) -> Tuple[object, List[torch.
     tensors += [packed["wr"], a["fp_w"], a["fp_b"], a["m_w"], a["m_b"]]
     if "in_w" in packed:
         tensors += [packed["in_w"], packed["in_b"]]
+    if adaptive:
+        for a, t in zip(packed["assign"][:-1], packed["token"]):
+            tensors += [a["fp_w"], a["fp_b"], a["m_w"], a["m_b"], t["w"], t["b"]]
     return (ctypes.c_void_p * len(tensors))(*[t.data_ptr() for t in tensors]), tensors

@@ -481,6 +481,83 @@ int lgb200_match(const lgb200_match_config* cfg, const void* const* table, int B
                  float* log_assignment, void* desc_out0, void* desc_out1,
                  void* workspace, long long workspace_bytes, void* stream);
 
+/* ---- adaptive matcher ---------------------------------------------------------------------------------------------
+ * The same forward with LightGlue's adaptive depth (early exit, lightglue.py:501-505, 569-580) and adaptive width
+ * (point pruning, :506-521, 560-567).  lgb200_match_adaptive makes the calls of LightGlue._forward_impl with every
+ * layer launched (pairs that stopped cost empty kernels) and its tail -- MatchAssignment of each pair's exit layer,
+ * filter_matches at the pruned counts -- on the device: no allocation, no synchronisation, no host read.  One capture
+ * at B x K x K serves every input and every count, as for lgb200_match; the outputs are bit-equal to LightGlue.forward
+ * with the same conf, in the layouts below. */
+typedef struct {
+  float depth_confidence; /* > 0: early exit after layers 0 .. n_layers-2; else off */
+  float width_confidence; /* > 0: point pruning; else off */
+} lgb200_adaptive_config;
+
+/* Adaptive table: *entries = the lgb200_weight_table_size entries + 6 (n_layers - 1), *pack_bytes likewise (every
+ * entry 256-byte aligned).  The first entries are exactly lgb200_pack_weights' table (an adaptive table also serves
+ * lgb200_match); then, per layer l < n_layers-1, at base + 6 l + j (base = 16 n_layers + 5 (+ 2)):
+ *    j  0 fp_w  W [256][256]  log_assignment.{l}.final_proj.weight     1 fp_b  F [256]  final_proj.bias
+ *       2 m_w   F [256]       log_assignment.{l}.matchability.weight   3 m_b   F [1]    matchability.bias
+ *       4 tk_w  F [256]       token_confidence.{l}.token.0.weight      5 tk_b  F [1]    token.0.bias
+ * (layer n_layers-1's MatchAssignment is the tail of the first part).  W and F as for lgb200_weight_table_size. */
+int lgb200_adaptive_table_size(const lgb200_match_config* cfg, int* entries, long long* pack_bytes);
+
+/* lgb200_pack_weights for the adaptive table: same arguments and rules, with these names required besides the
+ * REQUIRED WEIGHTS above (a missing one returns LGB200_ERR_WEIGHTS before anything is launched):
+ * BEGIN ADAPTIVE WEIGHTS
+ *   log_assignment.{l}.final_proj.weight            log_assignment.{l}.final_proj.bias
+ *   log_assignment.{l}.matchability.weight          log_assignment.{l}.matchability.bias
+ *   token_confidence.{l}.token.0.weight             token_confidence.{l}.token.0.bias
+ * END ADAPTIVE WEIGHTS
+ * for every layer l < L-1.  The confidence thresholds are not read: lgb200_match_adaptive computes
+ * LightGlue.confidence_threshold, clip(0.8 + 0.1 exp(-4 l / L), 0, 1) in double rounded to float, on the host. */
+int lgb200_pack_weights_adaptive(const lgb200_match_config* cfg, int n, const char* const* names,
+                                 const float* const* tensors, void* pack_buf, long long pack_bytes,
+                                 const void** table, void* stream);
+
+/* *bytes = the workspace of lgb200_match_adaptive for B pairs of capacity m x n.  It depends on neither the counts nor
+ * the confidences: lgb200_match_workspace's layout followed by, each 256-byte aligned, with T = 2 B Lp,
+ * act = 2 (bf16) / 4 (fp32) bytes and rot = 128 (bf16) / 256 (fp32) bytes per token:
+ *   ind, prune_cnt, conf, msig, ind_b   5 x T x 4      x_b  T x 256 x act      rot_b  T x rot
+ *   done | lens_active | total  (2 B + 2 B) x 4        per-exit-layer counts  n_layers x 2 B x 4 */
+int lgb200_match_adaptive_workspace(const lgb200_match_config* cfg, int B, int m, int n, long long* bytes);
+
+/* The adaptive forward.  cfg, table (from lgb200_pack_weights_adaptive), B, m, n and the inputs and outputs up to
+ * desc_out0/1 as for lgb200_match, with:
+ *   log_assignment  fp32 [B, m+1, n+1], dustbin row m, dustbin column n; pair b's valid block is [:k0_b, :k1_b] at its
+ *                   pruned counts (LightGlue.forward returns [B, max k0 + 1, max k1 + 1]: crop_log_assignment).
+ *   matches0/1, scores0/1  indexed by the un-pruned keypoint, as LightGlue.forward returns them.
+ *   desc_out0/1     the exit layer's descriptors, compacted by the pruning: rows < k_b, zeros past them.
+ * and, each nullable:
+ *   prune0/1        int32 [B, m|n]: the layer count of each keypoint (LightGlue.forward's prune0/1; n_layers for
+ *                   every keypoint without width pruning);
+ *   exit_layer      int32 [B]: the layer whose MatchAssignment gave the pair's outputs (n_layers-1 if it never exited);
+ *   final_counts    int32 [B][2]: the pruned counts (k0_b, k1_b).
+ * acfg NULL: LGB200_ERR_NULL.  Width pruning with Lp > 8192 (lgb200_prune_compact's limit): LGB200_ERR_SHAPE.  Both
+ * argument checks come before any launch; with either mode on, every table entry must be non-NULL.
+ * workspace: lgb200_match_adaptive_workspace bytes, 256-byte aligned.
+ * Both confidences <= 0: exactly the calls of lgb200_match (same outputs), then one kernel that fills prune0/1,
+ * exit_layer and final_counts if any of them is non-NULL.
+ * Otherwise, with d = 1 under depth and 0 else, w likewise for width, x = 1 in LGB200_F32X3 and 0 in LGB200_BF16, the
+ * kernel launches are those of lgb200_match with non-NULL counts on the same cfg and shapes, plus
+ *     1                                 the adaptive state (lens_active, total, done, ind, prune_cnt)
+ *   + (n_layers - 1) (2 d + (2 + x) w)  per layer but the last: token head + exit check, matchability + compaction
+ *                                       (+ the plane split in LGB200_F32X3)
+ *   + d (1 + (n_layers - 1) g)          the per-exit-layer counts and n_layers MatchAssignment groups instead of
+ *                                       one, g = the group's launches: final_proj, matchability and lgb200_assign_lse
+ *                                       (3) in LGB200_BF16; final_proj, matchability, lgb200_x3_similarity and
+ *                                       lgb200_x3_assign_lse (3 + [m > 0] + [n > 0]) in LGB200_F32X3
+ *   + 1                                 the descriptors, prune0/1, exit_layer and final_counts (when any is non-NULL)
+ * besides cudaMemsetAsync where the Python forward allocates zeros.  No cudaMemcpy: desc_out0/1 follow device counts. */
+int lgb200_match_adaptive(const lgb200_match_config* cfg, const lgb200_adaptive_config* acfg,
+                          const void* const* table, int B, int m, int n,
+                          const float* kpts0, const float* kpts1, const float* desc0, const float* desc1,
+                          const float* size0, const float* size1, const int32_t* counts0, const int32_t* counts1,
+                          int64_t* matches0, int64_t* matches1, float* scores0, float* scores1,
+                          float* log_assignment, void* desc_out0, void* desc_out1,
+                          int32_t* prune0, int32_t* prune1, int32_t* exit_layer, int32_t* final_counts,
+                          void* workspace, long long workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
